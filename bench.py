@@ -3,7 +3,7 @@
 calc_probs samples*points/sec, 18 scenarios, N = 1e6 prior draws per scenario.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--config 2|3|4] [--draws N] [--scaling weak|strong]
+                    [--config 2|3|4] [--draws N] [--scaling weak|strong] [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one batch of synthetic input: the 12 engine calls
 (6 TP-type, 6 EB-type) that a full 18-row `target.calc_probs` makes -- 15 target-star rows + NTP,
@@ -26,6 +26,18 @@ code (numpy seed), exactly as `calc_probs` makes them.
              oracle, device lnZ against the host log-mean-exp, probabilities.
   cpu_baseline / --impl reference: the same public call routed to the oracle port (C
              restatement + numpy masks, all host cores) on a bounded number of draws.
+
+--steps K times K steps in every GPU leg (value, e2e.engine, e2e, e2e.device_sampler).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned as
+float64 DIR/<name>.npy (a few kB in all), so that two builds can be compared output for output on
+the same seeded inputs:
+  lnZ, records, top_lnL, top_idx   the `value` leg: per scenario branch (engine-call order, TP
+             one branch, EB two) the evidence, its (m, s, n_finite, n_posinf, n_pass) record and
+             the 100 best draws (sorted best first, ties by index; NaN / -1 past n_top)
+  e2e_lnZ, e2e_prob, e2e_best, e2e_fpp_nfpp   the `e2e` leg (calc_probs): the 18 rows' lnZ and
+             probabilities, their best-draw table (columns E2E_BEST_COLUMNS) and (FPP, NFPP);
+             absent with --kernel-only
 
 N > 1 (torchrun, one rank per GPU): --scaling weak (default): every rank evaluates its own N
 draws per scenario (different seed per rank); --scaling strong: N draws in total, sharded.  One
@@ -54,6 +66,8 @@ N_ROWS = 18            # scenario rows of the configuration
 N_BEST = 100           # best draws returned per row (marginal_likelihoods.py:152)
 SEED = 2026
 METRIC = "calc_probs samples*points/sec (18 scenarios, N=1e6)"
+E2E_BEST_COLUMNS = ("M_s", "R_s", "P_orb", "inc", "b", "ecc", "w", "R_p", "M_EB", "R_EB")
+DUMP_LIMIT_BYTES = 64 << 20
 
 # FP64 issue slots per model point (DESIGN.md "Roofline", frozen from SURVEY.md 8d)
 SLOTS_ORBIT, SLOTS_INTERIOR, SLOTS_LIMB, SLOTS_STAMP = 90, 367, 489, 4
@@ -188,6 +202,30 @@ def _measured_peaks():
         return {}
 
 
+def _value_outputs(dev_calls, dev_tops, lnZ):
+    """What the value leg's last step returned, per scenario branch (see --dump-outputs)."""
+    rows = [r for _, _, res in dev_calls for r in res]
+    top_lnL = np.full((len(rows), N_BEST), np.nan)
+    top_idx = np.full((len(rows), N_BEST), -1.0)
+    for j, (r, (di, dv)) in enumerate(zip(rows, dev_tops)):
+        idx, val = di.cpu().numpy()[:r.n_top], dv.cpu().numpy()[:r.n_top]
+        order = np.lexsort((idx, -val))     # device-pointer calls return them unsorted
+        top_idx[j, :r.n_top], top_lnL[j, :r.n_top] = idx[order], val[order]
+    return {"lnZ": np.asarray(lnZ, np.float64),
+            "records": np.array([[r.m, r.s, r.n_finite, r.n_posinf, r.n_pass] for r in rows],
+                                np.float64),
+            "top_lnL": top_lnL, "top_idx": top_idx}
+
+
+def _dump_outputs(out_dir, arrays):
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "dump of %d bytes exceeds 64 MB" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _slice_call(c, lo, hi):
     """The draws [lo, hi) of a recorded engine call."""
     def sl(x):
@@ -240,6 +278,7 @@ def run_ours(args):
     # ---- device-resident copies (value path) and pinned host copies (engine-level e2e)
     keep = []
     dev_calls, host_calls = [], []
+    dev_tops = []                       # (top_idx, top_lnL) device buffers, one per branch
     h2d_bytes = d2h_bytes = 0
     # the engine-level leg keeps a second, page-locked copy of every column: skipped when that
     # would pin more than 4 GB of host memory (N = 1e7)
@@ -285,6 +324,7 @@ def run_ours(args):
             pi_ = torch.empty(N_BEST, dtype=torch.int64, pin_memory=True)
             pv = torch.empty(N_BEST, dtype=torch.float64, pin_memory=True)
             keep += [di, dv, pi_, pv]
+            dev_tops.append((di, dv))
             dres[b].top_cap = hres[b].top_cap = N_BEST
             dres[b].top_idx, dres[b].top_lnL = di.data_ptr(), dv.data_ptr()
             hres[b].top_idx, hres[b].top_lnL = pi_.numpy().ctypes.data, pv.numpy().ctypes.data
@@ -377,9 +417,13 @@ def run_ours(args):
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
+    # before the counting pass below overwrites the results of the last timed step
+    outputs = _value_outputs(dev_calls, dev_tops, lnZ) if args.dump_outputs else None
 
     if args.kernel_only:
         if rank == 0:
+            if outputs is not None:
+                _dump_outputs(args.dump_outputs, outputs)
             print(json.dumps({"lib": os.environ.get("TRI_B200_LIB", "default"),
                               "config": config, "ms_per_step": ms_total / args.steps,
                               "lnl_ms_per_step": stat["lnl_ms"] / args.steps,
@@ -412,7 +456,6 @@ def run_ours(args):
     # ---- e2e: the public call.  target.calc_probs with numpy's draws (parity mode), N_total
     # draws per scenario, sharded over the ranks by the package itself
     import triceratops_b200
-    e2e_steps = max(1, min(args.steps, 5))
 
     def public_call(sampler_mode, n_calls, n_warm):
         tgt = _workloads.make_target(config)
@@ -430,12 +473,16 @@ def run_ours(args):
         return walls, tgt
 
     n_warm = 2 if N_total <= 2_000_000 else 1
-    walls, tgt = public_call("host", e2e_steps, n_warm)
+    walls, tgt = public_call("host", args.steps, n_warm)
     e2e_s = float(np.mean(walls[n_warm:]))
     probs_gpu = np.asarray(tgt.probs.prob.values, float)
     lnZ_rows = np.asarray(tgt.lnZ, float)
     fpp, nfpp = float(tgt.FPP), float(tgt.NFPP)
-    dwalls, dtgt = public_call("device", 2, 1)
+    if outputs is not None:
+        outputs.update(e2e_lnZ=lnZ_rows, e2e_prob=probs_gpu, e2e_fpp_nfpp=[fpp, nfpp],
+                       e2e_best=tgt.probs[list(E2E_BEST_COLUMNS)].to_numpy(np.float64))
+    dwalls, dtgt = public_call("device", args.steps, 1)
+    dev_s = float(np.mean(dwalls[1:]))
 
     # ---- roofline of lnl_kernel (per launch, averaged over the timed launches)
     ns = calls[0]["lc"][4]
@@ -499,7 +546,7 @@ def run_ours(args):
                    "parallelism": "draws sharded, dp%d" % world},
         "e2e": {"value": N_ROWS * N_total * npts / e2e_s, "unit": "samples*points/s",
                 "h2d_bytes_per_step": int(h2d_bytes), "d2h_bytes_per_step": int(d2h_bytes),
-                "ms_per_step": e2e_s * 1e3, "steps": e2e_steps, "all_walls_s": walls,
+                "ms_per_step": e2e_s * 1e3, "steps": args.steps, "all_walls_s": walls,
                 "api": "target.calc_probs(time, flux, sigma, P_orb, contrast_curve_file, filt, "
                        "N=%d, parallel=True): numpy prior draws in the reference's order "
                        "(sequential generator), transforms, pinned staging + H2D, kernels, "
@@ -510,8 +557,8 @@ def run_ours(args):
                     "ms_per_step": engine_s * 1e3 / args.steps,
                     "api": "tri_submit_tp/eb + tri_wait on pinned host columns (draws already "
                            "made), up to %d calls in flight" % _cabi.TRI_MAX_INFLIGHT},
-                "device_sampler": {"value": N_ROWS * N_total * npts / dwalls[-1],
-                                   "ms_per_step": dwalls[-1] * 1e3,
+                "device_sampler": {"value": N_ROWS * N_total * npts / dev_s,
+                                   "ms_per_step": dev_s * 1e3, "steps": args.steps,
                                    "FPP": float(dtgt.FPP), "NFPP": float(dtgt.NFPP),
                                    "note": "opt-in mode: prior draws generated on the GPU "
                                            "(statistically equivalent, not numpy's stream)"}},
@@ -546,6 +593,8 @@ def run_ours(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_leg(config, lc, args.cpu_draws, steps=1, warmup=0)
     if rank == 0:
+        if outputs is not None:
+            _dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -686,7 +735,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--kernel-only", action="store_true",
                     help="A/B runs: the device-resident leg only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU legs' outputs: --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:
