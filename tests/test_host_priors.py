@@ -95,3 +95,19 @@ def test_trilegal_table_is_cached_per_file_version(tmp_path, trilegal_file):
     c = funcs.trilegal_results(path, -99.0)
     full = funcs.trilegal_results(trilegal_file, -99.0)
     assert c[0].size == full[0].size - 10
+
+
+@pytest.mark.parametrize("mission", ["TESS", "Kepler"])
+def test_dense_ldc_table_holds_the_rounded_lookup_of_every_node(mission):
+    """The device sampler's (Teff, logg) table at each tabulated Z: every grid node's entry is
+    what at_Z_rounded returns for that node, and there is no other entry."""
+    from triceratops_b200._ldc import grid_for
+    grid = grid_for(mission)
+    for Z in np.unique(grid.Zs):
+        at_Z = grid.Zs == Z
+        T, logg = grid.Teffs[at_Z].astype(float), grid.loggs[at_Z]
+        u1, u2 = grid.at_Z_rounded(Z, T, logg, 10000)
+        tab1, tab2 = grid.dense_table(Z)
+        it, ig = ((T - 3500) // 250).astype(int), np.round((logg - 3.5) / 0.5).astype(int)
+        assert np.array_equal(tab1[it, ig], u1) and np.array_equal(tab2[it, ig], u2)
+        assert np.isfinite(tab1).sum() == np.isfinite(tab2).sum() == at_Z.sum()

@@ -681,8 +681,3 @@ class TableExchange:
             pad = rows[-1:] if len(rows) else np.zeros((1, len(keys)))
             rows = np.concatenate([rows, np.repeat(pad, N_BEST - len(rows), axis=0)])
         return lnZ, n_pass, n_eval, {k: rows[:, i].copy() for i, k in enumerate(keys)}
-
-
-def merge_tables(lb, table, keys):
-    """One-shot form of TableExchange (a single lnZ_* call)."""
-    return TableExchange(lb, table, keys).result()

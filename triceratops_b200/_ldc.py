@@ -72,31 +72,33 @@ class LdcGrid:
                                       np.ascontiguousarray(self.u2s[at_Z][order]))
         return self._node_tables[key]
 
+    def dense_table(self, Z):
+        """(u1, u2) of node_table(Z) as two (27, 4) arrays indexed by ((Teff - 3500) / 250,
+        (logg - 3.5) / 0.5), NaN where the grid has no node -- the layout the device sampler's
+        kernel reads."""
+        codes, u1, u2 = self.node_table(Z)
+        it, ig = (codes // 100 - 3500) // 250, (codes % 100 - 35) // 5
+        tab1, tab2 = np.full((27, 4), np.nan), np.full((27, 4), np.nan)
+        tab1[it, ig], tab2[it, ig] = u1, u2
+        return tab1, tab2
+
     # ---- bound companions: round onto the grid at the target's Z    :945-972 / :1160-1187
     def at_Z_rounded(self, Z, Teffs, loggs, Teff_cap):
-        at_Z = self.Zs == self.Zs[np.abs(self.Zs - Z).argmin()]
-        T_at, g_at = self.Teffs[at_Z], self.loggs[at_Z]
-        u1_at, u2_at = self.u1s[at_Z], self.u2s[at_Z]
+        code_sorted, u1_at, u2_at = self.node_table(Z)
         rg = np.round(loggs / 0.5) * 0.5
         rg[rg < 3.5] = 3.5
         rg[rg > 5.0] = 5.0
         rT = np.round(Teffs / 250) * 250
         rT[rT < 3500] = 3500
         rT[rT > Teff_cap] = Teff_cap
-        # node code -> row; every draw must hit exactly one node, as with the reference's .item()
-        code_tab = T_at.astype(np.int64) * 100 + np.round(g_at * 10).astype(np.int64)
-        order = np.argsort(code_tab, kind="stable")
-        code_sorted = code_tab[order]
-        if np.any(np.diff(code_sorted) == 0):
-            raise ValueError("can only convert an array of size 1 to a Python scalar")
+        # every draw must hit exactly one node, as with the reference's .item()
         code = rT.astype(np.int64) * 100 + np.round(rg * 10).astype(np.int64)
         pos = np.searchsorted(code_sorted, code)
         pos[pos >= code_sorted.size] = code_sorted.size - 1
         hit = (code_sorted[pos] == code) & (rT == np.round(rT))
         if not np.all(hit):
             raise ValueError("can only convert an array of size 1 to a Python scalar")
-        rows = order[pos]
-        return u1_at[rows], u2_at[rows]
+        return u1_at[pos], u2_at[pos]
 
     # ---- background stars: nearest Teff, nearest logg, then nearest tabulated Z   :1913-1924
     def nearest_each(self, Teffs, loggs, Zs):

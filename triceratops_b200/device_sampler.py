@@ -28,13 +28,12 @@ import os
 
 import numpy as np
 import torch
-from pandas import read_csv
 
-from . import _cabi, _dispatch, funcs
+from . import _cabi, _dispatch, funcs, priors
+from . import marginal_likelihoods as ml
 from ._cabi import tri_bound_prior, tri_powerlaw, tri_sampler_args, tri_spline
-from ._constants import G, Msun, Rsun, pi
 from ._ldc import grid_for
-from .funcs import file_to_contrast_curve, trilegal_results
+from .funcs import file_to_contrast_curve
 
 N_SAMPLES = 100
 F64 = torch.float64
@@ -62,55 +61,20 @@ def _cached(key, make):
 
 
 # ------------------------------------------------------------------------------- descriptors
-def _powerlaw(edges, powers, amps):
-    """Constants of priors._piecewise_powerlaw for the kernel's inverse CDF."""
+def _powerlaw(spec):
+    """tri_powerlaw of a priors law (edges, powers, amps) for the kernel's inverse CDF; None:
+    every draw is 1.0."""
     L = tri_powerlaw()
+    if spec is None:
+        L.nseg, L.constant = 0, 1.0
+        return L
+    edges, powers, amps = spec
+    integrals, cum, L.norm = priors.powerlaw_tables(edges, powers, amps)
     L.nseg = len(powers)
-    tot = 0.0
     for k in range(L.nseg):
-        p1 = powers[k] + 1
-        integral = amps[k] * (edges[k + 1] ** p1 - edges[k] ** p1) / p1
-        tot += integral
-        L.powers[k], L.amps[k], L.integrals[k], L.cum[k] = powers[k], amps[k], integral, tot
-        L.epow[k] = edges[k] ** p1
-    L.norm = 1 / tot
+        L.powers[k], L.amps[k], L.integrals[k], L.cum[k] = powers[k], amps[k], integrals[k], cum[k]
+        L.epow[k] = edges[k] ** (powers[k] + 1)
     return L
-
-
-def _constant(value):
-    L = tri_powerlaw()
-    L.nseg, L.constant = 0, value
-    return L
-
-
-def _rp_laws():
-    """sample_rp (priors.py:16-116): host mass above / below 0.45 M_sun."""
-    edges = (0.5, 3.0, 6.0, 20.0)
-    out = []
-    for powers in ((0.0, -4.0, -0.5), (0.0, -7.0, -0.5)):
-        p1, p2, p3 = powers
-        A1 = edges[1] ** p1 / edges[1] ** p2
-        A2 = edges[2] ** p2 / edges[2] ** p3
-        out.append(_powerlaw(edges, powers, (1.0, A1, A2 * A1)))
-    return out
-
-
-def _mass_ratio_law(M_s, p2, F_twin):
-    """sample_q / sample_q_companion (priors.py:168-383)."""
-    p1 = 0.3
-    e2 = p2 + 1
-    if M_s >= 0.3:
-        q_lo = 0.1 if M_s >= 1.0 else 0.1 / M_s
-        A1 = (0.3 ** p1) / (0.3 ** p2)
-        A2 = (1 + F_twin / (1 - F_twin) * ((1.0 ** e2 - 0.3 ** e2) / e2)
-              / ((1.0 ** e2 - 0.95 ** e2) / e2))
-        return _powerlaw((q_lo, 0.3, 0.95, 1.0), (p1, p2, p2), (1.0, A1, A2 * A1))
-    if M_s > 0.1:
-        q_lo = 0.1 / M_s
-        A2 = (1 + F_twin / (1 - F_twin) * ((1.0 ** e2 - q_lo ** e2) / e2)
-              / ((1.0 ** e2 - 0.95 ** e2) / e2))
-        return _powerlaw((q_lo, 0.95, 1.0), (p2, p2), (1.0, A2))
-    return _constant(1.0)
 
 
 def _spline(spl, dev):
@@ -121,46 +85,18 @@ def _spline(spl, dev):
     return S
 
 
-def _bound_constants(M_s, plx, first_decade):
-    """Constants of lnprior_bound_TP / lnprior_bound_EB (priors.py:580-1005)."""
-    B = tri_bound_prior()
-    if np.isnan(plx):
-        plx = 0.1
-    B.d_pc = 1000 / plx
-    B.M_act = M_s
-    M = M_s if M_s >= 1.0 else 1.0
-    B.M_eff = M
-    lm = math.log10(M)
-    f1 = 0.020 + 0.04 * lm + 0.07 * lm ** 2
-    f2 = 0.039 + 0.07 * lm + 0.01 * lm ** 2
-    f3 = 0.078 - 0.05 * lm + 0.04 * lm ** 2
-    alpha, dlogP = 0.018, 0.7
-    slope = f2 - f1 - alpha * dlogP
-    slope2 = f3 - f2 - alpha * dlogP
-    B.f1, B.f2, B.f3, B.alpha, B.dlogP, B.slope, B.slope2 = f1, f2, f3, alpha, dlogP, slope, slope2
-    B.t2 = 0.5 * (2.0 * f1 + slope)
-    B.t3 = 0.5 * alpha * (3.4 ** 2 - 5.4 * 3.4 + 6.8) + f2 * (3.4 - 2.0)
-    B.t4 = (alpha * dlogP * (5.5 - 3.4) + f2 * (5.5 - 3.4)
-            + slope2 * (0.238095 * 5.5 ** 2 - 0.952381 * 5.5 + 0.485714))
-    B.t5 = f3 * (3.33333 - 17.3566 * math.exp(-0.3 * 8.0))
-    B.first_decade = int(first_decade)
-    return B
+def _bound_prior(M_s, plx, first_decade):
+    """tri_bound_prior of lnprior_bound_TP (first_decade False) / lnprior_bound_EB (True)."""
+    K = priors.bound_constants(M_s, plx)
+    return tri_bound_prior(
+        d_pc=K["d"], M_eff=K["M_s"], first_decade=int(first_decade),
+        **{n: K[n] for n in ("M_act", "f1", "f2", "f3", "alpha", "dlogP", "slope", "slope2", "t2",
+                             "t3", "t4", "t5")})
 
 
 def _ldc_tables(mission, Z, dev):
-    """_ldc.LdcGrid.at_Z_rounded as a dense (Teff, logg) table at the target's Z."""
-    def make():
-        grid = grid_for(mission)
-        at_Z = grid.Zs == grid.Zs[np.abs(grid.Zs - Z).argmin()]
-        T_at, g_at = grid.Teffs[at_Z], grid.loggs[at_Z]
-        tab1 = np.full((27, 4), np.nan)
-        tab2 = np.full((27, 4), np.nan)
-        it = ((T_at - 3500) // 250).astype(int)
-        ig = np.round((g_at - 3.5) / 0.5).astype(int)
-        tab1[it, ig] = grid.u1s[at_Z]
-        tab2[it, ig] = grid.u2s[at_Z]
-        return _t(tab1, dev), _t(tab2, dev)
-    return _cached(("ldc", mission, float(Z), str(dev)), make)
+    return _cached(("ldc", mission, float(Z), str(dev)),
+                   lambda: tuple(_t(tab, dev) for tab in grid_for(mission).dense_table(Z)))
 
 
 def _contrast(contrast_curve_file, dev):
@@ -175,18 +111,19 @@ def _contrast(contrast_curve_file, dev):
 
 
 class _Background:
-    """TRILEGAL population behind the target (e.g. :1452-1461), resident on the device."""
+    """marginal_likelihoods._Background (the TRILEGAL population behind the target), resident
+    on the device."""
 
     def __init__(self, trilegal_fname, Tmag, Jmag, Hmag, Kmag, mission, dev):
-        (Tm, masses, loggs, Teffs, Zs, Jm, Hm, Km) = trilegal_results(trilegal_fname, Tmag)
-        self.N_comp = int(Tm.shape[0])
-        delta = {"T": Tmag - Tm, "J": Jmag - Jm, "H": Hmag - Hm, "K": Kmag - Km}
-        self.mass, self.logg, self.teff = _t(masses, dev), _t(loggs, dev), _t(Teffs, dev)
-        self.radius = _t(np.sqrt(G * masses * Msun / 10 ** loggs) / Rsun, dev)
-        u1, u2 = grid_for(mission).nearest_each(Teffs, loggs, Zs)
+        pop = ml._Background(trilegal_fname, Tmag, Jmag, Hmag, Kmag)
+        self.N_comp = int(pop.N_comp)
+        self.mass, self.logg = _t(pop.masses, dev), _t(pop.loggs, dev)
+        self.teff = _t(pop.Teffs, dev)
+        self.radius = _t(pop.radii(), dev)
+        u1, u2 = grid_for(mission).nearest_each(pop.Teffs, pop.loggs, pop.Zs)
         self.u1, self.u2 = _t(u1, dev), _t(u2, dev)
-        self.dmag = {k: _t(v, dev) for k, v in delta.items()}
-        self.fr = {k: _t(10 ** (v / 2.5) / (1 + 10 ** (v / 2.5)), dev) for k, v in delta.items()}
+        self.dmag = {b: _t(pop.band(b), dev) for b in "TJHK"}
+        self.fr = {b: _t(pop.fluxratios_in(b), dev) for b in "TJHK"}
 
 
 def _background(trilegal_fname, mags, mission, dev):
@@ -200,13 +137,8 @@ def _band(filt):
 
 
 def _molusc(N, lo, hi, M_s, molusc_file, dev):
-    df = read_csv(molusc_file)
-    sma = df["semi-major axis(AU)"].values
-    e = df["eccentricity"].values
-    q = np.array(df[sma * (1 - e) > 10]["mass ratio"].values, dtype=float)
-    q[q < 0.1 / M_s] = 0.1 / M_s
     # padded to the TOTAL draw count, this rank takes its slice (as the host sampler does)
-    q = q[:N]
+    q = ml.molusc_q(M_s, molusc_file)[:N]
     return _t(np.pad(q, (0, N - len(q)))[lo:hi], dev)
 
 
@@ -244,9 +176,9 @@ def _sample(time, flux, sigma, exptime, nsamples, N, kind, host, diluter, P_orb,
     A.ecc_expo = 0.2 if P_mean <= 10 else 0.6
     A.M_s, A.R_s, A.Teff = float(M_s), float(R_s), float(Teff)
     A.u1, A.u2 = (float(u12[0]), float(u12[1])) if u12 is not None else (math.nan, math.nan)
-    A.rp_hi, A.rp_lo = _rp_laws()
-    A.q_pl = _mass_ratio_law(M_s, -0.5, 0.30)
-    A.qc_pl = _mass_ratio_law(M_s, -0.95, 0.05)
+    A.rp_hi, A.rp_lo = (_powerlaw(spec) for spec in priors.rp_specs())
+    A.q_pl = _powerlaw(priors.mass_ratio_spec(M_s, *priors.Q_LAW))
+    A.qc_pl = _powerlaw(priors.mass_ratio_spec(M_s, *priors.Q_COMPANION_LAW))
     keep = []
     A.hot_R, A.cool_R = _spline(funcs._hot_R, dev), _spline(funcs._cool_R, dev)
     A.hot_T, A.cool_T = _spline(funcs._hot_T, dev), _spline(funcs._cool_T, dev)
@@ -268,7 +200,7 @@ def _sample(time, flux, sigma, exptime, nsamples, N, kind, host, diluter, P_orb,
     A.prior_mode = 0
     if prior in ("bound_TP", "bound_EB") and molusc_file is None:
         A.prior_mode = 1
-        A.bound = _bound_constants(M_s, plx, prior == "bound_EB")
+        A.bound = _bound_prior(M_s, plx, prior == "bound_EB")
     elif prior == "background":
         A.prior_mode = 2
     if A.prior_mode:
@@ -288,10 +220,9 @@ def _sample(time, flux, sigma, exptime, nsamples, N, kind, host, diluter, P_orb,
         band = _band(filt)
         A.bg_dmag_cc = bg.dmag[band].data_ptr()
         A.bg_fr_cc = bg.fr[band].data_ptr()
-    # outputs: only the columns that are per-draw in this scenario
+    # outputs: only the columns that are per-draw in this scenario (and P, which is cheap; a
+    # fixed period reaches the engine as a scalar)
     want = {"body", "P", "inc", "ecc", "argp", "mtot"}
-    if type(P_orb) in [float, int]:
-        pass                                  # P is written anyway (cheap), passed as a scalar
     if kind == 1:
         want |= {"ebfr", "q", "meb"}
     if host != 0:
@@ -334,44 +265,21 @@ def _take_rows(columns, idx, dev):
     return out
 
 
-def _semi_major_axis(mtot, P):
-    return ((G * mtot * Msun) / (4 * pi ** 2) * (P * 86400) ** 2) ** (1 / 3)
-
-
-_KEYS = ('M_s', 'R_s', 'u1', 'u2', 'P_orb', 'inc', 'b', 'R_p', 'ecc', 'argp', 'M_EB', 'R_EB',
-         'fluxratio_EB', 'fluxratio_comp')
-
-
 def _table(lb, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, rps=None,
            masses=None, radii=None, fluxratios=None):
-    """This rank's half of a result dictionary (reference marginal_likelihoods.py:155-171): the
-    rows of its best local draws, registered for the merge across ranks (_finished)."""
+    """This rank's half of a result dictionary: the rows of its best local draws, registered
+    for the merge across ranks (_finished)."""
     idx = torch.as_tensor(np.asarray(lb.idx, dtype=np.int64), device=dev)
-    n = len(lb.idx)
-    got = _take_rows(dict(M_host=M_host, R_host=R_host, u1=u1, u2=u2, P=P, mtot=mtot, inc=incs,
-                          ecc=eccs, argp=argps, cfr=cfr, rps=rps, masses=masses, radii=radii,
-                          fluxratios=fluxratios), idx, dev)
-    P_i = got["P"] * (2 if twin else 1)
-    a_i = _semi_major_axis(got["mtot"], P_i)
-    ecc, argp, inc, Rh = got["ecc"], got["argp"], got["inc"], got["R_host"]
-    r = a_i * (1 - ecc ** 2) / (1 + ecc * np.sin(argp * np.pi / 180))
-    zeros = np.zeros(n)
-    local = {
-        'M_s': got["M_host"], 'R_s': Rh, 'u1': got["u1"], 'u2': got["u2"], 'P_orb': P_i,
-        'inc': inc, 'b': r * np.cos(inc * pi / 180) / (Rh * Rsun),
-        'R_p': got.get("rps", zeros), 'ecc': ecc, 'argp': argp,
-        'M_EB': got.get("masses", zeros), 'R_EB': got.get("radii", zeros),
-        'fluxratio_EB': got.get("fluxratios", zeros),
-        'fluxratio_comp': got["cfr"] if torch.is_tensor(cfr) else zeros,
-    }
-    return _dispatch.TableExchange(lb, local, _KEYS)
+    got = _take_rows(dict(M_s=M_host, R_s=R_host, u1=u1, u2=u2, P=P, mtot=mtot, inc=incs, ecc=eccs,
+                          argp=argps, R_p=rps, M_EB=masses, R_EB=radii, fluxratio_EB=fluxratios,
+                          fluxratio_comp=cfr if torch.is_tensor(cfr) else None), idx, dev)
+    return _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS)
 
 
 def _finished(exchange):
-    from .marginal_likelihoods import ScenarioResult
     lnZ, n_pass, n_eval, merged = exchange.result()
     merged['lnZ'] = lnZ
-    out = ScenarioResult(merged)
+    out = ml.ScenarioResult(merged)
     out.n_pass, out.n_evaluated = n_pass, n_eval
     return out
 
@@ -424,14 +332,10 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
             _dispatch.deliver(lambda: table(1), prepare))
 
 
-def _logg(M, R):
-    return math.log10(G * (M * Msun) / (R * Rsun) ** 2)
-
-
 # ------------------------------------------------------------------------------- scenarios
 def lnZ_TTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N=1000000, parallel=False,
             mission="TESS", flatpriors=False, exptime=0.00139, nsamples=20):
-    u12 = grid_for(mission).nearest(Z, Teff, _logg(M_s, R_s))
+    u12 = grid_for(mission).nearest(Z, Teff, ml._logg(M_s, R_s))
     s = _sample(time, flux, sigma, exptime, nsamples, int(N), 0, 0, 0, P_orb, M_s, R_s, Teff, u12,
                 flatpriors, mission)
     return _run(s, int(N), M_s, R_s, u12, False)
@@ -439,7 +343,7 @@ def lnZ_TTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N=1000000, parallel=Fal
 
 def lnZ_TEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N=1000000, parallel=False,
             mission="TESS", flatpriors=False, exptime=0.00139, nsamples=20):
-    u12 = grid_for(mission).nearest(Z, Teff, _logg(M_s, R_s))
+    u12 = grid_for(mission).nearest(Z, Teff, ml._logg(M_s, R_s))
     s = _sample(time, flux, sigma, exptime, nsamples, int(N), 1, 0, 0, P_orb, M_s, R_s, Teff, u12,
                 flatpriors, mission)
     return _run(s, int(N), M_s, R_s, u12, False, scalar_loop=not parallel)
@@ -448,7 +352,7 @@ def lnZ_TEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N=1000000, parallel=Fal
 def _bound(kind, host, prior, Teff_cap, time, flux, sigma, P_orb, M_s, R_s, Teff, Z, plx,
            contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples,
            molusc_file):
-    u12 = None if host == 1 else grid_for(mission).nearest(Z, Teff, _logg(M_s, R_s))
+    u12 = None if host == 1 else grid_for(mission).nearest(Z, Teff, ml._logg(M_s, R_s))
     s = _sample(time, flux, sigma, exptime, nsamples, int(N), kind, host, 1, P_orb, M_s, R_s,
                 Teff, u12, flatpriors, mission, Z=Z, Teff_cap=Teff_cap, prior=prior, plx=plx,
                 contrast_curve_file=contrast_curve_file, filt=filt, molusc_file=molusc_file)
@@ -492,7 +396,7 @@ def _behind(kind, host, time, flux, sigma, P_orb, M_s, R_s, Teff, Z, mags, trile
             contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples):
     dev = _device()
     bg = _background(trilegal_fname, mags, mission, dev)
-    u12 = None if host == 2 else grid_for(mission).nearest(Z, Teff, _logg(M_s, R_s))
+    u12 = None if host == 2 else grid_for(mission).nearest(Z, Teff, ml._logg(M_s, R_s))
     # randint upper bound N_comp - 1 in D*, N_comp in B* (:1463, :1672 vs :1926, :2139)
     idx_hi = bg.N_comp if host == 2 else bg.N_comp - 1
     s = _sample(time, flux, sigma, exptime, nsamples, int(N), kind, host, 2, P_orb, M_s, R_s,

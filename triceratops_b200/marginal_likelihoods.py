@@ -21,6 +21,8 @@ vs :406, :417-418), and a draw whose period-P transit probability exceeds 1 is s
 branches (marginal_likelihoods.py:316-319) -- and is reproduced by the engine's scalar_loop flag.
 TP-type scenarios give the same numbers either way.
 """
+import functools
+
 import numpy as np
 from pandas import read_csv
 
@@ -40,7 +42,22 @@ _SAMPLER = {"mode": "host"}
 def _sampler_mode():
     return _SAMPLER["mode"]
 
+
+def _device_sampler_twin(fn):
+    """In device-sampler mode the call goes, arguments unchanged, to the device_sampler function
+    of the same name (which takes the same parameters in the same order)."""
+    @functools.wraps(fn)
+    def call(*args, **kwargs):
+        if _sampler_mode() == "device":
+            from . import device_sampler
+            return getattr(device_sampler, fn.__name__)(*args, **kwargs)
+        return fn(*args, **kwargs)
+    return call
+
+
 N_SAMPLES = 100
+RESULT_KEYS = ('M_s', 'R_s', 'u1', 'u2', 'P_orb', 'inc', 'b', 'R_p', 'ecc', 'argp', 'M_EB', 'R_EB',
+               'fluxratio_EB', 'fluxratio_comp')
 
 __all__ = ["lnZ_TTP", "lnZ_TEB", "lnZ_PTP", "lnZ_PEB", "lnZ_STP", "lnZ_SEB", "lnZ_DTP",
            "lnZ_DEB", "lnZ_BTP", "lnZ_BEB",
@@ -73,14 +90,20 @@ def _logg(M, R):
     return np.log10(G * (M * Msun) / (R * Rsun) ** 2)
 
 
-def _semi_major_axis(mtot, P):
-    return ((G * mtot * Msun) / (4 * pi ** 2) * (P * 86400) ** 2) ** (1 / 3)
-
-
-def _impact(a, ecc, argp, inc, R_host):
-    """b of marginal_likelihoods.py:107-108 for the selected draws."""
+def result_table(n_zeros, twin, M_s, R_s, u1, u2, P, mtot, inc, ecc, argp, R_p=None, M_EB=None,
+                 R_EB=None, fluxratio_EB=None, fluxratio_comp=None):
+    """The reference's result dictionary (marginal_likelihoods.py:155-171, keys RESULT_KEYS)
+    from the rows of the best draws: the twin branch reports the doubled period, a and the
+    impact parameter b follow from the orbit, and a column the scenario does not have is
+    n_zeros zeros."""
+    P_orb = 2 * P if twin else P
+    a = ((G * mtot * Msun) / (4 * pi ** 2) * (P_orb * 86400) ** 2) ** (1 / 3)
     r = a * (1 - ecc ** 2) / (1 + ecc * np.sin(argp * np.pi / 180))
-    return r * np.cos(inc * pi / 180) / (R_host * Rsun)
+    b = r * np.cos(inc * pi / 180) / (R_s * Rsun)
+    given = dict(M_s=M_s, R_s=R_s, u1=u1, u2=u2, P_orb=P_orb, inc=inc, b=b, R_p=R_p, ecc=ecc,
+                 argp=argp, M_EB=M_EB, R_EB=R_EB, fluxratio_EB=fluxratio_EB,
+                 fluxratio_comp=fluxratio_comp)
+    return {k: np.zeros(n_zeros) if given[k] is None else given[k] for k in RESULT_KEYS}
 
 
 def _draw_ecc(N, planet, P_mean):
@@ -185,7 +208,9 @@ class _CompanionDraw:
     def finish(self, M_s):
         if self.molusc_file is None:
             return sample_q_companion(self.x, M_s)
-        return _companion_q(self.N, M_s, self.molusc_file)
+        q = molusc_q(M_s, self.molusc_file)
+        # zero-padded to N draws; a table with more than N rows raises, as in the reference
+        return np.pad(q, (0, self.N - len(q)))
 
     def column(self, M_s):
         """What a scenario's block gets per draw: the deviates (the block applies `transform`)
@@ -196,17 +221,16 @@ class _CompanionDraw:
         return sample_q_companion(col, M_s) if self.molusc_file is None else col
 
 
-def _companion_q(N, M_s, molusc_file):
-    """Mass ratios of bound companions: prior draws or a MOLUSC table (e.g. :455-464)."""
-    if molusc_file is None:
-        return sample_q_companion(_fastrng.rand(N), M_s)
+def molusc_q(M_s, molusc_file):
+    """Mass ratios of the bound companions a MOLUSC table lists with a(1 - e) > 10 AU, raised to
+    at least 0.1 / M_s (e.g. :455-464)."""
     df = read_csv(molusc_file)
     sma = df["semi-major axis(AU)"].values
     e = df["eccentricity"].values
     # copy: pandas >= 3 hands out read-only views (the reference assigns into .values)
     q = np.array(df[sma * (1 - e) > 10]["mass ratio"].values, dtype=float)
     q[q < 0.1 / M_s] = 0.1 / M_s
-    return np.pad(q, (0, N - len(q)))
+    return q
 
 
 def _fluxratio(masses, M_s, filt="TESS"):
@@ -275,46 +299,17 @@ class ScenarioResult(dict):
     n_evaluated = 0
 
 
-def _finish(br, table):
-    out = ScenarioResult(table)
+def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, **body):
+    """ScenarioResult of one branch: rows br.idx of the scenario's columns; `body` holds the
+    per-draw columns of the transiting body (R_p, or M_EB, R_EB and fluxratio_EB)."""
+    idx = br.idx
+    rows = {k: v[idx] for k, v in body.items()}
+    out = ScenarioResult(result_table(
+        N_SAMPLES, twin, _take(M_host, idx), _take(R_host, idx), _take(u1, idx), _take(u2, idx),
+        _take(P, idx), _take(mtot, idx), incs[idx], eccs[idx], argps[idx],
+        fluxratio_comp=_take(cfr, idx) if np.ndim(cfr) else None, **rows), lnZ=br.lnZ)
     out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
     return out
-
-
-def _tp_result(br, M_host, R_host, u1, u2, P, mtot, incs, rps, eccs, argps, cfr):
-    idx = br.idx
-    P_i = _take(P, idx)
-    a_i = _semi_major_axis(_take(mtot, idx), P_i)
-    zeros = np.zeros(N_SAMPLES)
-    return _finish(br, {
-        'M_s': _take(M_host, idx), 'R_s': _take(R_host, idx),
-        'u1': _take(u1, idx), 'u2': _take(u2, idx),
-        'P_orb': P_i, 'inc': incs[idx],
-        'b': _impact(a_i, eccs[idx], argps[idx], incs[idx], _take(R_host, idx)),
-        'R_p': rps[idx], 'ecc': eccs[idx], 'argp': argps[idx],
-        'M_EB': zeros, 'R_EB': zeros.copy(), 'fluxratio_EB': zeros.copy(),
-        'fluxratio_comp': _take(cfr, idx) if np.ndim(cfr) else zeros.copy(),
-        'lnZ': br.lnZ,
-    })
-
-
-def _eb_result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, masses, radii,
-               fluxratios, cfr):
-    idx = br.idx
-    P_i = _take(P, idx)
-    P_eff = 2 * P_i if twin else P_i
-    a_i = _semi_major_axis(_take(mtot, idx), P_eff)
-    zeros = np.zeros(N_SAMPLES)
-    return _finish(br, {
-        'M_s': _take(M_host, idx), 'R_s': _take(R_host, idx),
-        'u1': _take(u1, idx), 'u2': _take(u2, idx),
-        'P_orb': P_eff, 'inc': incs[idx],
-        'b': _impact(a_i, eccs[idx], argps[idx], incs[idx], _take(R_host, idx)),
-        'R_p': zeros, 'ecc': eccs[idx], 'argp': argps[idx],
-        'M_EB': masses[idx], 'R_EB': radii[idx], 'fluxratio_EB': fluxratios[idx],
-        'fluxratio_comp': _take(cfr, idx) if np.ndim(cfr) else zeros.copy(),
-        'lnZ': br.lnZ,
-    })
 
 
 def _run_tp(N, M_host, R_host, u1, u2, P, mtot, rps, incs, eccs, argps, cfr, lnprior,
@@ -322,8 +317,8 @@ def _run_tp(N, M_host, R_host, u1, u2, P, mtot, rps, incs, eccs, argps, cfr, lnp
     pb = _dispatch.submit_tp(N, rps, P, incs, eccs, argps, mtot, R_host, u1, u2, cfr,
                              lnprior=lnprior, extra_mask=extra_mask,
                              companion_is_host=companion_is_host)
-    return _dispatch.deliver(lambda: _tp_result(pb.finish(), M_host, R_host, u1, u2, P, mtot,
-                                                incs, rps, eccs, argps, cfr), pb.prepare)
+    return _dispatch.deliver(lambda: _result(pb.finish(), False, M_host, R_host, u1, u2, P, mtot,
+                                             incs, eccs, argps, cfr, R_p=rps), pb.prepare)
 
 
 def _run_eb(N, M_host, R_host, u1, u2, P, mtot, incs, qs, eccs, argps, masses, radii,
@@ -331,12 +326,16 @@ def _run_eb(N, M_host, R_host, u1, u2, P, mtot, incs, qs, eccs, argps, masses, r
     pb = _dispatch.submit_eb(N, radii, fluxratios, qs, P, incs, eccs, argps, mtot, R_host,
                              u1, u2, cfr, lnprior=lnprior, extra_mask=extra_mask,
                              companion_is_host=companion_is_host, scalar_loop=scalar_loop)
-    common = (M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, masses, radii, fluxratios, cfr)
-    return (_dispatch.deliver(lambda: _eb_result(pb.finish()[0], False, *common), pb.prepare),
-            _dispatch.deliver(lambda: _eb_result(pb.finish()[1], True, *common), pb.prepare))
+    common = (M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr)
+    body = dict(M_EB=masses, R_EB=radii, fluxratio_EB=fluxratios)
+    return (_dispatch.deliver(lambda: _result(pb.finish()[0], False, *common, **body),
+                              pb.prepare),
+            _dispatch.deliver(lambda: _result(pb.finish()[1], True, *common, **body),
+                              pb.prepare))
 
 
 # ------------------------------------------------------------------- target-star scenarios
+@_device_sampler_twin
 def lnZ_TTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, N: int = 1000000, parallel: bool = False,
@@ -344,9 +343,6 @@ def lnZ_TTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20):
     """Transiting planet on the target star (marginal_likelihoods.py:39-172).  Also used for a
     nearby star (NTP) by calc_probs."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_TTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -361,6 +357,7 @@ def _draw_binary(N, M_s, P_mean):
     return _BinaryDraws(N, P_mean).finish(M_s)
 
 
+@_device_sampler_twin
 def lnZ_TEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, N: int = 1000000, parallel: bool = False,
@@ -368,9 +365,6 @@ def lnZ_TEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20):
     """Eclipsing binary on the target star, periods P and 2P (marginal_likelihoods.py:175-383).
     Also used for a nearby star (NEB, NEBx2P) by calc_probs."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_TEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -393,6 +387,7 @@ def lnZ_TEB(time: np.ndarray, flux: np.ndarray, sigma: float,
 
 
 # ---------------------------------------------------------------- bound-companion scenarios
+@_device_sampler_twin
 def lnZ_PTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, plx: float, contrast_curve_file: str = None,
@@ -402,9 +397,6 @@ def lnZ_PTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20,
             molusc_file: str = None):
     """Planet on the target, diluted by an unresolved bound companion (:386-586)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_PTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, plx, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples, molusc_file)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -439,6 +431,7 @@ def lnZ_PTP(time: np.ndarray, flux: np.ndarray, sigma: float,
                    lnprior, extra, False)
 
 
+@_device_sampler_twin
 def lnZ_PEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, plx: float, contrast_curve_file: str = None,
@@ -448,9 +441,6 @@ def lnZ_PEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20,
             molusc_file: str = None):
     """EB on the target, diluted by an unresolved bound companion (:589-866)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_PEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, plx, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples, molusc_file)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -500,6 +490,7 @@ def _companion_stars(N, M_s, R_s, Teff, Z, mission, qs_comp, Teff_cap):
     return masses_comp, radii_comp, Teffs_comp, fluxratios_comp, u1s, u2s
 
 
+@_device_sampler_twin
 def lnZ_STP(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float, Z: float,
             plx: float, contrast_curve_file: str = None,
@@ -509,9 +500,6 @@ def lnZ_STP(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20,
             molusc_file: str = None):
     """Planet on an unresolved bound companion of the target (:869-1077)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_STP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, plx, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples, molusc_file)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -547,6 +535,7 @@ def lnZ_STP(time: np.ndarray, flux: np.ndarray, sigma: float,
                    argps, fluxratios_comp, lnprior, extra, True)
 
 
+@_device_sampler_twin
 def lnZ_SEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, plx: float, contrast_curve_file: str = None,
@@ -556,9 +545,6 @@ def lnZ_SEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             exptime: float = 0.00139, nsamples: int = 20,
             molusc_file: str = None):
     """EB on an unresolved bound companion of the target (:1080-1376)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_SEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, plx, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples, molusc_file)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -601,6 +587,7 @@ def lnZ_SEB(time: np.ndarray, flux: np.ndarray, sigma: float,
 
 
 # --------------------------------------------------------------------- background scenarios
+@_device_sampler_twin
 def lnZ_DTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, Tmag: float, Jmag: float, Hmag: float,
@@ -610,9 +597,6 @@ def lnZ_DTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             mission: str = "TESS", flatpriors: bool = False,
             exptime: float = 0.00139, nsamples: int = 20):
     """Planet on the target, diluted by a chance-aligned background star (:1379-1568)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_DTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, Tmag, Jmag, Hmag, Kmag, trilegal_fname, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -640,6 +624,7 @@ def lnZ_DTP(time: np.ndarray, flux: np.ndarray, sigma: float,
                    None, False)
 
 
+@_device_sampler_twin
 def lnZ_DEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Z: float, Tmag: float, Jmag: float, Hmag: float,
@@ -649,9 +634,6 @@ def lnZ_DEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             mission: str = "TESS", flatpriors: bool = False,
             exptime: float = 0.00139, nsamples: int = 20):
     """EB on the target, diluted by a chance-aligned background star (:1571-1837)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_DEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Z, Tmag, Jmag, Hmag, Kmag, trilegal_fname, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -683,6 +665,7 @@ def lnZ_DEB(time: np.ndarray, flux: np.ndarray, sigma: float,
                    fluxratios, cfr, lnprior, None, False, scalar_loop=not parallel)
 
 
+@_device_sampler_twin
 def lnZ_BTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Tmag: float, Jmag: float, Hmag: float, Kmag: float,
@@ -692,9 +675,6 @@ def lnZ_BTP(time: np.ndarray, flux: np.ndarray, sigma: float,
             mission: str = "TESS", flatpriors: bool = False,
             exptime: float = 0.00139, nsamples: int = 20):
     """Planet on a chance-aligned background star (:1840-2035)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_BTP(time, flux, sigma, P_orb, M_s, R_s, Teff, Tmag, Jmag, Hmag, Kmag, trilegal_fname, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -726,6 +706,7 @@ def lnZ_BTP(time: np.ndarray, flux: np.ndarray, sigma: float,
                    argps, cfr, lnprior, extra, True)
 
 
+@_device_sampler_twin
 def lnZ_BEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             P_orb: float, M_s: float, R_s: float, Teff: float,
             Tmag: float, Jmag: float, Hmag: float, Kmag: float,
@@ -735,9 +716,6 @@ def lnZ_BEB(time: np.ndarray, flux: np.ndarray, sigma: float,
             mission: str = "TESS", flatpriors: bool = False,
             exptime: float = 0.00139, nsamples: int = 20):
     """EB on a chance-aligned background star (:2038-2362)."""
-    if _sampler_mode() == "device":
-        from . import device_sampler
-        return device_sampler.lnZ_BEB(time, flux, sigma, P_orb, M_s, R_s, Teff, Tmag, Jmag, Hmag, Kmag, trilegal_fname, contrast_curve_file, filt, N, parallel, mission, flatpriors, exptime, nsamples)
     N = int(N)
     _dispatch.use_lightcurve(time, flux, sigma, exptime, nsamples)
     P, P_mean = _periods(P_orb, N)
@@ -813,13 +791,9 @@ class _PossibleHosts:
         self.u1s, self.u2s = grid_for(mission).nearest_each(self.Teffs, self.loggs, self.Zs)
 
 
-_EMPTY_KEYS = ('M_s', 'R_s', 'u1', 'u2', 'P_orb', 'inc', 'b', 'R_p', 'ecc', 'argp', 'M_EB',
-               'R_EB', 'fluxratio_EB', 'fluxratio_comp')
-
-
 def _no_hosts(with_b):
     # what the reference returns when no TRILEGAL star is similar enough (:2438-2454, :2648-2665)
-    res = {k: 0 for k in _EMPTY_KEYS if with_b or k != 'b'}
+    res = {k: 0 for k in RESULT_KEYS if with_b or k != 'b'}
     res['lnZ'] = -np.inf
     return res
 

@@ -24,17 +24,14 @@ from scipy.special import ndtr
 from . import _bufpool, _dispatch
 from ._numerics import _normalize_probabilities
 from .funcs import renorm_flux
-from .marginal_likelihoods import (lnZ_BEB, lnZ_BTP, lnZ_DEB, lnZ_DTP, lnZ_PEB, lnZ_PTP, lnZ_SEB,
-                                   lnZ_STP, lnZ_TEB, lnZ_TTP)
+from .marginal_likelihoods import (RESULT_KEYS, lnZ_BEB, lnZ_BTP, lnZ_DEB, lnZ_DTP, lnZ_PEB,
+                                   lnZ_PTP, lnZ_SEB, lnZ_STP, lnZ_TEB, lnZ_TTP)
 
 _STAR_COLUMNS = ("ID", "Tmag", "Jmag", "Hmag", "Kmag", "ra", "dec", "mass", "rad", "Teff", "plx",
                  "fluxratio", "tdepth")
 
 # scenario rows whose results may still be in flight while the next scenario is being drawn
 _PIPELINE_DEPTH = 3
-
-_RESULT_KEYS = ("M_s", "R_s", "u1", "u2", "P_orb", "inc", "b", "R_p", "ecc", "argp", "M_EB",
-                "R_EB", "fluxratio_EB", "fluxratio_comp")
 
 # (drop_scenario key, first row, star_num, scenario names) in the reference's order
 # (triceratops.py:784-1332)
@@ -153,7 +150,7 @@ class target:
         targets = np.zeros(n_rows, dtype=np.dtype("i8"))
         star_num = np.zeros(n_rows, dtype=np.dtype("i8"))
         scenarios = np.zeros(n_rows, dtype=np.dtype("U6"))
-        best = {k: np.zeros(n_rows) for k in _RESULT_KEYS}
+        best = {k: np.zeros(n_rows) for k in RESULT_KEYS}
         lnZ = np.zeros(n_rows)
 
         # Results are read a few scenarios after they were requested: the GPU works on one
@@ -177,7 +174,7 @@ class target:
         def fill(rows, parts):
             for j, res in zip(rows, parts):
                 res = _dispatch.resolve(res)
-                for k in _RESULT_KEYS:
+                for k in RESULT_KEYS:
                     best[k][j] = res[k][0]
                 lnZ[j] = res["lnZ"]
 
