@@ -122,6 +122,20 @@ int tri_set_lightcurve(const double* time, const double* flux, int64_t npts, dou
 int tri_set_lightcurve_err(const double* time, const double* flux, const double* flux_err,
                            int64_t npts, double exptime, int32_t nsamples);
 
+/* Mixed cadence (an extension: the reference passes one exposure time and one supersampling
+ * count, pytransit's QuadraticModel.set_data takes one per light curve): exptime[j] and
+ * nsamples[j] per time stamp.  The stamps are grouped by their distinct (exptime, nsamples)
+ * pairs, compared exactly; each group is modelled with its own exposure and sample count, and
+ * chi^2 is the sum over all stamps.  flux_err NULL: the scalar `sigma` as in tri_set_lightcurve,
+ * else one error per stamp as in tri_set_lightcurve_err (`sigma` is ignored).  The Gaussian
+ * constant, the secondary-eclipse pass and its depth cut do not depend on the cadence.  One
+ * distinct pair gives exactly the device state of the scalar calls.  TRI_EINVAL for an exptime
+ * that is not finite or < 0, nsamples < 1, or more than TRI_MAX_CADENCES distinct pairs. */
+#define TRI_MAX_CADENCES 8
+int tri_set_lightcurve_cadence(const double* time, const double* flux, const double* flux_err,
+                               double sigma, const double* exptime, const int32_t* nsamples,
+                               int64_t npts);
+
 /* L2 seam, host buffers: replaces the body of lnZ_* between the prior draws and _log_mean_exp. */
 int tri_eval_tp(const tri_tp_args* args, tri_result* out);
 int tri_eval_eb(const tri_eb_args* args, tri_result out[2]); /* [0]=EB, [1]=EBx2P */

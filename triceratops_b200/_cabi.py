@@ -15,6 +15,7 @@ c_uint8_p = ctypes.POINTER(ctypes.c_uint8)
 
 TRI_OK, TRI_ECUDA, TRI_EINVAL, TRI_ESTATE, TRI_ENODEVICE = 0, -1, -2, -3, -4
 TRI_MAX_INFLIGHT = 4     # include/triceratops_b200.h
+TRI_MAX_CADENCES = 8     # include/triceratops_b200.h
 
 
 class TriError(RuntimeError):
@@ -104,7 +105,7 @@ EXPORTS = ("tri_init", "tri_shutdown", "tri_last_error", "tri_set_lightcurve", "
            "tri_fetch_lnl", "tri_log_mean_exp", "tri_last_timing", "tri_fp64_peak", "tri_sm_count",
            "tri_submit_tp", "tri_submit_eb", "tri_submit_tp_dev", "tri_submit_eb_dev", "tri_wait",
            "tri_dev_splev", "tri_set_counting", "tri_set_lightcurve_err", "tri_dev_sample",
-           "tri_struct_sizes")
+           "tri_struct_sizes", "tri_set_lightcurve_cadence")
 
 _lib = None
 
@@ -133,6 +134,9 @@ def load():
                                      ctypes.c_double, ctypes.c_int32]
     L.tri_set_lightcurve_err.argtypes = [c_double_p, c_double_p, c_double_p, ctypes.c_int64,
                                          ctypes.c_double, ctypes.c_int32]
+    L.tri_set_lightcurve_cadence.argtypes = [c_double_p, c_double_p, c_double_p, ctypes.c_double,
+                                             c_double_p, ctypes.POINTER(ctypes.c_int32),
+                                             ctypes.c_int64]
     L.tri_eval_tp.argtypes = [ctypes.POINTER(tri_tp_args), ctypes.POINTER(tri_result)]
     L.tri_eval_eb.argtypes = [ctypes.POINTER(tri_eb_args), ctypes.POINTER(tri_result)]
     L.tri_eval_tp_dev.argtypes = [ctypes.POINTER(tri_tp_args), ctypes.POINTER(tri_result),

@@ -291,9 +291,11 @@ class CallGroup:
         with self.lock:
             seq = self.seq
             self.seq += 1
+            # (bytes: exptime and nsamples may be arrays, one value per stamp)
             key = None if lc is None else (
                 np.asarray(lc[0]).tobytes(), np.asarray(lc[1]).tobytes(),
-                np.asarray(lc[2], dtype=np.float64).tobytes()) + tuple(lc[3:])
+                np.asarray(lc[2], dtype=np.float64).tobytes(),
+                np.asarray(lc[3], dtype=np.float64).tobytes(), np.asarray(lc[4]).tobytes())
             send_lc = lc if key != self.lc_key else None
             self.lc_key = key
             hdr = dict(op="call", seq=seq, kind=kind, N=N, arrays=arrays, scalars=scalars,

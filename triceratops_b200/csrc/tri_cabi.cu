@@ -187,6 +187,7 @@ struct Ctx {
     int* d_perm = nullptr;   // sorted stamp -> caller's stamp
     size_t lc_cap = 0;
     LightCurve lc{};
+    CadenceTable cad{};   // n > 1: mixed cadence (lnl_seg_kernel), else n == 1
     Slot slots[kSlots + 1];
     int64_t next_ticket = 1;
     Slot* last = nullptr;    // the call completed last (tri_last_timing, tri_fetch_lnl)
@@ -284,7 +285,11 @@ void finish_result(const LsePartial& r, int64_t N, tri_result* out) {
 
 int launch_lnl(Slot& S, LnlArgs& A, cudaStream_t s) {
     size_t smem = lnl_smem_bytes();
-    if (g.count_work) lnl_kernel<true><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
+    if (g.cad.n > 1) {   // mixed cadence: the segmented instantiation
+        A.cad = g.cad;
+        if (g.count_work) lnl_seg_kernel<true><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
+        else lnl_seg_kernel<false><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
+    } else if (g.count_work) lnl_kernel<true><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
     else lnl_kernel<false><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
     S.launches += 1;
     CU(cudaGetLastError());
@@ -689,8 +694,12 @@ int tri_sm_count(int32_t* n) {
     return TRI_OK;
 }
 
+// `grp` (mixed cadence, tri_set_lightcurve_cadence): cadence group of every stamp, whose
+// exposure and sample count `groups` holds (groups->n >= 2); exptime / nsamples are then the
+// largest of the groups.  nullptr: one cadence (exptime, nsamples).
 static int set_lightcurve(const double* time, const double* flux, const double* err,
-                          int64_t npts, double sigma, double exptime, int32_t nsamples) {
+                          int64_t npts, double sigma, double exptime, int32_t nsamples,
+                          const int* grp = nullptr, const CadenceTable* groups = nullptr) {
     int rc = need_ready(false);
     if (rc) return rc;
     if (!time || !flux || npts <= 0) return fail(TRI_EINVAL, "empty light curve");
@@ -712,8 +721,13 @@ static int set_lightcurve(const double* time, const double* flux, const double* 
     // chi^2 is a plain sum over stamps, so the stamps may be visited in time order
     std::vector<int64_t> order(npts);
     std::iota(order.begin(), order.end(), 0);
-    std::stable_sort(order.begin(), order.end(),
-                     [&](int64_t x, int64_t y) { return time[x] < time[y]; });
+    if (grp)   // (group, time): each group is one contiguous, time-sorted slice
+        std::stable_sort(order.begin(), order.end(), [&](int64_t x, int64_t y) {
+            return grp[x] < grp[y] || (grp[x] == grp[y] && time[x] < time[y]);
+        });
+    else
+        std::stable_sort(order.begin(), order.end(),
+                         [&](int64_t x, int64_t y) { return time[x] < time[y]; });
     std::vector<double> t(npts), f(npts), pre(npts + 1), wgt(err ? npts : 0);
     long double run = 0.0L;
     pre[0] = 0.0;
@@ -760,14 +774,31 @@ static int set_lightcurve(const double* time, const double* flux, const double* 
     g.lc.weight = err ? g.d_weight : nullptr;
     g.lc.npts = (int)npts; g.lc.nsamples = nsamples; g.lc.sigma = sigma; g.lc.exptime = exptime;
     g.lc.tmin = t.front(); g.lc.tmax = t.back();
-    // stage the light curve in shared memory only when that costs no occupancy
+    g.cad = CadenceTable{};
+    g.cad.n = 1;
+    if (grp) {
+        g.cad = *groups;
+        g.lc.tmin = *std::min_element(t.begin(), t.end());
+        g.lc.tmax = *std::max_element(t.begin(), t.end());
+        int j = 0;
+        for (int c = 0; c < g.cad.n; ++c) {
+            g.cad.off[c] = j;
+            while (j < npts && grp[order[j]] == c) ++j;
+            g.cad.tmin[c] = t[g.cad.off[c]];
+            g.cad.tmax[c] = t[j - 1];
+        }
+        g.cad.off[g.cad.n] = j;
+    }
+    // stage the light curve in shared memory only when that costs no occupancy (of the
+    // instantiation that will run)
     {
+        void (*kern)(LnlArgs) = g.cad.n > 1 ? lnl_seg_kernel<false> : lnl_kernel<false>;
         int bps0 = 0, bps1 = 0;
         size_t need = (size_t)(3 * (size_t)npts + 1) * sizeof(double);
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps0, lnl_kernel<false>, kLnlThreads, 0));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps0, kern, kLnlThreads, 0));
         g.lnl_smem = 0;
         if (need <= 48 * 1024) {
-            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps1, lnl_kernel<false>, kLnlThreads, need));
+            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps1, kern, kLnlThreads, need));
             if (bps1 >= bps0) g.lnl_smem = need;
         }
         g.lnl_blocks_per_sm = std::max(1, bps0);
@@ -785,6 +816,53 @@ int tri_set_lightcurve_err(const double* time, const double* flux, const double*
                            int64_t npts, double exptime, int32_t nsamples) {
     if (!flux_err) return fail(TRI_EINVAL, "flux_err is NULL");
     return set_lightcurve(time, flux, flux_err, npts, 0.0, exptime, nsamples);
+}
+
+static_assert(kMaxCadences == TRI_MAX_CADENCES, "cadence table size");
+
+int tri_set_lightcurve_cadence(const double* time, const double* flux, const double* flux_err,
+                               double sigma, const double* exptime, const int32_t* nsamples,
+                               int64_t npts) {
+    int rc = need_ready(false);
+    if (rc) return rc;
+    if (!time || !flux || npts <= 0) return fail(TRI_EINVAL, "empty light curve");
+    if (!exptime || !nsamples) return fail(TRI_EINVAL, "exptime or nsamples is NULL");
+    if (npts > (int64_t)1 << 28) return fail(TRI_EINVAL, "light curve too long");
+    // distinct (exptime, nsamples) pairs, compared exactly
+    std::vector<std::pair<double, int32_t>> pairs;
+    for (int64_t j = 0; j < npts; j++) {
+        const double e = exptime[j];
+        const int32_t n = nsamples[j];
+        if (!std::isfinite(e) || e < 0.0)
+            return fail(TRI_EINVAL, "exptime must be finite and >= 0 at every stamp");
+        if (n < 1) return fail(TRI_EINVAL, "nsamples must be >= 1 at every stamp");
+        const std::pair<double, int32_t> pr(e, n);
+        if (std::find(pairs.begin(), pairs.end(), pr) != pairs.end()) continue;
+        if ((int)pairs.size() == TRI_MAX_CADENCES)
+            return fail(TRI_EINVAL, "more than TRI_MAX_CADENCES distinct (exptime, nsamples) "
+                                    "pairs: round the exposure times to their cadences");
+        pairs.push_back(pr);
+    }
+    const double sig = flux_err ? 0.0 : sigma;
+    if (pairs.size() == 1)   // one cadence: exactly the scalar calls
+        return set_lightcurve(time, flux, flux_err, npts, sig, pairs[0].first, pairs[0].second);
+    std::sort(pairs.begin(), pairs.end());
+    CadenceTable cad{};
+    cad.n = (int)pairs.size();
+    double emax = 0.0;
+    int32_t nmax = 1;
+    for (int c = 0; c < cad.n; ++c) {
+        cad.exptime[c] = pairs[c].first;
+        cad.nsamples[c] = pairs[c].second;
+        emax = std::max(emax, pairs[c].first);
+        nmax = std::max(nmax, pairs[c].second);
+    }
+    std::vector<int> grp(npts);
+    for (int64_t j = 0; j < npts; j++)
+        grp[j] = (int)(std::find(pairs.begin(), pairs.end(),
+                                 std::pair<double, int32_t>(exptime[j], nsamples[j]))
+                       - pairs.begin());
+    return set_lightcurve(time, flux, flux_err, npts, sig, emax, nmax, grp.data(), &cad);
 }
 
 // ---- submit / wait --------------------------------------------------------------------------

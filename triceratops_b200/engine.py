@@ -32,6 +32,37 @@ def get_engine(device=None):
     return _engine
 
 
+def cadence_columns(exptime, nsamples, npts):
+    """Check the cadence of a light curve of `npts` stamps: `exptime` and `nsamples` are each a
+    scalar or one value per stamp.  Returns (exptime, nsamples) as a float and an int when they
+    hold one (exptime, nsamples) pair, else as a float64 and an int32 array of npts values (at
+    most TRI_MAX_CADENCES distinct pairs, compared exactly).  Raises ValueError."""
+    e = np.asarray(exptime)
+    n = np.asarray(nsamples)
+    for name, x in (("exptime", e), ("nsamples", n)):
+        if x.ndim > 1 or (x.ndim == 1 and x.size != npts):
+            raise ValueError("%s has shape %s; the light curve has %d time stamps"
+                             % (name, x.shape, npts))
+        if x.dtype.kind not in "biuf":
+            raise ValueError("%s must be numeric" % name)
+    e = np.broadcast_to(e.astype(np.float64), (npts,))
+    if not np.all(np.isfinite(e)) or np.any(e < 0):
+        raise ValueError("exptime must be finite and >= 0 at every stamp")
+    if n.dtype.kind == "f" and not np.all(np.isfinite(n) & (n == np.floor(n))):
+        raise ValueError("nsamples must be integral")
+    if np.any(n < 1) or np.any(n > np.iinfo(np.int32).max):
+        raise ValueError("nsamples must be >= 1 at every stamp")
+    n = np.broadcast_to(n.astype(np.int32), (npts,))
+    pairs = np.unique(np.stack([e, n.astype(np.float64)]), axis=1)
+    if pairs.shape[1] > _cabi.TRI_MAX_CADENCES:
+        raise ValueError("%d distinct (exptime, nsamples) pairs, at most %d are supported: round "
+                         "the exposure times to their cadences"
+                         % (pairs.shape[1], _cabi.TRI_MAX_CADENCES))
+    if pairs.shape[1] == 1:
+        return float(e[0]), int(n[0])
+    return np.ascontiguousarray(e), np.ascontiguousarray(n)
+
+
 class BranchResult:
     """One scenario branch: lnZ pieces + optional per-draw arrays."""
     __slots__ = ("lnZ", "m", "s", "n_finite", "n_posinf", "n_pass", "n_stamps", "n_interior",
@@ -146,11 +177,32 @@ class Engine:
     # ------------------------------------------------------------------ light curve
     @_locked
     def set_lightcurve(self, time, flux, sigma, exptime, nsamples):
+        """Make (time, flux, sigma, exptime, nsamples) the current light curve.  sigma: a scalar
+        or one error per stamp (tri_set_lightcurve_err); exptime and nsamples: scalars or one
+        value per stamp, for a light curve that mixes cadences (tri_set_lightcurve_cadence, see
+        cadence_columns).  Per-stamp cadences that hold one pair are the scalar call."""
         time = _cabi.f64(time)
         flux = _cabi.f64(flux)
         if time.shape != flux.shape or time.ndim != 1:
             raise ValueError("time and flux must be 1-D arrays of equal length")
-        if np.ndim(sigma) == 0:
+        if np.ndim(exptime) != 0 or np.ndim(nsamples) != 0:
+            exptime, nsamples = cadence_columns(exptime, nsamples, time.size)
+        if np.ndim(exptime) != 0:   # several cadences (tri_set_lightcurve_cadence)
+            err = None
+            if np.ndim(sigma) != 0:
+                err = _cabi.f64(sigma)
+                if err.shape != time.shape:
+                    raise ValueError("per-point errors must have the shape of time")
+            key = (time.tobytes(), flux.tobytes(),
+                   err.tobytes() if err is not None else np.float64(sigma).tobytes(),
+                   exptime.tobytes(), nsamples.tobytes())
+            if key == self._lc_key:
+                return
+            _cabi.check(self.lib.tri_set_lightcurve_cadence(
+                _cabi.dptr(time), _cabi.dptr(flux), _cabi.dptr(err) if err is not None else None,
+                float(sigma) if err is None else 0.0, _cabi.dptr(exptime),
+                nsamples.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), time.size))
+        elif np.ndim(sigma) == 0:
             key = (time.tobytes(), flux.tobytes(), float(sigma), float(exptime), int(nsamples))
             if key == self._lc_key:
                 return

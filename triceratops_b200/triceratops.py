@@ -137,7 +137,16 @@ class target:
                    verbose: int = 1, flatpriors: bool = False,
                    exptime: float = 0.00139, nsamples: int = 20,
                    molusc_file: str = None):
-        """Relative probability of every scenario, FPP and NFPP (triceratops.py:673-1485)."""
+        """Relative probability of every scenario, FPP and NFPP (triceratops.py:673-1485).
+
+        Extensions of the reference's arguments: `flux_err_0` may hold one error per time stamp
+        (chi^2 is then weighted per point; the Gaussian constant and the secondary-depth cut use
+        their mean), and `exptime` and `nsamples` may each hold one value per time stamp, for a
+        light curve that mixes cadences (e.g. 30-min and 200-s TESS FFIs with 2-min target
+        pixels).  The stamps are then modelled in groups of equal (exptime, nsamples), at most
+        TRI_MAX_CADENCES = 8 of them, each with its own integration time and supersampling.
+        Per-stamp arrays lose the rows whose time or flux is NaN, like time and flux."""
+        n_in = np.size(time)
         keep = ~np.isnan(time) & ~np.isnan(flux_0)
         time = time[keep]
         flux_0 = flux_0[keep]
@@ -145,6 +154,18 @@ class target:
             # an error per time stamp (an extension of the reference's scalar flux_err_0, see
             # tri_set_lightcurve_err): chi^2 is weighted per point, the scalar formulas use the mean
             flux_err_0 = np.asarray(flux_err_0, dtype=float)[keep]
+        if np.ndim(exptime) != 0 or np.ndim(nsamples) != 0:
+            # per-stamp cadence (tri_set_lightcurve_cadence)
+            cad = []
+            for name, x in (("exptime", exptime), ("nsamples", nsamples)):
+                if np.ndim(x) != 0:
+                    x = np.asarray(x)
+                    if x.shape != (n_in,):
+                        raise ValueError("%s has shape %s; the light curve has %d time stamps"
+                                         % (name, x.shape, n_in))
+                    x = x[keep]
+                cad.append(x)
+            exptime, nsamples = cad
         filtered = self.stars[self.stars["tdepth"] > 0]
         n_rows = 3 * len(filtered) + 12
         targets = np.zeros(n_rows, dtype=np.dtype("i8"))
