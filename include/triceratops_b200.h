@@ -205,8 +205,8 @@ int tri_log_mean_exp(const double* logw, int64_t n, tri_result* out);
 
 /* Device time [ms] of the kernels of the most recent eval/lnl call, from CUDA events on the
  * stream they ran on: geometry, light-curve/chi^2 (with the fused evidence epilogue), the
- * finalize kernel (merge of the block records + best-draw selection), and their launch count
- * (3 per evaluation). */
+ * finalize kernel (merge of the block records + best-draw selection; with tri_set_moments on,
+ * also the moments kernel), and their launch count (3 per evaluation, 4 with moments). */
 int tri_last_timing(double* geometry_ms, double* lnl_ms, double* lse_ms, int32_t* launches);
 
 /* Device-side prior sampler support (opt-in mode, triceratops_b200.set_sampler("device")):
@@ -292,6 +292,18 @@ int tri_fp64_peak(double* dfma_per_s);
  * roofline model -- n_stamps, n_interior, n_limb of tri_result -- in the hot loop (about 1.5 %
  * slower); when off those three fields are 0.  bench.py turns it on for one untimed pass. */
 int tri_set_counting(int32_t on);
+
+/* Second moment of the importance weights (off by default; captured per submission, like
+ * tri_set_counting).  When on, every evaluation also runs one short kernel after the evidence
+ * merge that sums s2 = sum over the finite ln-weights x of exp(2 (x - m)) per branch, with x =
+ * lnL + lnprior formed as for lnZ and m the branch's record.  From (N, m, s, s2) follow the
+ * standard error of lnZ and the effective sample size (triceratops_b200._numerics). */
+int tri_set_moments(int32_t on);
+
+/* s2 of branch 0 (and 1 for an EB-type call) of the evaluation most recently returned by
+ * tri_eval_* / tri_eval_*_dev / tri_wait; NaN where moments were off for it (and for s2[1] of a
+ * TP-type call).  A submission keeps its s2 until it is waited for. */
+int tri_last_moments(double s2[2]);
 
 /* sizeof() of the ABI structs, in the order tri_col, tri_tp_args, tri_eb_args, tri_result,
  * tri_powerlaw, tri_spline, tri_bound_prior, tri_sampler_args (the first n of them), so that a

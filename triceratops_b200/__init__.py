@@ -60,6 +60,15 @@ def unpatch():
         setattr(mod, name, fn)
 
 
+def mc_errors():
+    """Context manager: lnZ_* calls made inside it also return the Monte-Carlo error of their
+    evidence -- attributes N, s2, lnZ_err and ess of each result (marginal_likelihoods.
+    ScenarioResult).  The GPU then runs one extra short kernel per evaluation; lnZ and the
+    best-draw tables are the same bits as without it.  calc_probs(mc_errors=True) uses it."""
+    from . import _dispatch
+    return _dispatch.mc_errors()
+
+
 def set_sampler(mode="host", seed=None):
     """Where the prior draws are made.
 

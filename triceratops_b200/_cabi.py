@@ -105,7 +105,8 @@ EXPORTS = ("tri_init", "tri_shutdown", "tri_last_error", "tri_set_lightcurve", "
            "tri_fetch_lnl", "tri_log_mean_exp", "tri_last_timing", "tri_fp64_peak", "tri_sm_count",
            "tri_submit_tp", "tri_submit_eb", "tri_submit_tp_dev", "tri_submit_eb_dev", "tri_wait",
            "tri_dev_splev", "tri_set_counting", "tri_set_lightcurve_err", "tri_dev_sample",
-           "tri_struct_sizes", "tri_set_lightcurve_cadence")
+           "tri_struct_sizes", "tri_set_lightcurve_cadence", "tri_set_moments",
+           "tri_last_moments")
 
 _lib = None
 
@@ -166,6 +167,8 @@ def load():
                                   ctypes.POINTER(ctypes.c_int32)]
     L.tri_fp64_peak.argtypes = [c_double_p]
     L.tri_set_counting.argtypes = [ctypes.c_int32]
+    L.tri_set_moments.argtypes = [ctypes.c_int32]
+    L.tri_last_moments.argtypes = [c_double_p]
     L.tri_dev_sample.argtypes = [ctypes.POINTER(tri_sampler_args), ctypes.c_void_p]
     L.tri_struct_sizes.argtypes = [ctypes.POINTER(ctypes.c_int64), ctypes.c_int32]
     L.tri_sm_count.argtypes = [ctypes.POINTER(ctypes.c_int32)]

@@ -4,7 +4,7 @@ ranks (one process per GPU), the single small collective that merges the per-ran
 (reference marginal_likelihoods.py:152-154).
 
 Sharding follows SURVEY.md section 8e: rank r evaluates the contiguous slice
-[r*N/G, (r+1)*N/G) of every scenario's draws and contributes one 206-double record per scenario
+[r*N/G, (r+1)*N/G) of every scenario's draws and contributes one 207-double record per scenario
 branch -- (m, s, counts) + its 100 best (lnL, global index) candidates; no per-draw data is
 exchanged.
 
@@ -100,9 +100,35 @@ def best_indices(lnL, n_best=N_BEST):
     return cand[order][:n_best]
 
 
+# ---- Monte-Carlo error bars (tri_set_moments) ----------------------------------------------------
+_moments = 0      # > 0 inside mc_errors(): engine calls also return s2 (process-wide)
+
+
+@contextlib.contextmanager
+def mc_errors():
+    """Inside this context the engine also sums the second moment of the weights of every
+    scenario branch, and the lnZ_* results carry N, s2, lnZ_err and ess (ScenarioResult)."""
+    global _moments
+    _moments += 1
+    try:
+        yield
+    finally:
+        _moments -= 1
+
+
+def _sync_moments(eng):
+    """Switch the engine's moment pass to what the caller's context asks for (engines without
+    one -- test stand-ins -- are left alone while moments are off)."""
+    want = _moments > 0
+    if want or getattr(eng, "_moments", False):
+        eng.set_moments(want)
+
+
 class Branch:
-    """Globally combined result of one scenario branch."""
-    __slots__ = ("lnZ", "idx", "n_pass", "n_evaluated", "lnL_local", "lo", "hi")
+    """Globally combined result of one scenario branch: lnZ, its (m, s, s2, n_finite, n_posinf)
+    record (s2 None without moments), the best draws' indices and finite lnL values."""
+    __slots__ = ("lnZ", "idx", "n_pass", "n_evaluated", "lnL_local", "lo", "hi", "N", "m", "s",
+                 "s2", "n_finite", "n_posinf", "vals")
 
 
 def _local_best(res, eng, single_rank):
@@ -126,7 +152,7 @@ def _local_best(res, eng, single_rank):
     return idx, res.lnL[idx], int(np.isfinite(res.lnL).sum())
 
 
-H = 6   # header of a branch record: m, s, n_finite, n_posinf, n_pass, n_evaluated
+H = 7   # header of a branch record: m, s, n_finite, n_posinf, n_pass, n_evaluated, s2
 
 
 def _allgather(mat, d):
@@ -151,34 +177,46 @@ def gather_records(records, N_total):
                                     N_total) for j in range(len(records))]
 
 
-def _local_record(res, lo, eng):
-    """This rank's 206-double record of one branch (zero-weight padding is not exchanged)."""
-    local_best, local_vals, n_eval = _local_best(res, eng, False)
+def record_row(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals):
+    """The 207-double record of a branch over one slice of draws (a rank's, or a round's of
+    refinement): header, then its best finite (lnL, global index) candidates; s2 None -> NaN."""
     rec = np.full(H + 2 * N_BEST, np.nan)
-    rec[0:H] = (res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval)
-    local_best, local_vals = np.asarray(local_best), np.asarray(local_vals)
-    fin = np.isfinite(local_vals)
-    local_best, local_vals = local_best[fin], local_vals[fin]
-    k = local_best.size
-    rec[H:H + k] = local_vals
-    rec[H + N_BEST:H + N_BEST + k] = (local_best + lo).astype(np.float64)
+    rec[0:H] = (m, s, n_finite, n_posinf, n_pass, n_eval, np.nan if s2 is None else s2)
+    idx, vals = np.asarray(idx), np.asarray(vals)
+    fin = np.isfinite(vals)
+    idx, vals = idx[fin], vals[fin]
+    k = idx.size
+    rec[H:H + k] = vals
+    rec[H + N_BEST:H + N_BEST + k] = idx.astype(np.float64)
     return rec
 
 
+def _local_record(res, lo, eng):
+    """This rank's record of one branch (zero-weight padding is not exchanged)."""
+    local_best, local_vals, n_eval = _local_best(res, eng, False)
+    return record_row(res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval,
+                      getattr(res, "s2", None), np.asarray(local_best) + lo, local_vals)
+
+
 def _merge_records(allrec, lo, hi, N, lnL_local=None):
-    """[world, 206] -> Branch: lnZ from the (m, s) records, best draws from the candidates."""
+    """[slices, 207] -> Branch: lnZ from the (m, s) records, best draws from the candidates.
+    The slices are ranks, or rounds of refinement (calc_probs)."""
     br = Branch()
-    br.lo, br.hi, br.lnL_local = lo, hi, lnL_local
+    br.lo, br.hi, br.lnL_local, br.N = lo, hi, lnL_local, N
     parts = [(r[0], r[1], int(r[2]), int(r[3])) for r in allrec]
     br.lnZ = _engine_mod.combine_lse(parts, N)
     br.n_pass = int(sum(r[4] for r in allrec))
     br.n_evaluated = int(sum(r[5] for r in allrec))
+    br.m, br.s, s2, br.n_finite, br.n_posinf = _engine_mod.combine_moments(
+        [(r[0], r[1], r[6], r[2], r[3]) for r in allrec])
+    br.s2 = None if np.isnan(allrec[:, 6]).any() else s2
     vals = allrec[:, H:H + N_BEST].ravel()
     gidx = allrec[:, H + N_BEST:H + 2 * N_BEST].ravel()
     ok = ~np.isnan(gidx)
     vals, gidx = vals[ok], gidx[ok].astype(np.int64)
     order = np.lexsort((gidx, -vals))
     idx = gidx[order][:N_BEST]
+    br.vals = vals[order][:N_BEST]
     want = min(N_BEST, N)
     if idx.size < want:
         # fewer finite draws than table rows: the reference fills the table with zero-weight
@@ -196,9 +234,12 @@ def _gather_branch(res, lo, hi, N, eng=None):
     d = _dist()
     if d is None:
         br = Branch()
-        br.lo, br.hi, br.lnL_local = lo, hi, res.lnL
-        br.idx, _, br.n_evaluated = _local_best(res, eng, True)
+        br.lo, br.hi, br.lnL_local, br.N = lo, hi, res.lnL, N
+        br.idx, vals, br.n_evaluated = _local_best(res, eng, True)
+        br.vals = np.asarray(vals)[np.isfinite(vals)]
         br.lnZ, br.n_pass = res.lnZ, res.n_pass
+        br.m, br.s, br.n_finite, br.n_posinf = res.m, res.s, res.n_finite, res.n_posinf
+        br.s2 = getattr(res, "s2", None)
         return br
     rec = _local_record(res, lo, eng)
     return _merge_records(_allgather(rec[None, :], d)[:, 0, :], lo, hi, N, res.lnL)
@@ -267,6 +308,7 @@ class CallGroup:
         kw = dict(extra_mask=mask, companion_is_host=hdr["is_host"], n_best=N_BEST)
         if hdr["scalar_loop"]:
             kw["scalar_loop"] = True
+        _sync_moments(eng)
         fn = getattr(eng, "submit_" + name, None)
         if fn is not None:
             return fn(n, cols, lightcurve=lc, **kw)
@@ -408,6 +450,7 @@ class _Done:
 
 def _submit(eng, name, *args, **kw):
     lc = current_lightcurve()
+    _sync_moments(eng)
     fn = getattr(eng, "submit_" + name, None)
     if fn is not None:
         return fn(*args, lightcurve=lc, **kw)
@@ -643,24 +686,32 @@ class TableExchange:
         self.rows = np.stack([np.asarray(table[k], dtype=np.float64) for k in keys], axis=1) \
             if len(lb.idx) else np.zeros((0, len(keys)))
         self.group, self.key = _group if _dist() is not None else None, None
+        self.s2 = getattr(res, "s2", None)
         if _dist() is not None:
-            W = 6 + N_BEST * (1 + len(keys))
+            W = H + N_BEST * (1 + len(keys))
             rec = np.full(W, np.nan)
-            rec[0:6] = (res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, self.n_eval)
+            rec[0:H] = (res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, self.n_eval,
+                        np.nan if self.s2 is None else self.s2)
             k = len(lb.vals)
-            rec[6:6 + k] = lb.vals
-            rec[6 + N_BEST:6 + N_BEST + k * len(keys)] = self.rows.ravel()
+            rec[H:H + k] = lb.vals
+            rec[H + N_BEST:H + N_BEST + k * len(keys)] = self.rows.ravel()
             self.rec = rec
             if self.group is not None:
                 self.key = self.group.add(rec)
 
     def result(self):
-        """(lnZ, n_pass, n_evaluated, merged table padded to N_BEST rows)."""
+        """(lnZ, n_pass, n_evaluated, merged table padded to N_BEST rows).  Also sets
+        `record` = (m, s, s2, n_finite, n_posinf) of the whole branch (s2 None without
+        moments) and, on one rank, `top` = (lnL, draw index) of the table's finite rows."""
         lb, keys, res = self.lb, self.keys, self.lb.res
         vals, rows, n_eval = lb.vals, self.rows, self.n_eval
         d = _dist()
+        self.top = None
         if d is None:
             lnZ, n_pass = res.lnZ, int(res.n_pass)
+            self.record = (res.m, res.s, self.s2, res.n_finite, res.n_posinf)
+            order = np.argsort(-vals, kind="stable")[:N_BEST]
+            self.top = (vals[order], np.asarray(lb.idx)[order])
         else:
             allrec = (self.group.rows(self.key) if self.group is not None
                       else _allgather(self.rec[None, :], d)[:, 0, :])
@@ -668,12 +719,15 @@ class TableExchange:
                                           lb.N)
             n_pass = int(sum(r[4] for r in allrec))
             n_eval = int(sum(r[5] for r in allrec))
+            m, s, s2, n_fin, n_pinf = _engine_mod.combine_moments(
+                [(r[0], r[1], r[6], r[2], r[3]) for r in allrec])
+            self.record = (m, s, None if np.isnan(allrec[:, 6]).any() else s2, n_fin, n_pinf)
             vs, rs = [], []
             for r in allrec:
-                v = r[6:6 + N_BEST]
+                v = r[H:H + N_BEST]
                 ok = ~np.isnan(v)
                 vs.append(v[ok])
-                rs.append(r[6 + N_BEST:6 + N_BEST + int(ok.sum()) * len(keys)]
+                rs.append(r[H + N_BEST:H + N_BEST + int(ok.sum()) * len(keys)]
                           .reshape(-1, len(keys)))
             vals, rows = np.concatenate(vs), np.concatenate(rs)
         order = np.argsort(-vals, kind="stable")[:N_BEST]

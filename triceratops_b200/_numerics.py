@@ -38,3 +38,94 @@ def _normalize_probabilities(lnZ: np.ndarray):
     if np.isneginf(lnZ).all():
         return np.zeros(len(lnZ)), 'all_neginf'
     return np.exp(lnZ - _logsumexp(lnZ)), 'ok'
+
+
+# ---- Monte-Carlo error of the evidences ---------------------------------------------------------
+# Each lnZ is the log-mean-exp of N ln-weights lnw = lnL + lnprior.  With m = max finite lnw,
+# s = sum exp(lnw - m) and s2 = sum exp(2 (lnw - m)) over the finite entries:
+#   ess = s^2 / s2                          (effective sample size)
+#   r   = (N s2 / s^2 - 1) / (N - 1)        (unbiased sample variance of the weights / N, over Z^2)
+#   lnZ_err = sqrt(r)                       (delta method: sd(Z) / Z)
+
+def lse_moments(logw):
+    """(m, s, s2, n_finite, n_posinf) of an array of ln-weights: the record the GPU keeps per
+    branch, with the second moment of tri_set_moments."""
+    logw = np.asarray(logw, dtype=float)
+    n_posinf = int(np.isposinf(logw).sum())
+    fin = logw[np.isfinite(logw)]
+    if not fin.size:
+        return -np.inf, 0.0, 0.0, 0, n_posinf
+    m = float(fin.max())
+    t = np.exp(fin - m)
+    return m, float(t.sum()), float((t * t).sum()), int(fin.size), n_posinf
+
+
+def mc_error(N, m, s, s2, n_finite, n_posinf):
+    """(lnZ_err, ess, r) of one branch of N draws from its (m, s, s2) record.  lnZ_err is NaN
+    when a weight is +inf, when nothing is finite (lnZ = -inf: the row then carries no variance,
+    r = 0) and for N < 2."""
+    if n_posinf > 0:
+        return np.nan, np.nan, np.nan
+    if n_finite == 0 or not s > 0:
+        return np.nan, 0.0, 0.0
+    ess = s * s / s2
+    if N < 2:
+        return np.nan, ess, np.nan
+    r = max((N * s2 / (s * s) - 1.0) / (N - 1), 0.0)
+    return float(np.sqrt(r)), float(ess), float(r)
+
+
+def evidence_covariance(lnZ, r, calls, N_calls):
+    """Covariance of the scaled evidences Z_j = exp(lnZ_j - max lnZ) of the scenario rows.
+    `calls`: the rows of each scenario call (one row, or the two branches of an EB-type call,
+    which share their draws with disjoint masks); `N_calls`: the draws of each call.  Rows of
+    different calls are independent: Var(Z_j) = r_j Z_j^2; the branches a, b of one call have
+    Cov = -Z_a Z_b / (N - 1).  Returns (Z, V)."""
+    lnZ = np.asarray(lnZ, dtype=float)
+    Z = np.exp(lnZ - np.max(lnZ))
+    V = np.zeros((lnZ.size, lnZ.size))
+    for rows, N in zip(calls, N_calls):
+        for a in rows:
+            if Z[a] > 0:
+                V[a, a] = r[a] * Z[a] ** 2
+        if len(rows) == 2 and N > 1:
+            a, b = rows
+            V[a, b] = V[b, a] = -Z[a] * Z[b] / (N - 1)
+    return Z, V
+
+
+def sum_gradient(Z, R):
+    """Gradient over Z of F_R = sum_{i in R} Z_i / sum_j Z_j: (1{j in R} - F_R) / T."""
+    T = Z.sum()
+    ind = np.zeros(Z.size)
+    ind[list(R)] = 1.0
+    return (ind - Z[list(R)].sum() / T) / T
+
+
+def probability_errors(lnZ, r, calls, N_calls, fpp_rows=(0, 3, 9), nfpp_from=15):
+    """Delta-method errors of the scenario probabilities, FPP and NFPP.
+
+    Returns (prob_err [rows], FPP_err, NFPP_err, var_fpp_by_call [calls]); the last one is the
+    additive contribution of each call to Var(FPP) (calls are independent).  All NaN when the
+    probabilities are not defined (a NaN or +inf lnZ, or every lnZ -inf) or an error is NaN."""
+    lnZ = np.asarray(lnZ, dtype=float)
+    r = np.asarray(r, dtype=float)
+    n = lnZ.size
+    nan = (np.full(n, np.nan), np.nan, np.nan, np.full(len(calls), np.nan))
+    if np.isnan(lnZ).any() or np.isposinf(lnZ).any() or np.isneginf(lnZ).all():
+        return nan
+    Z, V = evidence_covariance(lnZ, r, calls, N_calls)
+    if np.isnan(V).any():
+        return nan
+    prob_err = np.empty(n)
+    for i in range(n):
+        g = sum_gradient(Z, (i,))
+        prob_err[i] = np.sqrt(max(g @ V @ g, 0.0))
+    g = sum_gradient(Z, fpp_rows)
+    contrib = np.array([g[rows] @ V[np.ix_(rows, rows)] @ g[rows] for rows in calls])
+    fpp_err = float(np.sqrt(max(contrib.sum(), 0.0)))
+    nfpp_err = 0.0
+    if n > nfpp_from:
+        g = sum_gradient(Z, range(nfpp_from, n))
+        nfpp_err = float(np.sqrt(max(g @ V @ g, 0.0)))
+    return prob_err, fpp_err, nfpp_err, contrib

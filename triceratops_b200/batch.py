@@ -43,9 +43,12 @@ def run_job(job):
                        job["flux_err"], job["P_orb"], **kw)
     finally:
         set_sampler("host")
-    return {"ID": job["ID"], "FPP": float(tgt.FPP), "NFPP": float(tgt.NFPP),
-            "FPP_degenerate": bool(tgt.FPP_degenerate), "lnZ": np.asarray(tgt.lnZ),
-            "probs": tgt.probs.to_dict(orient="list"), "wall_s": _time.perf_counter() - t0}
+    out = {"ID": job["ID"], "FPP": float(tgt.FPP), "NFPP": float(tgt.NFPP),
+           "FPP_degenerate": bool(tgt.FPP_degenerate), "lnZ": np.asarray(tgt.lnZ),
+           "probs": tgt.probs.to_dict(orient="list"), "wall_s": _time.perf_counter() - t0}
+    if tgt.FPP_err is not None:    # (calc_probs with mc_errors / fpp_err_target)
+        out["FPP_err"], out["NFPP_err"] = float(tgt.FPP_err), float(tgt.NFPP_err)
+    return out
 
 
 def _worker(worker_id, n_gpus, jobs, out_q, n_workers=None):

@@ -145,8 +145,9 @@ struct Slot {
     HostArena pinned;   // pinned copies of pageable host columns, on their way to `staging`
     unsigned long long* d_counters = nullptr;  // [8]
     unsigned long long* h_counters = nullptr;  // pinned [8]
-    LsePartial* d_lse_out = nullptr;           // [2]
-    LsePartial* h_lse_out = nullptr;           // pinned [2]
+    LsePartial* d_lse_out = nullptr;           // [2], then s2 of the two branches (kLseOutBytes)
+    LsePartial* h_lse_out = nullptr;           // pinned, same layout
+    unsigned int* d_mom_done = nullptr;        // moments_kernel's block counter
     TopkState* d_topk = nullptr;               // [2]
     TopkState* h_topk = nullptr;               // pinned [2]
     unsigned int* d_hist16 = nullptr;          // [2][kTopkBins], zero between calls
@@ -157,6 +158,8 @@ struct Slot {
     int64_t ticket = 0;   // 0 = free
     int branches = 0;     // 1 = TP-type, 2 = EB-type
     int64_t N = 0;
+    bool moments = false; // tri_set_moments at submission: s2 follows the records
+    double s2[2] = {NAN, NAN};
     bool host = false;    // host-buffer call: best-draw candidates are sorted in tri_wait
     bool want_top[2] = {false, false};
     tri_result want[2];   // the caller's records: its pointers go back into the results
@@ -176,6 +179,7 @@ struct Ctx {
     int sm_count = 0;
     int lnl_blocks_per_sm = 0;
     bool count_work = false;   // tri_set_counting: run the instantiation with work counters
+    bool moments = false;      // tri_set_moments: second moment of the weights per branch
     size_t lnl_smem = 0;   // dynamic shared memory used to stage the light curve (0 = none)
     cudaStream_t stream = nullptr;        // kernels and result read-back
     cudaStream_t copy_stream = nullptr;   // host columns -> staging (overlaps the kernels)
@@ -191,7 +195,11 @@ struct Ctx {
     Slot slots[kSlots + 1];
     int64_t next_ticket = 1;
     Slot* last = nullptr;    // the call completed last (tri_last_timing, tri_fetch_lnl)
+    double last_s2[2] = {NAN, NAN};   // s2 of the evaluation tri_wait returned last
 };
+
+// d_lse_out / h_lse_out: the branches' evidence records, then their s2 (moments_kernel)
+constexpr size_t kLseOutBytes = 2 * sizeof(LsePartial) + 2 * sizeof(double);
 
 Ctx g;
 
@@ -270,6 +278,7 @@ size_t scratch_bytes(int64_t N, bool eb) {
     b += (n * 8 + 256) * (eb ? 4 : 2);   // a, lnl (+ p, lnl_twin)
     b += (n * 8 + 256) * 2;              // items, cval
     b += (size_t)lnl_grid() * sizeof(LsePartial) * 2 + 512;
+    b += (size_t)lse_blocks(N) * sizeof(double) * 2 + 256;   // moments_kernel partials
     return b + 4096;
 }
 
@@ -317,6 +326,25 @@ int launch_finalize(Slot& S, const Scratch& W, int64_t N, int branches, const tr
     if (branches == 1) S.want_top[1] = false;
     F.st = S.d_topk;
     finalize_kernel<<<branches, kFinThreads, 0, s>>>(F);
+    S.launches += 1;
+    CU(cudaGetLastError());
+    return TRI_OK;
+}
+
+// s2 of the call's branches after finalize_kernel (only with tri_set_moments on)
+int launch_moments(Slot& S, const Scratch& W, int64_t N, int branches, Col lnprior,
+                   cudaStream_t s) {
+    MomentsArgs M{};
+    M.lnl[0] = W.lnl;
+    M.lnl[1] = W.lnl_twin;
+    M.lnprior = lnprior;
+    M.N = N;
+    M.branches = branches;
+    M.lse = S.d_lse_out;
+    M.partials = S.scratch.take<double>(2 * (size_t)lse_blocks(N));
+    M.done = S.d_mom_done;
+    M.s2_out = reinterpret_cast<double*>(S.d_lse_out + 2);
+    moments_kernel<<<lse_blocks(N), kMomThreads, 0, s>>>(M);
     S.launches += 1;
     CU(cudaGetLastError());
     return TRI_OK;
@@ -370,10 +398,16 @@ int enqueue_tp(Slot& S, const tri_tp_args& a, const tri_result& r, cudaStream_t 
     CU(cudaEventRecord(S.ev[2], s));
     rc = launch_finalize(S, W, N, 1, &r, s);
     if (rc) return rc;
+    S.moments = g.moments;
+    if (S.moments) {
+        rc = launch_moments(S, W, N, 1, to_col(a.lnprior), s);
+        if (rc) return rc;
+    }
     CU(cudaMemcpyAsync(S.h_topk, S.d_topk, sizeof(TopkState), cudaMemcpyDeviceToHost, s));
     S.lnl[0] = W.lnl; S.lnl[1] = nullptr;
     CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, sizeof(LsePartial), cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, S.moments ? kLseOutBytes : sizeof(LsePartial),
+                       cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
                        cudaMemcpyDeviceToHost, s));
     return TRI_OK;
@@ -431,10 +465,16 @@ int enqueue_eb(Slot& S, const tri_eb_args& a, const tri_result r[2], cudaStream_
     CU(cudaEventRecord(S.ev[2], s));
     rc = launch_finalize(S, W, N, 2, r, s);
     if (rc) return rc;
+    S.moments = g.moments;
+    if (S.moments) {
+        rc = launch_moments(S, W, N, 2, to_col(a.lnprior), s);
+        if (rc) return rc;
+    }
     CU(cudaMemcpyAsync(S.h_topk, S.d_topk, 2 * sizeof(TopkState), cudaMemcpyDeviceToHost, s));
     S.lnl[0] = W.lnl; S.lnl[1] = W.lnl_twin;
     CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, 2 * sizeof(LsePartial), cudaMemcpyDeviceToHost,
+    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out,
+                       S.moments ? kLseOutBytes : 2 * sizeof(LsePartial), cudaMemcpyDeviceToHost,
                        s));
     CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
                        cudaMemcpyDeviceToHost, s));
@@ -454,6 +494,9 @@ void sort_candidates(int64_t n, int64_t* idx, double* val) {
 
 // After the slot's `done` event: turn the pinned landing zone into the caller's records.
 void finish_slot(Slot& S, tri_result* out) {
+    const double* h_s2 = reinterpret_cast<const double*>(S.h_lse_out + 2);
+    for (int b = 0; b < 2; ++b)
+        S.s2[b] = !S.moments || b >= S.branches ? NAN : S.N == 0 ? 0.0 : h_s2[b];
     for (int b = 0; b < S.branches; ++b) {
         tri_result r = S.want[b];   // keeps the caller's pointers and top_cap
         if (S.N == 0) {
@@ -562,6 +605,7 @@ int check_eb(const tri_eb_args* a, const void* out) {
 // mark the slot in flight and hand out its ticket
 void commit(Slot& S, int branches, int64_t N, bool host, const tri_result* want,
             int64_t* ticket) {
+    if (N == 0) S.moments = g.moments;   // (no kernels: enqueue_* did not run)
     S.branches = branches;
     S.N = N;
     S.host = host;
@@ -615,8 +659,10 @@ int tri_init(int device) {
     g.tab.inv_dm = 1.0 / g.tab.dm;
     for (Slot& S : g.slots) {
         CU(cudaMalloc(&S.d_counters, 8 * sizeof(unsigned long long)));
-        CU(cudaMalloc(&S.d_lse_out, 2 * sizeof(LsePartial)));
-        CU(cudaMallocHost(&S.h_lse_out, 2 * sizeof(LsePartial)));
+        CU(cudaMalloc(&S.d_lse_out, kLseOutBytes));
+        CU(cudaMallocHost(&S.h_lse_out, kLseOutBytes));
+        CU(cudaMalloc(&S.d_mom_done, sizeof(unsigned int)));
+        CU(cudaMemset(S.d_mom_done, 0, sizeof(unsigned int)));
         CU(cudaMallocHost(&S.h_counters, 8 * sizeof(unsigned long long)));
         CU(cudaMalloc(&S.d_topk, 2 * sizeof(TopkState)));
         CU(cudaMalloc(&S.d_hist16, 2 * (size_t)kTopkBins * sizeof(unsigned int)));
@@ -650,6 +696,7 @@ int tri_shutdown(void) {
         cudaFree(S.d_counters);
         cudaFree(S.d_lse_out);
         cudaFreeHost(S.h_lse_out);
+        cudaFree(S.d_mom_done);
         cudaFreeHost(S.h_counters);
         cudaFree(S.d_topk);
         cudaFree(S.d_hist16);
@@ -684,6 +731,22 @@ int tri_set_counting(int32_t on) {
     int rc = need_ready(false);
     if (rc) return rc;
     g.count_work = on != 0;
+    return TRI_OK;
+}
+
+int tri_set_moments(int32_t on) {
+    int rc = need_ready(false);
+    if (rc) return rc;
+    g.moments = on != 0;
+    return TRI_OK;
+}
+
+int tri_last_moments(double s2[2]) {
+    int rc = need_ready(false);
+    if (rc) return rc;
+    if (!s2) return fail(TRI_EINVAL, "NULL argument");
+    s2[0] = g.last_s2[0];
+    s2[1] = g.last_s2[1];
     return TRI_OK;
 }
 
@@ -1095,6 +1158,8 @@ int tri_wait(int64_t ticket, tri_result* out) {
     finish_slot(*S, out);
     S->ticket = 0;
     g.last = S;
+    g.last_s2[0] = S->s2[0];
+    g.last_s2[1] = S->s2[1];
     if (S->host && S->N > 0) {   // per-draw outputs (parity runs): copied now, synchronously
         for (int b = 0; b < S->branches; ++b) {
             if (S->d_out_lnl[b])

@@ -1276,6 +1276,77 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(FinalizeArgs F) {
     }
 }
 
+// ---- second moment of the weights (tri_set_moments) ---------------------------------------------
+// s2[b] = sum over the finite ln-weights x of branch b of exp(2 (x - m_b)), with m_b the branch's
+// maximum from finalize_kernel and x formed exactly as lnl_kernel's epilogue forms it (lnL +
+// lnprior), so that every term is <= 1.  Reads the per-draw lnL arrays in draw order: block k
+// sums a contiguous range, the last block to finish merges the block sums in block order, so the
+// result does not depend on scheduling.
+constexpr int kMomThreads = 256;
+
+struct MomentsArgs {
+    const double* lnl[2];         // per-draw lnL of branch 0 / 1 (-inf where not evaluated)
+    Col lnprior;                  // ptr nullptr: none
+    int64_t N;
+    int branches;
+    const LsePartial* lse;        // [branches] evidence records of finalize_kernel
+    double* partials;             // [2][gridDim.x]
+    unsigned int* done;           // block counter, 0 between launches
+    double* s2_out;               // [branches]
+};
+
+__device__ __forceinline__ double block_sum_mom(double v, double* sh) {
+    sh[threadIdx.x] = v;
+    __syncthreads();
+    for (int o = kMomThreads / 2; o > 0; o >>= 1) {
+        if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
+        __syncthreads();
+    }
+    double r = sh[0];
+    __syncthreads();
+    return r;
+}
+
+__global__ void __launch_bounds__(kMomThreads) moments_kernel(MomentsArgs M) {
+    __shared__ double sh[kMomThreads];
+    __shared__ bool last;
+    const int64_t per = (M.N + gridDim.x - 1) / gridDim.x;
+    const int64_t lo = (int64_t)blockIdx.x * per;
+    const int64_t hi = lo + per < M.N ? lo + per : M.N;
+    for (int b = 0; b < M.branches; ++b) {
+        const double m = M.lse[b].m;
+        const double* lnl = b ? M.lnl[1] : M.lnl[0];   // (constant indices: no stack copy)
+        double acc = 0.0;
+        if (isfinite(m)) {
+            for (int64_t i = lo + threadIdx.x; i < hi; i += kMomThreads) {
+                double x = lnl[i];
+                if (M.lnprior.p) x += M.lnprior.at(i);
+                if (isfinite(x)) {
+                    const double t = exp(x - m);
+                    acc += t * t;
+                }
+            }
+        }
+        acc = block_sum_mom(acc, sh);
+        if (threadIdx.x == 0) M.partials[(size_t)b * gridDim.x + blockIdx.x] = acc;
+    }
+    __threadfence();
+    if (threadIdx.x == 0) last = atomicAdd(M.done, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    const int nb = (int)gridDim.x;
+    const int chunk = (nb + kMomThreads - 1) / kMomThreads;
+    for (int b = 0; b < M.branches; ++b) {
+        double acc = 0.0;
+        for (int q = threadIdx.x * chunk; q < (int)(threadIdx.x + 1) * chunk && q < nb; ++q)
+            acc += __ldcg(M.partials + (size_t)b * nb + q);
+        acc = block_sum_mom(acc, sh);
+        if (threadIdx.x == 0) M.s2_out[b] = acc;
+    }
+    if (threadIdx.x == 0) *M.done = 0u;
+}
+
 // ---- standalone log-mean-exp of an array (tri_log_mean_exp, _numerics.py:12-51) ----------------
 constexpr int kLseThreads = 256;
 

@@ -281,6 +281,7 @@ def _finished(exchange):
     merged['lnZ'] = lnZ
     out = ml.ScenarioResult(merged)
     out.n_pass, out.n_evaluated = n_pass, n_eval
+    out.set_moments(exchange.lb.N, exchange.record, exchange.top)
     return out
 
 

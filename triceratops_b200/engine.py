@@ -66,7 +66,8 @@ def cadence_columns(exptime, nsamples, npts):
 class BranchResult:
     """One scenario branch: lnZ pieces + optional per-draw arrays."""
     __slots__ = ("lnZ", "m", "s", "n_finite", "n_posinf", "n_pass", "n_stamps", "n_interior",
-                 "n_limb", "lnL", "mask", "N", "top_idx", "top_lnL", "n_evaluated", "branch")
+                 "n_limb", "lnL", "mask", "N", "top_idx", "top_lnL", "n_evaluated", "branch",
+                 "s2")
 
     def __init__(self, r, N, lnL, mask, top=None, branch=0):
         self.lnZ, self.m, self.s = r.lnZ, r.m, r.s
@@ -75,6 +76,7 @@ class BranchResult:
         self.n_interior, self.n_limb = r.n_interior, r.n_limb
         self.lnL, self.mask, self.N = lnL, mask, N
         self.branch = branch
+        self.s2 = None       # second moment of the weights (Engine.set_moments), set on wait
         if top is not None:
             self.top_idx, self.top_lnL = top[0][:r.n_top], top[1][:r.n_top]
             self.n_evaluated = r.n_evaluated
@@ -100,6 +102,7 @@ class Pending:
     def __init__(self, engine, ticket, rr, n_branches, keep, build, n_best):
         self._engine, self._ticket, self._rr, self._nb = engine, ticket, rr, n_branches
         self._keep, self._build, self._n_best = keep, build, n_best
+        self._moments = engine._moments     # (tri_set_moments is captured per submission)
         self._out = None
 
     def done(self):
@@ -121,6 +124,11 @@ class Pending:
                 if self in eng._inflight:
                     eng._inflight.remove(self)
             out = self._build(self._rr)
+            if self._moments:
+                s2 = (ctypes.c_double * 2)()
+                _cabi.check(eng.lib.tri_last_moments(s2))
+                for b, br in enumerate(out):
+                    br.s2 = s2[b]
             # fewer finite draws than the table has rows: the caller pads the table from the
             # full lnL array, which is only reachable until the next evaluation completes
             for b, br in enumerate(out):
@@ -148,6 +156,21 @@ def combine_lse(parts, N_total):
     return m + math.log(S) - math.log(N_total)
 
 
+def combine_moments(parts):
+    """Merged (m, s, s2, n_finite, n_posinf) of (m, s, s2, n_finite, n_posinf) records over
+    disjoint slices of draws (ranks, or rounds of refinement): s and s2 are rescaled to the
+    common maximum, s by exp(m_r - m) and s2 by exp(2 (m_r - m)).  lnZ itself is combine_lse's."""
+    n_fin = sum(int(p[3]) for p in parts)
+    n_pinf = sum(int(p[4]) for p in parts)
+    fin = [p for p in parts if p[3] > 0]
+    if not fin:
+        return -math.inf, 0.0, 0.0, n_fin, n_pinf
+    m = max(p[0] for p in fin)
+    s = sum(p[1] * math.exp(p[0] - m) for p in fin)
+    s2 = sum(p[2] * math.exp(2.0 * (p[0] - m)) for p in fin)
+    return m, s, s2, n_fin, n_pinf
+
+
 class Engine:
     def __init__(self, device=None):
         self.lib = _cabi.load()
@@ -161,6 +184,7 @@ class Engine:
         self._inflight = []      # Pendings not waited for yet, oldest first
         self._side_streams = None
         self._side_turn = 0
+        self._moments = False
 
     @_locked
     def _make_room(self):
@@ -543,6 +567,13 @@ class Engine:
     def set_counting(self, on):
         """Work counters of the roofline model (n_stamps, n_interior, n_limb) on / off."""
         _cabi.check(self.lib.tri_set_counting(int(bool(on))))
+
+    @_locked
+    def set_moments(self, on):
+        """Second moment of the weights per branch (tri_set_moments): BranchResult.s2 of the
+        evaluations submitted while it is on, None otherwise."""
+        _cabi.check(self.lib.tri_set_moments(int(bool(on))))
+        self._moments = bool(on)
 
     @_locked
     def fp64_peak(self):

@@ -28,6 +28,7 @@ from pandas import read_csv
 
 from . import _blocks, _dispatch, _fastrng
 from . import _hostpar
+from ._numerics import mc_error
 from ._constants import G, Msun, Rsun, pi
 from ._ldc import grid_for
 from .funcs import (file_to_contrast_curve, flux_relation, stellar_relations, trilegal_results)
@@ -291,12 +292,30 @@ def _background_prior(bg, N, contrast_curve_file, dmag_tess, dmag_cc):
 
 
 class ScenarioResult(dict):
-    """The reference's result dictionary (same keys) with two diagnostics as attributes:
-    n_pass (draws surviving the geometric mask) and n_evaluated (draws with a finite lnL; when
-    it is below 100 the tail of the best-draw table holds draws of zero weight in arbitrary
-    order, as in the reference)."""
+    """The reference's result dictionary (same keys) with diagnostics as attributes: n_pass
+    (draws surviving the geometric mask) and n_evaluated (draws with a finite lnL; when it is
+    below 100 the tail of the best-draw table holds draws of zero weight in arbitrary order, as
+    in the reference).  Inside `triceratops_b200.mc_errors()` also the Monte-Carlo error of
+    lnZ: N (draws), s2 (second moment of the weights, _numerics), lnZ_err (standard error of
+    lnZ) and ess (effective sample size); None otherwise."""
     n_pass = 0
     n_evaluated = 0
+    N = None
+    s2 = None
+    lnZ_err = None
+    ess = None
+    # (m, s, s2, n_finite, n_posinf) of the branch and (lnL, draw index) of the table's finite
+    # rows: what calc_probs merges when it refines a scenario with more draws
+    record = None
+    top = None
+
+    def set_moments(self, N, record, top):
+        """Attach the branch's evidence record; the error fields when it carries s2."""
+        self.N, self.record, self.top = int(N), tuple(record), top
+        if record[2] is not None:
+            self.s2 = float(record[2])
+            self.lnZ_err, self.ess, _ = mc_error(N, record[0], record[1], record[2], record[3],
+                                                 record[4])
 
 
 def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, **body):
@@ -309,6 +328,8 @@ def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, *
         _take(P, idx), _take(mtot, idx), incs[idx], eccs[idx], argps[idx],
         fluxratio_comp=_take(cfr, idx) if np.ndim(cfr) else None, **rows), lnZ=br.lnZ)
     out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
+    out.set_moments(br.N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
+                    (br.vals, np.asarray(idx)[:len(br.vals)]))
     return out
 
 

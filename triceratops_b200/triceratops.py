@@ -13,6 +13,7 @@ from a stars table the caller already has (the reference's `target.stars` DataFr
 from an online session), optionally its `pix_coords`, and a saved TRILEGAL file.
 """
 import collections
+import contextlib
 import functools
 import sys
 import warnings
@@ -22,10 +23,10 @@ from pandas import DataFrame
 from scipy.special import ndtr
 
 from . import _bufpool, _dispatch
-from ._numerics import _normalize_probabilities
+from ._numerics import _normalize_probabilities, mc_error, probability_errors
 from .funcs import renorm_flux
-from .marginal_likelihoods import (RESULT_KEYS, lnZ_BEB, lnZ_BTP, lnZ_DEB, lnZ_DTP, lnZ_PEB,
-                                   lnZ_PTP, lnZ_SEB, lnZ_STP, lnZ_TEB, lnZ_TTP)
+from .marginal_likelihoods import (RESULT_KEYS, ScenarioResult, lnZ_BEB, lnZ_BTP, lnZ_DEB,
+                                   lnZ_DTP, lnZ_PEB, lnZ_PTP, lnZ_SEB, lnZ_STP, lnZ_TEB, lnZ_TTP)
 
 _STAR_COLUMNS = ("ID", "Tmag", "Jmag", "Hmag", "Kmag", "ra", "dec", "mass", "rad", "Teff", "plx",
                  "fluxratio", "tdepth")
@@ -136,7 +137,8 @@ class target:
                    drop_scenario: list = [],
                    verbose: int = 1, flatpriors: bool = False,
                    exptime: float = 0.00139, nsamples: int = 20,
-                   molusc_file: str = None):
+                   molusc_file: str = None, mc_errors: bool = False,
+                   fpp_err_target: float = None, N_max: int = None):
         """Relative probability of every scenario, FPP and NFPP (triceratops.py:673-1485).
 
         Extensions of the reference's arguments: `flux_err_0` may hold one error per time stamp
@@ -145,7 +147,32 @@ class target:
         light curve that mixes cadences (e.g. 30-min and 200-s TESS FFIs with 2-min target
         pixels).  The stamps are then modelled in groups of equal (exptime, nsamples), at most
         TRI_MAX_CADENCES = 8 of them, each with its own integration time and supersampling.
-        Per-stamp arrays lose the rows whose time or flux is NaN, like time and flux."""
+        Per-stamp arrays lose the rows whose time or flux is NaN, like time and flux.
+
+        Monte-Carlo error bars (not in the reference; lnZ, probs, FPP and NFPP are the same
+        bits with and without them): `mc_errors=True` also sets `lnZ_err`, `ess` and `N_draws`
+        (per row), `FPP_err` and `NFPP_err` (delta method over the rows' evidences, see
+        _numerics.probability_errors) and adds a `prob_err` column to `probs`; without it these
+        attributes are None.  `fpp_err_target` (implies mc_errors) then refines: after each
+        round, the scenario calls that carry the largest shares of Var(FPP) -- from the top,
+        until they add up to at least half of it -- get as many new draws as they have so far,
+        at most `N_max` in all per call (default 16 N); the new draws merge with the old ones
+        as one more disjoint slice.  Rounds stop when FPP_err <= fpp_err_target or no
+        contributing call can grow.  Host sampler: the new draws continue numpy's global
+        generator; device sampler: each round is a new scenario call (a fresh Philox stream).
+        Refinement needs all draws on this process (no draw sharding over a process group)."""
+        if fpp_err_target is not None:
+            if not (np.isfinite(fpp_err_target) and fpp_err_target > 0):
+                raise ValueError("fpp_err_target must be positive and finite")
+            mc_errors = True
+            if N_max is None:
+                N_max = 16 * int(N)
+            if _dispatch._dist() is not None:
+                raise ValueError("fpp_err_target refines scenarios on one process: it cannot be "
+                                 "combined with draws sharded over a process group (vet whole "
+                                 "targets per rank instead, batch.vet_many)")
+        if N_max is not None and int(N_max) < int(N):
+            raise ValueError("N_max (%d) must be >= N (%d)" % (int(N_max), int(N)))
         n_in = np.size(time)
         keep = ~np.isnan(time) & ~np.isnan(flux_0)
         time = time[keep]
@@ -173,6 +200,8 @@ class target:
         scenarios = np.zeros(n_rows, dtype=np.dtype("U6"))
         best = {k: np.zeros(n_rows) for k in RESULT_KEYS}
         lnZ = np.zeros(n_rows)
+        row_results = [None] * n_rows      # (mc_errors) the resolved result of every row
+        calls = []                         # (mc_errors) (rows, make(n_draws)) per scenario call
 
         # Results are read a few scenarios after they were requested: the GPU works on one
         # scenario while the host draws the priors of the next (_dispatch.deferring), and with
@@ -198,6 +227,7 @@ class target:
                 for k in RESULT_KEYS:
                     best[k][j] = res[k][0]
                 lnZ[j] = res["lnZ"]
+                row_results[j] = res
 
         def settle(keep):
             while len(waiting) > keep:
@@ -220,7 +250,8 @@ class target:
                 for j in rows:
                     lnZ[j] = -np.inf
                 return
-            waiting.append((rows, chain.run(fn)))
+            calls.append((rows, fn))
+            waiting.append((rows, chain.run(functools.partial(fn, N))))
             settle(_PIPELINE_DEPTH)
 
         def say(msg):
@@ -240,8 +271,9 @@ class target:
         switch_interval = sys.getswitchinterval()
         sys.setswitchinterval(_dispatch.gil_switch_interval())
         _bufpool.note_call()       # (page-locked column buffers from a process's second call on)
+        moments = _dispatch.mc_errors() if mc_errors else contextlib.nullcontext()
         try:
-            with _dispatch.deferring():
+            with moments, _dispatch.deferring():
                 for i, ID in enumerate(filtered["ID"].values if not follower else ()):
                     star = {c: filtered[c].values[i] for c in _STAR_COLUMNS}
                     flux, flux_err = renorm_flux(flux_0, flux_err_0, star["fluxratio"])
@@ -249,7 +281,8 @@ class target:
                     mags = (star["Tmag"], star["Jmag"], star["Hmag"], star["Kmag"])
                     Z = 0.0
                     lc = (time, flux, flux_err, P_orb)
-                    tail = (N, parallel, self.mission, flatpriors, exptime, nsamples)
+                    tail = dict(parallel=parallel, mission=self.mission, flatpriors=flatpriors,
+                                exptime=exptime, nsamples=nsamples)
 
                     if i == 0:
                         if np.isnan(M_s) or np.isnan(R_s) or np.isnan(Teff) or np.isnan(plx):
@@ -257,26 +290,26 @@ class target:
                                   + ". Please ensure a stellar mass (in M_Sun), radius (in R_Sun), "
                                   + "Teff (in K), and plx (in mas) are provided in the .stars dataframe.")
                             break
-                        bind = functools.partial      # (the loop variables change under the threads)
+                        # (bound now: the loop variables change under the threads)
                         runners = {
-                            "TP": bind(lnZ_TTP, *lc, M_s, R_s, Teff, Z, *tail),
-                            "EB": bind(lnZ_TEB, *lc, M_s, R_s, Teff, Z, *tail),
-                            "PTP": bind(lnZ_PTP, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
-                                        filt, *tail, molusc_file),
-                            "PEB": bind(lnZ_PEB, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
-                                        filt, *tail, molusc_file),
-                            "STP": bind(lnZ_STP, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
-                                        filt, *tail, molusc_file),
-                            "SEB": bind(lnZ_SEB, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
-                                        filt, *tail, molusc_file),
-                            "DTP": bind(lnZ_DTP, *lc, M_s, R_s, Teff, Z, *mags, trilegal_fname,
-                                        contrast_curve_file, filt, *tail),
-                            "DEB": bind(lnZ_DEB, *lc, M_s, R_s, Teff, Z, *mags, trilegal_fname,
-                                        contrast_curve_file, filt, *tail),
-                            "BTP": bind(lnZ_BTP, *lc, M_s, R_s, Teff, *mags, trilegal_fname,
-                                        contrast_curve_file, filt, *tail),
-                            "BEB": bind(lnZ_BEB, *lc, M_s, R_s, Teff, *mags, trilegal_fname,
-                                        contrast_curve_file, filt, *tail),
+                            "TP": _bind(lnZ_TTP, *lc, M_s, R_s, Teff, Z, **tail),
+                            "EB": _bind(lnZ_TEB, *lc, M_s, R_s, Teff, Z, **tail),
+                            "PTP": _bind(lnZ_PTP, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
+                                         filt, **tail, molusc_file=molusc_file),
+                            "PEB": _bind(lnZ_PEB, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
+                                         filt, **tail, molusc_file=molusc_file),
+                            "STP": _bind(lnZ_STP, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
+                                         filt, **tail, molusc_file=molusc_file),
+                            "SEB": _bind(lnZ_SEB, *lc, M_s, R_s, Teff, Z, plx, contrast_curve_file,
+                                         filt, **tail, molusc_file=molusc_file),
+                            "DTP": _bind(lnZ_DTP, *lc, M_s, R_s, Teff, Z, *mags, trilegal_fname,
+                                         contrast_curve_file, filt, **tail),
+                            "DEB": _bind(lnZ_DEB, *lc, M_s, R_s, Teff, Z, *mags, trilegal_fname,
+                                         contrast_curve_file, filt, **tail),
+                            "BTP": _bind(lnZ_BTP, *lc, M_s, R_s, Teff, *mags, trilegal_fname,
+                                         contrast_curve_file, filt, **tail),
+                            "BEB": _bind(lnZ_BEB, *lc, M_s, R_s, Teff, *mags, trilegal_fname,
+                                         contrast_curve_file, filt, **tail),
                         }
                         for key, row, num, names in _TARGET_SCENARIOS:
                             if len(names) == 1:
@@ -299,9 +332,9 @@ class target:
                             + str(ID) + ".")
                         row = 15 + 3 * (i - 1)
                         launch(row, ID, 1, ("NTP",),
-                               functools.partial(lnZ_TTP, *lc, M_s, R_s, Teff, Z, *tail))
+                               _bind(lnZ_TTP, *lc, M_s, R_s, Teff, Z, **tail))
                         launch(row + 1, ID, 1, ("NEB", "NEBx2P"),
-                               functools.partial(lnZ_TEB, *lc, M_s, R_s, Teff, Z, *tail))
+                               _bind(lnZ_TEB, *lc, M_s, R_s, Teff, Z, **tail))
                 settle(0)
                 ok = True
         finally:
@@ -313,20 +346,27 @@ class target:
             finally:
                 if not ok:
                     _dispatch.close_group()
+        err = None
         try:
             if follower:
-                targets, star_num, scenarios, best, lnZ = group.follow(eng)
+                with _dispatch.mc_errors() if mc_errors else contextlib.nullcontext():
+                    targets, star_num, scenarios, best, lnZ, err = group.follow(eng)
             elif group is not None:
                 group.exchange()
                 for rows, parts in held:
                     fill(rows, parts)
+                if mc_errors:
+                    err = _refine(calls, row_results, lnZ, best, None, None)
                 if group.scatter:
-                    group.publish((targets, star_num, scenarios, best, lnZ))
+                    group.publish((targets, star_num, scenarios, best, lnZ, err))
         finally:
             self.collectives = None if group is None else {
                 "record_exchanges": group.collectives, "scatters": group.scatters}
             _dispatch.close_group()
 
+        if mc_errors and group is None:
+            with _dispatch.mc_errors():
+                err = _refine(calls, row_results, lnZ, best, fpp_err_target, N_max)
         relative_probs, status = _normalize_probabilities(lnZ)
         if status == 'anomaly':
             warnings.warn(
@@ -359,4 +399,95 @@ class target:
         prob = self.probs.prob
         self.FPP = 1 - (prob[0] + prob[3] + prob[9])
         self.NFPP = np.sum(prob[15:]) if len(prob) > 15 else 0.0
+        self.lnZ_err = self.ess = self.N_draws = self.FPP_err = self.NFPP_err = None
+        if err is not None:
+            self.lnZ_err, self.ess, self.N_draws = err["lnZ_err"], err["ess"], err["N"]
+            self.FPP_err, self.NFPP_err = err["FPP_err"], err["NFPP_err"]
+            self.probs["prob_err"] = err["prob_err"]
         return
+
+
+def _bind(fn, *args, **kw):
+    """One scenario call as a function of its number of draws: fn(*args, N=n, **kw)."""
+    def make(n):
+        return fn(*args, N=n, **kw)
+    return make
+
+
+def _row_errors(calls, lnZ):
+    """Per-row (lnZ_err, ess, N) and the delta-method errors of the rows' probabilities, FPP and
+    NFPP from the current result of every scenario call (`calls`: dicts with rows, N, cur)."""
+    n = len(lnZ)
+    lnZ_err, ess, r = np.full(n, np.nan), np.zeros(n), np.zeros(n)
+    N_draws = np.zeros(n, dtype=np.int64)
+    for c in calls:
+        for j, res in zip(c["rows"], c["cur"]):
+            N_draws[j] = c["N"]
+            if res.s2 is None:        # (an engine without the moment pass)
+                r[j] = np.nan
+                continue
+            lnZ_err[j], ess[j], r[j] = mc_error(c["N"], res.record[0], res.record[1],
+                                                res.record[2], res.record[3], res.record[4])
+    prob_err, fpp_err, nfpp_err, contrib = probability_errors(
+        lnZ, r, [c["rows"] for c in calls], [c["N"] for c in calls])
+    return dict(lnZ_err=lnZ_err, ess=ess, N=N_draws, prob_err=prob_err, FPP_err=fpp_err,
+                NFPP_err=nfpp_err), contrib
+
+
+def _merge_round(old, new, offset):
+    """One branch's result over the draws of `old` followed by `new` (drawn after them: its
+    indices start at `offset`), merged like the records of two ranks (_dispatch._merge_records):
+    lnZ over all draws, the best-draw table the top 100 of both, each row from the round that
+    drew it."""
+    N = old.N + new.N
+    allrec = np.stack([
+        _dispatch.record_row(r.record[0], r.record[1], r.record[3], r.record[4], r.n_pass,
+                             r.n_evaluated, r.record[2], np.asarray(r.top[1]) + off, r.top[0])
+        for r, off in ((old, 0), (new, offset))])
+    br = _dispatch._merge_records(allrec, 0, N, N)
+    where = {}
+    for src, off in ((new, offset), (old, 0)):
+        for pos, i in enumerate(np.asarray(src.top[1])[:len(src.top[0])]):
+            where.setdefault(int(i) + off, (src, pos))
+    k = len(br.vals)
+    picks = [where[int(i)] for i in br.idx[:k]]
+    # rows of zero weight (fewer than 100 finite draws in all): old's padding rows
+    picks += [(old, pos) for pos in range(k, len(old[RESULT_KEYS[0]]))]
+    out = ScenarioResult({key: np.array([src[key][pos] for src, pos in picks])
+                          for key in RESULT_KEYS}, lnZ=br.lnZ)
+    out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
+    out.set_moments(N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
+                    (br.vals, br.idx[:k]))
+    return out
+
+
+def _refine(calls, row_results, lnZ, best, target, N_max):
+    """Error bars of calc_probs; with `target`, refinement rounds until FPP_err <= target or no
+    call that contributes to Var(FPP) can grow (N_max draws per call).  Updates lnZ and best in
+    place for the refined rows; returns the error fields."""
+    state = [dict(rows=rows, make=make, N=int(row_results[rows[0]].N),
+                  cur=[row_results[j] for j in rows]) for rows, make in calls]
+    err, contrib = _row_errors(state, lnZ)
+    while target is not None and np.isfinite(err["FPP_err"]) and err["FPP_err"] > target:
+        total, acc, picked = contrib.sum(), 0.0, []
+        for ci in np.argsort(-contrib, kind="stable"):
+            if not contrib[ci] > 0 or acc >= 0.5 * total:
+                break
+            if state[ci]["N"] < N_max:
+                picked.append(ci)
+                acc += contrib[ci]
+        if not picked:
+            break
+        for ci in picked:
+            c = state[ci]
+            n_new = min(c["N"], N_max - c["N"])
+            out = c["make"](n_new)
+            parts = out if isinstance(out, tuple) else (out,)
+            c["cur"] = [_merge_round(old, new, c["N"]) for old, new in zip(c["cur"], parts)]
+            c["N"] += n_new
+            for j, res in zip(c["rows"], c["cur"]):
+                lnZ[j] = res["lnZ"]
+                for k in RESULT_KEYS:
+                    best[k][j] = res[k][0]
+        err, contrib = _row_errors(state, lnZ)
+    return err
