@@ -206,7 +206,8 @@ int tri_log_mean_exp(const double* logw, int64_t n, tri_result* out);
 /* Device time [ms] of the kernels of the most recent eval/lnl call, from CUDA events on the
  * stream they ran on: geometry, light-curve/chi^2 (with the fused evidence epilogue), the
  * finalize kernel (merge of the block records + best-draw selection; with tri_set_moments on,
- * also the moments kernel), and their launch count (3 per evaluation, 4 with moments). */
+ * also the moments kernel; with tri_set_posterior K > 0, also the two resampling kernels), and
+ * their launch count (3 per evaluation, 4 with moments, 2 more with posterior samples). */
 int tri_last_timing(double* geometry_ms, double* lnl_ms, double* lse_ms, int32_t* launches);
 
 /* Device-side prior sampler support (opt-in mode, triceratops_b200.set_sampler("device")):
@@ -304,6 +305,28 @@ int tri_set_moments(int32_t on);
  * tri_eval_* / tri_eval_*_dev / tri_wait; NaN where moments were off for it (and for s2[1] of a
  * TP-type call).  A submission keeps its s2 until it is waited for. */
 int tri_last_moments(double s2[2]);
+
+/* Posterior samples by systematic importance resampling (off by default).  With K > 0 every
+ * evaluation submitted afterwards also draws K samples from the N prior draws of each branch,
+ * with weights w_i = exp(x_i - m), x_i = lnL_i + lnprior_i formed as for lnZ and m the branch's
+ * record (0 where x_i is not finite): with C the prefix sums of w in draw order and T = C_{N-1},
+ * sample k (k < K) is draw min{i : C_i > (U + k) T / K}, positions at or above T going to the
+ * last draw at which C increases.  U in [0, 1) is a hash of (seed, stream, branch)
+ * (triceratops_b200._numerics.posterior_uniform).  Two more kernels run per evaluation, after
+ * the evidence merge (and the moments kernel); their results do not depend on scheduling or on
+ * the SM count.  K, seed and stream are captured per submission.  Growing K beyond what any
+ * earlier call set lets the evaluations in flight finish first, then grows the per-slot index
+ * buffers (no evaluation allocates them).  TRI_EINVAL for K < 0 or K > TRI_MAX_POSTERIOR. */
+#define TRI_MAX_POSTERIOR (1 << 20)
+int tri_set_posterior(int64_t K, uint64_t seed, uint64_t stream);
+
+/* Posterior sample indices (ascending, local to the call's draws) of branch `branch` of the
+ * evaluation most recently returned by tri_eval_* / tri_eval_*_dev / tri_wait, copied to
+ * idx[0..*n).  *n = K, or 0 when posterior samples were off for it or the posterior is empty (a
+ * weight is +inf, or no weight is finite); *total = T, the sum of the weights relative to the
+ * branch's m (NaN when off, +inf or 0 when empty).  A submission keeps its samples until it is
+ * waited for.  TRI_EINVAL for a branch the evaluation does not have, or cap < K. */
+int tri_last_posterior(int32_t branch, int64_t* idx, int64_t cap, int64_t* n, double* total);
 
 /* sizeof() of the ABI structs, in the order tri_col, tri_tp_args, tri_eb_args, tri_result,
  * tri_powerlaw, tri_spline, tri_bound_prior, tri_sampler_args (the first n of them), so that a

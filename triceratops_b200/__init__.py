@@ -69,6 +69,18 @@ def mc_errors():
     return _dispatch.mc_errors()
 
 
+def posterior_samples(K, seed=0):
+    """Context manager: lnZ_* calls made inside it also draw K posterior samples of every
+    scenario branch, by systematic importance resampling of its prior draws on the GPU with
+    weights exp(lnL + lnprior).  Each result's `posterior` then holds them as a table (the
+    result keys plus `draw`, the global draw index), `post_total` their total weight.  lnZ,
+    the best-draw tables and numpy's generator are the same as without it.  Each call takes
+    the next stream of a counter that starts at 0 in each context; `seed` and the stream fix
+    the samples.  calc_probs(posterior_samples=K) uses it."""
+    from . import _dispatch
+    return _dispatch.posterior_samples(K, seed)
+
+
 def set_sampler(mode="host", seed=None):
     """Where the prior draws are made.
 

@@ -16,6 +16,7 @@ c_uint8_p = ctypes.POINTER(ctypes.c_uint8)
 TRI_OK, TRI_ECUDA, TRI_EINVAL, TRI_ESTATE, TRI_ENODEVICE = 0, -1, -2, -3, -4
 TRI_MAX_INFLIGHT = 4     # include/triceratops_b200.h
 TRI_MAX_CADENCES = 8     # include/triceratops_b200.h
+TRI_MAX_POSTERIOR = 1 << 20   # include/triceratops_b200.h
 
 
 class TriError(RuntimeError):
@@ -106,7 +107,7 @@ EXPORTS = ("tri_init", "tri_shutdown", "tri_last_error", "tri_set_lightcurve", "
            "tri_submit_tp", "tri_submit_eb", "tri_submit_tp_dev", "tri_submit_eb_dev", "tri_wait",
            "tri_dev_splev", "tri_set_counting", "tri_set_lightcurve_err", "tri_dev_sample",
            "tri_struct_sizes", "tri_set_lightcurve_cadence", "tri_set_moments",
-           "tri_last_moments")
+           "tri_last_moments", "tri_set_posterior", "tri_last_posterior")
 
 _lib = None
 
@@ -169,6 +170,9 @@ def load():
     L.tri_set_counting.argtypes = [ctypes.c_int32]
     L.tri_set_moments.argtypes = [ctypes.c_int32]
     L.tri_last_moments.argtypes = [c_double_p]
+    L.tri_set_posterior.argtypes = [ctypes.c_int64, ctypes.c_uint64, ctypes.c_uint64]
+    L.tri_last_posterior.argtypes = [ctypes.c_int32, ctypes.POINTER(ctypes.c_int64),
+                                     ctypes.c_int64, ctypes.POINTER(ctypes.c_int64), c_double_p]
     L.tri_dev_sample.argtypes = [ctypes.POINTER(tri_sampler_args), ctypes.c_void_p]
     L.tri_struct_sizes.argtypes = [ctypes.POINTER(ctypes.c_int64), ctypes.c_int32]
     L.tri_sm_count.argtypes = [ctypes.POINTER(ctypes.c_int32)]

@@ -21,6 +21,7 @@ import threading
 
 import numpy as np
 
+from . import _cabi, _numerics
 from . import engine as _engine_mod
 
 N_BEST = 100
@@ -124,11 +125,74 @@ def _sync_moments(eng):
         eng.set_moments(want)
 
 
+# ---- posterior samples (tri_set_posterior) ------------------------------------------------------
+_post = None      # [K, seed, next stream] inside posterior_samples() (process-wide)
+_post_lock = threading.Lock()
+
+
+def check_posterior_K(K):
+    """K as an int, or ValueError: an integer in [1, TRI_MAX_POSTERIOR]."""
+    if isinstance(K, bool) or not isinstance(K, (int, np.integer)):
+        raise ValueError("posterior_samples must be an integer, got %r" % (K,))
+    if not 1 <= int(K) <= _cabi.TRI_MAX_POSTERIOR:
+        raise ValueError("posterior_samples must be in [1, %d], got %d"
+                         % (_cabi.TRI_MAX_POSTERIOR, int(K)))
+    return int(K)
+
+
+@contextlib.contextmanager
+def posterior_samples(K, seed=0):
+    """Inside this context every scenario evaluation also draws K posterior samples per branch
+    (systematic importance resampling on the GPU).  Each engine call takes the next stream of a
+    per-context counter, unless the caller names it (call_stream)."""
+    global _post
+    K = check_posterior_K(K)
+    prev, _post = _post, [K, int(seed), 0]
+    try:
+        yield
+    finally:
+        _post = prev
+
+
+@contextlib.contextmanager
+def call_stream(stream):
+    """The stream of the posterior samples of the engine calls this thread makes inside."""
+    prev = getattr(_tls, "post_stream", None)
+    _tls.post_stream = int(stream)
+    try:
+        yield
+    finally:
+        _tls.post_stream = prev
+
+
+def _next_post():
+    """(K, seed, stream) of the engine call being submitted, None when posterior samples are
+    off."""
+    if _post is None:
+        return None
+    s = getattr(_tls, "post_stream", None)
+    if s is None:
+        with _post_lock:
+            s = _post[2]
+            _post[2] += 1
+    return _post[0], _post[1], s
+
+
+def _post_kw(eng, post):
+    """Switch the engine's posterior samples to `post` (engines without them -- test
+    stand-ins -- are left alone while they are off); the submission's keyword."""
+    if post is not None or getattr(eng, "_post_K", 0):
+        eng.set_posterior(post[0] if post else 0, post[1] if post else 0)
+    return {} if post is None else {"post_stream": post[2]}
+
+
 class Branch:
     """Globally combined result of one scenario branch: lnZ, its (m, s, s2, n_finite, n_posinf)
-    record (s2 None without moments), the best draws' indices and finite lnL values."""
+    record (s2 None without moments), the best draws' indices and finite lnL values; with
+    posterior samples, their global draw indices (ascending) and total weight relative to
+    exp(m), else None."""
     __slots__ = ("lnZ", "idx", "n_pass", "n_evaluated", "lnL_local", "lo", "hi", "N", "m", "s",
-                 "s2", "n_finite", "n_posinf", "vals")
+                 "s2", "n_finite", "n_posinf", "vals", "post_idx", "post_total")
 
 
 def _local_best(res, eng, single_rank):
@@ -177,10 +241,15 @@ def gather_records(records, N_total):
                                     N_total) for j in range(len(records))]
 
 
-def record_row(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals):
+def record_row(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals, post=None):
     """The 207-double record of a branch over one slice of draws (a rank's, or a round's of
-    refinement): header, then its best finite (lnL, global index) candidates; s2 None -> NaN."""
-    rec = np.full(H + 2 * N_BEST, np.nan)
+    refinement): header, then its best finite (lnL, global index) candidates; s2 None -> NaN.
+    With posterior samples, post = (K, T, global indices) appends [T, K indices] (NaN where
+    the posterior is empty)."""
+    rec = np.full(H + 2 * N_BEST + (0 if post is None else 1 + post[0]), np.nan)
+    if post is not None:
+        rec[H + 2 * N_BEST] = post[1]
+        rec[H + 2 * N_BEST + 1:H + 2 * N_BEST + 1 + len(post[2])] = post[2]
     rec[0:H] = (m, s, n_finite, n_posinf, n_pass, n_eval, np.nan if s2 is None else s2)
     idx, vals = np.asarray(idx), np.asarray(vals)
     fin = np.isfinite(vals)
@@ -191,18 +260,43 @@ def record_row(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals):
     return rec
 
 
-def _local_record(res, lo, eng):
+def _local_record(res, lo, eng, post=None):
     """This rank's record of one branch (zero-weight padding is not exchanged)."""
     local_best, local_vals, n_eval = _local_best(res, eng, False)
     return record_row(res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval,
-                      getattr(res, "s2", None), np.asarray(local_best) + lo, local_vals)
+                      getattr(res, "s2", None), np.asarray(local_best) + lo, local_vals,
+                      _local_post(res, lo, post))
 
 
-def _merge_records(allrec, lo, hi, N, lnL_local=None):
-    """[slices, 207] -> Branch: lnZ from the (m, s) records, best draws from the candidates.
-    The slices are ranks, or rounds of refinement (calc_probs)."""
+def _local_post(res, lo, post):
+    """(K, T, global indices) of a local result's posterior samples, None when off."""
+    idx = getattr(res, "post_idx", None)
+    if idx is None or post is None:
+        return None
+    return post[0], res.post_total, np.asarray(idx, dtype=np.int64) + lo
+
+
+def merge_record_posteriors(allrec, post, branch):
+    """(global indices, total weight relative to the merged maximum) of the posterior tails of
+    [slices, ...] records (record_row), merged in slice order; (None, None) without them."""
+    P = H + 2 * N_BEST
+    if post is None or allrec.shape[1] <= P:
+        return None, None
+    parts = []
+    for r in allrec:
+        t = r[P + 1:P + 1 + post[0]]
+        parts.append((r[0], r[P], t[~np.isnan(t)].astype(np.int64)))
+    idx, _, W = _numerics.merge_posteriors(parts, post[0], post[1], post[2], branch)
+    return idx, W
+
+
+def _merge_records(allrec, lo, hi, N, lnL_local=None, post=None, branch=0):
+    """[slices, 207] -> Branch: lnZ from the (m, s) records, best draws from the candidates,
+    posterior samples (post = (K, seed, stream) of the call) from the records' tails.  The
+    slices are ranks, or rounds of refinement (calc_probs)."""
     br = Branch()
     br.lo, br.hi, br.lnL_local, br.N = lo, hi, lnL_local, N
+    br.post_idx, br.post_total = merge_record_posteriors(allrec, post, branch)
     parts = [(r[0], r[1], int(r[2]), int(r[3])) for r in allrec]
     br.lnZ = _engine_mod.combine_lse(parts, N)
     br.n_pass = int(sum(r[4] for r in allrec))
@@ -229,7 +323,7 @@ def _merge_records(allrec, lo, hi, N, lnL_local=None):
     return br
 
 
-def _gather_branch(res, lo, hi, N, eng=None):
+def _gather_branch(res, lo, hi, N, eng=None, post=None, branch=0):
     """Merge per-rank results of one branch right away (a single lnZ_* call)."""
     d = _dist()
     if d is None:
@@ -240,9 +334,12 @@ def _gather_branch(res, lo, hi, N, eng=None):
         br.lnZ, br.n_pass = res.lnZ, res.n_pass
         br.m, br.s, br.n_finite, br.n_posinf = res.m, res.s, res.n_finite, res.n_posinf
         br.s2 = getattr(res, "s2", None)
+        lp = _local_post(res, lo, post)
+        br.post_idx, br.post_total = (None, None) if lp is None else (lp[2], lp[1])
         return br
-    rec = _local_record(res, lo, eng)
-    return _merge_records(_allgather(rec[None, :], d)[:, 0, :], lo, hi, N, res.lnL)
+    rec = _local_record(res, lo, eng, post)
+    return _merge_records(_allgather(rec[None, :], d)[:, 0, :], lo, hi, N, res.lnL, post,
+                          branch)
 
 
 # ---- one exchange per calc_probs ----------------------------------------------------------------
@@ -309,6 +406,7 @@ class CallGroup:
         if hdr["scalar_loop"]:
             kw["scalar_loop"] = True
         _sync_moments(eng)
+        kw.update(_post_kw(eng, hdr["post"]))
         fn = getattr(eng, "submit_" + name, None)
         if fn is not None:
             return fn(n, cols, lightcurve=lc, **kw)
@@ -317,7 +415,8 @@ class CallGroup:
                 eng.set_lightcurve(*lc)
             return _Done(getattr(eng, "eval_" + name)(n, cols, **kw))
 
-    def scatter_submit(self, eng, kind, N, cols, extra_mask, is_host, scalar_loop=False):
+    def scatter_submit(self, eng, kind, N, cols, extra_mask, is_host, scalar_loop=False,
+                       post=None):
         """Rank 0: announce one engine call, scatter its per-draw columns, evaluate the own
         slice.  Returns (pending, lo, hi, seq)."""
         import torch
@@ -342,7 +441,8 @@ class CallGroup:
             self.lc_key = key
             hdr = dict(op="call", seq=seq, kind=kind, N=N, arrays=arrays, scalars=scalars,
                        absent=absent, has_mask=extra_mask is not None, is_host=bool(is_host),
-                       scalar_loop=bool(scalar_loop), bounds=bounds, chunk=chunk, ncol=ncol, lc=send_lc)
+                       scalar_loop=bool(scalar_loop), bounds=bounds, chunk=chunk, ncol=ncol, lc=send_lc,
+                       post=post)
             self._bcast(hdr)
             pin = self.device == "cuda"
             buf = torch.zeros((self.world, max(ncol, 1), chunk), dtype=torch.float64,
@@ -390,7 +490,7 @@ class CallGroup:
             res = pending.result()
             lo = hdr["bounds"][self.rank]
             for b, r in enumerate(res if isinstance(res, tuple) else (res,)):
-                self.add(_local_record(r, lo, eng), ("s", hdr["seq"], b))
+                self.add(_local_record(r, lo, eng, hdr["post"]), ("s", hdr["seq"], b))
         self.exchange()
         return self._bcast()
 
@@ -448,9 +548,10 @@ class _Done:
         return self._out
 
 
-def _submit(eng, name, *args, **kw):
+def _submit(eng, name, *args, post=None, **kw):
     lc = current_lightcurve()
     _sync_moments(eng)
+    kw.update(_post_kw(eng, post))
     fn = getattr(eng, "submit_" + name, None)
     if fn is not None:
         return fn(*args, lightcurve=lc, **kw)
@@ -466,8 +567,9 @@ class PendingBranches:
     Branch (TP-type) or the (EB, EBx2P) pair -- right away with its own collective for a single
     lnZ_* call, after the group's one exchange inside calc_probs.  Both are idempotent."""
 
-    def __init__(self, pending, lo, hi, N, eng, seq=None):
+    def __init__(self, pending, lo, hi, N, eng, seq=None, post=None):
         self._pending, self._lo, self._hi, self._N, self._eng = pending, lo, hi, N, eng
+        self._post = post
         self._seq, self._group = seq, _group
         self._res = self._keys = self._out = None
         self._lock = threading.Lock()
@@ -481,7 +583,7 @@ class PendingBranches:
                 self._pending = None
                 g = self._group
                 if g is not None:
-                    self._keys = [g.add(_local_record(r, self._lo, self._eng),
+                    self._keys = [g.add(_local_record(r, self._lo, self._eng, self._post),
                                         None if self._seq is None else ("s", self._seq, b))
                                   for b, r in enumerate(self._res)]
 
@@ -491,11 +593,13 @@ class PendingBranches:
             if self._out is None:
                 g = self._group
                 if g is None:
-                    out = [_gather_branch(r, self._lo, self._hi, self._N, self._eng)
-                           for r in self._res]
+                    out = [_gather_branch(r, self._lo, self._hi, self._N, self._eng,
+                                          self._post, b)
+                           for b, r in enumerate(self._res)]
                 else:
-                    out = [_merge_records(g.rows(k), self._lo, self._hi, self._N, r.lnL)
-                           for k, r in zip(self._keys, self._res)]
+                    out = [_merge_records(g.rows(k), self._lo, self._hi, self._N, r.lnL,
+                                          self._post, b)
+                           for b, (k, r) in enumerate(zip(self._keys, self._res))]
                 self._out = tuple(out) if self._tuple else out[0]
         return self._out
 
@@ -503,19 +607,21 @@ class PendingBranches:
 def _submit_sharded(kind, N, cols, extra_mask, companion_is_host, scalar_loop=False):
     eng = get_engine()
     g = _group
+    post = _next_post()
     if g is not None and g.scatter:
         # calc_probs under a process group, numpy draws: this is rank 0 (the others follow)
         pending, lo, hi, seq = g.scatter_submit(eng, kind, N, cols, extra_mask,
-                                                companion_is_host, scalar_loop)
-        return PendingBranches(pending, lo, hi, N, eng, seq)
+                                                companion_is_host, scalar_loop, post)
+        return PendingBranches(pending, lo, hi, N, eng, seq, post)
     lo, hi = shard_bounds(N)
     sl = {k: _slice(v, lo, hi) for k, v in cols.items()}
     lnprior = sl.pop("lnprior")
     kw = {"scalar_loop": True} if scalar_loop else {}
     p = _submit(eng, kind, hi - lo, *sl.values(), lnprior=lnprior,
                 extra_mask=_mask_slice(extra_mask, lo, hi),
-                companion_is_host=companion_is_host, want_lnL=False, n_best=N_BEST, **kw)
-    return PendingBranches(p, lo, hi, N, eng)
+                companion_is_host=companion_is_host, want_lnL=False, n_best=N_BEST, post=post,
+                **kw)
+    return PendingBranches(p, lo, hi, N, eng, post=post)
 
 
 def submit_tp(N, rp, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr, lnprior=None,
@@ -679,8 +785,11 @@ class TableExchange:
     themselves live on the rank that made them), merged across ranks by `result()` -- with the
     CallGroup's one exchange inside calc_probs, with its own all-gather otherwise."""
 
-    def __init__(self, lb, table, keys):
+    def __init__(self, lb, table, keys, post=None):
+        """post: ((K, seed, stream) of the call, branch, this rank's posterior table -- the
+        keys and `draw`, global draw indices) or None without posterior samples."""
         self.lb, self.keys = lb, keys
+        self.post = post
         res = lb.res
         self.n_eval = int(res.n_evaluated) if res.n_evaluated is not None else int(len(lb.idx))
         self.rows = np.stack([np.asarray(table[k], dtype=np.float64) for k in keys], axis=1) \
@@ -689,7 +798,16 @@ class TableExchange:
         self.s2 = getattr(res, "s2", None)
         if _dist() is not None:
             W = H + N_BEST * (1 + len(keys))
+            if post is not None:   # tail: T, K draw indices, K rows (NaN where empty)
+                W += 1 + post[0][0] * (1 + len(keys))
             rec = np.full(W, np.nan)
+            if post is not None:
+                P, pt = H + N_BEST * (1 + len(keys)), post[2]
+                n = len(pt["draw"])
+                rec[P] = res.post_total
+                rec[P + 1:P + 1 + n] = pt["draw"]
+                rec[P + 1 + post[0][0]:P + 1 + post[0][0] + n * len(keys)] = np.stack(
+                    [np.asarray(pt[k], dtype=np.float64) for k in keys], axis=1).ravel()
             rec[0:H] = (res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, self.n_eval,
                         np.nan if self.s2 is None else self.s2)
             k = len(lb.vals)
@@ -707,6 +825,9 @@ class TableExchange:
         vals, rows, n_eval = lb.vals, self.rows, self.n_eval
         d = _dist()
         self.top = None
+        self.posterior = self.post_total = None
+        if d is None and self.post is not None:
+            self.posterior, self.post_total = self.post[2], res.post_total
         if d is None:
             lnZ, n_pass = res.lnZ, int(res.n_pass)
             self.record = (res.m, res.s, self.s2, res.n_finite, res.n_posinf)
@@ -722,6 +843,8 @@ class TableExchange:
             m, s, s2, n_fin, n_pinf = _engine_mod.combine_moments(
                 [(r[0], r[1], r[6], r[2], r[3]) for r in allrec])
             self.record = (m, s, None if np.isnan(allrec[:, 6]).any() else s2, n_fin, n_pinf)
+            if self.post is not None:
+                self._merge_posterior(allrec)
             vs, rs = [], []
             for r in allrec:
                 v = r[H:H + N_BEST]
@@ -737,3 +860,21 @@ class TableExchange:
             pad = rows[-1:] if len(rows) else np.zeros((1, len(keys)))
             rows = np.concatenate([rows, np.repeat(pad, N_BEST - len(rows), axis=0)])
         return lnZ, n_pass, n_eval, {k: rows[:, i].copy() for i, k in enumerate(keys)}
+
+    def _merge_posterior(self, allrec):
+        """Posterior table of the whole branch from the ranks' record tails (rank order)."""
+        (K, seed, stream), branch, nk = self.post[0], self.post[1], len(self.keys)
+        P = H + N_BEST * (1 + nk)
+        parts, draws, rows = [], [], []
+        for r in allrec:
+            dr = r[P + 1:P + 1 + K]
+            n = int((~np.isnan(dr)).sum())
+            parts.append((r[0], r[P], dr[:n].astype(np.int64)))
+            draws.append(dr[:n].astype(np.int64))
+            rows.append(r[P + 1 + K:P + 1 + K + n * nk].reshape(n, nk))
+        idx, _, W = _numerics.merge_posteriors(parts, K, seed, stream, branch)
+        draws, rows = np.concatenate(draws), np.concatenate(rows)
+        pos = np.searchsorted(draws, idx)      # (slices are disjoint and ascending)
+        self.posterior = {k: rows[pos, i] for i, k in enumerate(self.keys)}
+        self.posterior["draw"] = idx
+        self.post_total = W

@@ -129,3 +129,81 @@ def probability_errors(lnZ, r, calls, N_calls, fpp_rows=(0, 3, 9), nfpp_from=15)
         g = sum_gradient(Z, range(nfpp_from, n))
         nfpp_err = float(np.sqrt(max(g @ V @ g, 0.0)))
     return prob_err, fpp_err, nfpp_err, contrib
+
+
+# ---- posterior samples: systematic importance resampling ----------------------------------------
+# For one slice of draws, sample k < K is draw min{i : C_i > (U + k) T / K}, with C the prefix sums
+# of w_i = exp(lnw_i - m) in draw order and T = C_{N-1} (tri_set_posterior).  U in [0, 1) is a
+# hash of (seed, stream, salt), so that no state is taken from numpy's global generator.  Salts:
+# 2 j + branch, with j = 0 for the GPU's own resampling of a slice, j = 1 for the allocation of
+# merge_posteriors and j = 2 + r for its thinning of slice r.
+_M64 = (1 << 64) - 1
+
+
+def _splitmix64(x):
+    x = (x + 0x9E3779B97F4A7C15) & _M64
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & _M64
+    return x ^ (x >> 31)
+
+
+def posterior_uniform(seed, stream, salt):
+    """U in [0, 1) from (seed, stream, salt): three splitmix64 steps, the top 53 bits times
+    2^-53.  posterior_select_kernel computes the same bits."""
+    h = _splitmix64(int(seed) & _M64)
+    h = _splitmix64(h ^ (int(stream) & _M64))
+    h = _splitmix64(h ^ (int(salt) & _M64))
+    return (h >> 11) * 2.0 ** -53
+
+
+def _systematic_counts(U, W, K, edges):
+    """Number of positions (U + k) W / K, k < K, below each of the non-decreasing `edges`."""
+    step = W / K
+    u = (U + np.arange(K, dtype=np.float64)) * step
+    return np.searchsorted(u, np.asarray(edges, dtype=np.float64), side="left")
+
+
+def merge_posteriors(parts, K, seed, stream, branch=0):
+    """Merge the K-sample posteriors of disjoint slices of draws, in slice order (ranks in rank
+    order, or rounds of refinement).  parts: (m_r, T_r, idx_r) per slice -- the slice's record
+    maximum, its sum of weights relative to exp(m_r), its K sample indices (global, ascending;
+    None when the slice had posterior samples off).
+
+    With m = max m_r and W_r = T_r exp(m_r - m), slice r gets c_r of the K merged samples, the
+    number of positions (U_0 + k) W / K in [sum_{r'<r} W_r', sum_{r'<=r} W_r') (so c_r is
+    floor or ceil of K W_r / W), and contributes its samples at positions floor((j + U_r) K /
+    c_r), j < c_r.  Each draw then has K w_i / W expected copies, as from one slice of all the
+    draws; a sharded run gives the same distribution as one rank, not the same bits.  One slice
+    is returned unchanged.  Returns (idx, m, W): empty idx when a T_r is +inf or no weight is
+    finite, None when a slice had samples off."""
+    K = int(K)
+    if any(p[2] is None for p in parts):
+        return None, np.nan, np.nan
+    if any(np.isposinf(p[1]) for p in parts):
+        return np.zeros(0, dtype=np.int64), np.nan, np.inf
+    live = [p for p in parts if p[1] > 0 and len(p[2])]
+    if not live:
+        return np.zeros(0, dtype=np.int64), -np.inf, 0.0
+    m = max(p[0] for p in live)
+    if len(parts) == 1:
+        return np.asarray(parts[0][2], dtype=np.int64), m, float(parts[0][1])
+    Wr = np.array([p[1] * np.exp(p[0] - m) if (p[1] > 0 and len(p[2])) else 0.0
+                   for p in parts])
+    cum = np.cumsum(Wr)
+    W = float(cum[-1])
+    ends = _systematic_counts(posterior_uniform(seed, stream, 2 + branch), W, K, cum)
+    # (positions that rounding left at or above W: the last slice of positive weight)
+    ends[int(np.flatnonzero(Wr > 0)[-1]):] = K
+    c = np.diff(np.concatenate([[0], ends]))
+    out = []
+    for r, (p, cr) in enumerate(zip(parts, c)):
+        if cr == 0:
+            continue
+        idx = np.asarray(p[2], dtype=np.int64)
+        if cr >= len(idx):
+            out.append(idx)
+            continue
+        U = posterior_uniform(seed, stream, 2 * (2 + r) + branch)
+        pos = np.floor((np.arange(cr) + U) * (len(idx) / cr)).astype(np.int64)
+        out.append(idx[np.minimum(pos, len(idx) - 1)])
+    return np.concatenate(out), m, W

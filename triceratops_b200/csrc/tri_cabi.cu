@@ -145,9 +145,12 @@ struct Slot {
     HostArena pinned;   // pinned copies of pageable host columns, on their way to `staging`
     unsigned long long* d_counters = nullptr;  // [8]
     unsigned long long* h_counters = nullptr;  // pinned [8]
-    LsePartial* d_lse_out = nullptr;           // [2], then s2 of the two branches (kLseOutBytes)
-    LsePartial* h_lse_out = nullptr;           // pinned, same layout
+    LsePartial* d_lse_out = nullptr;           // [2], then s2 and T of the two branches
+    LsePartial* h_lse_out = nullptr;           // pinned, same layout (kLseOutBytes)
     unsigned int* d_mom_done = nullptr;        // moments_kernel's block counter
+    unsigned int* d_post_done = nullptr;       // [2] posterior_sums_kernel's block counters
+    int64_t* d_post_idx[2] = {nullptr, nullptr};   // [g.post_cap] posterior samples per branch
+    int64_t* h_post_idx[2] = {nullptr, nullptr};   // pinned landing zone, same size
     TopkState* d_topk = nullptr;               // [2]
     TopkState* h_topk = nullptr;               // pinned [2]
     unsigned int* d_hist16 = nullptr;          // [2][kTopkBins], zero between calls
@@ -160,6 +163,9 @@ struct Slot {
     int64_t N = 0;
     bool moments = false; // tri_set_moments at submission: s2 follows the records
     double s2[2] = {NAN, NAN};
+    int64_t post_K = 0;   // tri_set_posterior at submission (0: off)
+    unsigned long long post_seed = 0, post_stream = 0;
+    double post_T[2] = {NAN, NAN};
     bool host = false;    // host-buffer call: best-draw candidates are sorted in tri_wait
     bool want_top[2] = {false, false};
     tri_result want[2];   // the caller's records: its pointers go back into the results
@@ -196,10 +202,22 @@ struct Ctx {
     int64_t next_ticket = 1;
     Slot* last = nullptr;    // the call completed last (tri_last_timing, tri_fetch_lnl)
     double last_s2[2] = {NAN, NAN};   // s2 of the evaluation tri_wait returned last
+    // posterior samples (tri_set_posterior): K of the next submissions, and the capacity of
+    // every slot's index buffers (grown only by tri_set_posterior)
+    int64_t post_K = 0, post_cap = 0;
+    unsigned long long post_seed = 0, post_stream = 0;
+    // the samples of the evaluation tri_wait returned last: its slot's pinned buffers are
+    // swapped in here, so that the slot can be reused at once
+    int64_t* h_post_last[2] = {nullptr, nullptr};
+    int64_t last_post_K = 0;
+    int last_branches = 0;
+    double last_post_T[2] = {NAN, NAN};
 };
 
-// d_lse_out / h_lse_out: the branches' evidence records, then their s2 (moments_kernel)
-constexpr size_t kLseOutBytes = 2 * sizeof(LsePartial) + 2 * sizeof(double);
+// d_lse_out / h_lse_out: the branches' evidence records, then their s2 (moments_kernel), then
+// their T (posterior_sums_kernel)
+constexpr size_t kLseS2Bytes = 2 * sizeof(LsePartial) + 2 * sizeof(double);
+constexpr size_t kLseOutBytes = kLseS2Bytes + 2 * sizeof(double);
 
 Ctx g;
 
@@ -272,6 +290,8 @@ int lse_blocks(int64_t N) {
     return (int)std::max<int64_t>(1, std::min<int64_t>(b, 4 * (int64_t)g.sm_count));
 }
 
+int64_t post_tiles(int64_t N) { return (N + kPostTile - 1) / kPostTile; }
+
 size_t scratch_bytes(int64_t N, bool eb) {
     size_t n = (size_t)N;
     size_t b = 0;
@@ -279,6 +299,7 @@ size_t scratch_bytes(int64_t N, bool eb) {
     b += (n * 8 + 256) * 2;              // items, cval
     b += (size_t)lnl_grid() * sizeof(LsePartial) * 2 + 512;
     b += (size_t)lse_blocks(N) * sizeof(double) * 2 + 256;   // moments_kernel partials
+    if (g.post_K > 0) b += (size_t)(2 * post_tiles(N) + 1) * sizeof(double) * 2 + 512;
     return b + 4096;
 }
 
@@ -350,6 +371,50 @@ int launch_moments(Slot& S, const Scratch& W, int64_t N, int branches, Col lnpri
     return TRI_OK;
 }
 
+// posterior samples of the call's branches after finalize_kernel (and moments_kernel): tile sums
+// and offsets, then the selection; the indices travel to the slot's pinned landing zone
+int launch_posterior(Slot& S, const Scratch& W, int64_t N, int branches, Col lnprior,
+                     cudaStream_t s) {
+    PosteriorArgs P{};
+    P.lnl[0] = W.lnl;
+    P.lnl[1] = W.lnl_twin;
+    P.lnprior = lnprior;
+    P.N = N;
+    P.tiles = post_tiles(N);
+    P.lse = S.d_lse_out;
+    P.tile_sum = S.scratch.take<double>(2 * (size_t)P.tiles);
+    P.tile_off = S.scratch.take<double>(2 * (size_t)(P.tiles + 1));
+    P.done = S.d_post_done;
+    P.total = reinterpret_cast<double*>(S.d_lse_out + 2) + 2;
+    P.idx[0] = S.d_post_idx[0];
+    P.idx[1] = S.d_post_idx[1];
+    P.K = S.post_K;
+    P.seed = S.post_seed;
+    P.stream = S.post_stream;
+    dim3 grid((unsigned)P.tiles, (unsigned)branches);
+    posterior_sums_kernel<<<grid, kPostThreads, 0, s>>>(P);
+    CU(cudaGetLastError());
+    posterior_select_kernel<<<grid, kPostThreads, 0, s>>>(P);
+    S.launches += 2;
+    CU(cudaGetLastError());
+    for (int b = 0; b < branches; ++b)
+        CU(cudaMemcpyAsync(S.h_post_idx[b], S.d_post_idx[b], (size_t)S.post_K * sizeof(int64_t),
+                           cudaMemcpyDeviceToHost, s));
+    return TRI_OK;
+}
+
+// bytes of d_lse_out that a call's read-back needs
+size_t lse_out_bytes(const Slot& S, int branches) {
+    return S.post_K > 0 ? kLseOutBytes : S.moments ? kLseS2Bytes
+                                                   : branches * sizeof(LsePartial);
+}
+
+void capture_posterior(Slot& S) {
+    S.post_K = g.post_K;
+    S.post_seed = g.post_seed;
+    S.post_stream = g.post_stream;
+}
+
 // Queue one TP-type evaluation on `s` for slot S: every pointer in `a` and in `r` (lnL_out,
 // mask_out, top_idx, top_lnL) is a device pointer.  Nothing here waits for the GPU; the small
 // result record lands in the slot's pinned buffers and is read by finish_slot.
@@ -403,11 +468,16 @@ int enqueue_tp(Slot& S, const tri_tp_args& a, const tri_result& r, cudaStream_t 
         rc = launch_moments(S, W, N, 1, to_col(a.lnprior), s);
         if (rc) return rc;
     }
+    capture_posterior(S);
+    if (S.post_K > 0) {
+        rc = launch_posterior(S, W, N, 1, to_col(a.lnprior), s);
+        if (rc) return rc;
+    }
     CU(cudaMemcpyAsync(S.h_topk, S.d_topk, sizeof(TopkState), cudaMemcpyDeviceToHost, s));
     S.lnl[0] = W.lnl; S.lnl[1] = nullptr;
     CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, S.moments ? kLseOutBytes : sizeof(LsePartial),
-                       cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, lse_out_bytes(S, 1), cudaMemcpyDeviceToHost,
+                       s));
     CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
                        cudaMemcpyDeviceToHost, s));
     return TRI_OK;
@@ -470,11 +540,15 @@ int enqueue_eb(Slot& S, const tri_eb_args& a, const tri_result r[2], cudaStream_
         rc = launch_moments(S, W, N, 2, to_col(a.lnprior), s);
         if (rc) return rc;
     }
+    capture_posterior(S);
+    if (S.post_K > 0) {
+        rc = launch_posterior(S, W, N, 2, to_col(a.lnprior), s);
+        if (rc) return rc;
+    }
     CU(cudaMemcpyAsync(S.h_topk, S.d_topk, 2 * sizeof(TopkState), cudaMemcpyDeviceToHost, s));
     S.lnl[0] = W.lnl; S.lnl[1] = W.lnl_twin;
     CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out,
-                       S.moments ? kLseOutBytes : 2 * sizeof(LsePartial), cudaMemcpyDeviceToHost,
+    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, lse_out_bytes(S, 2), cudaMemcpyDeviceToHost,
                        s));
     CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
                        cudaMemcpyDeviceToHost, s));
@@ -497,6 +571,8 @@ void finish_slot(Slot& S, tri_result* out) {
     const double* h_s2 = reinterpret_cast<const double*>(S.h_lse_out + 2);
     for (int b = 0; b < 2; ++b)
         S.s2[b] = !S.moments || b >= S.branches ? NAN : S.N == 0 ? 0.0 : h_s2[b];
+    for (int b = 0; b < 2; ++b)   // (N == 0: no draw, an empty posterior)
+        S.post_T[b] = S.post_K == 0 || b >= S.branches ? NAN : S.N == 0 ? 0.0 : h_s2[2 + b];
     for (int b = 0; b < S.branches; ++b) {
         tri_result r = S.want[b];   // keeps the caller's pointers and top_cap
         if (S.N == 0) {
@@ -605,7 +681,10 @@ int check_eb(const tri_eb_args* a, const void* out) {
 // mark the slot in flight and hand out its ticket
 void commit(Slot& S, int branches, int64_t N, bool host, const tri_result* want,
             int64_t* ticket) {
-    if (N == 0) S.moments = g.moments;   // (no kernels: enqueue_* did not run)
+    if (N == 0) {   // (no kernels: enqueue_* did not run)
+        S.moments = g.moments;
+        capture_posterior(S);
+    }
     S.branches = branches;
     S.N = N;
     S.host = host;
@@ -663,6 +742,8 @@ int tri_init(int device) {
         CU(cudaMallocHost(&S.h_lse_out, kLseOutBytes));
         CU(cudaMalloc(&S.d_mom_done, sizeof(unsigned int)));
         CU(cudaMemset(S.d_mom_done, 0, sizeof(unsigned int)));
+        CU(cudaMalloc(&S.d_post_done, 2 * sizeof(unsigned int)));
+        CU(cudaMemset(S.d_post_done, 0, 2 * sizeof(unsigned int)));
         CU(cudaMallocHost(&S.h_counters, 8 * sizeof(unsigned long long)));
         CU(cudaMalloc(&S.d_topk, 2 * sizeof(TopkState)));
         CU(cudaMalloc(&S.d_hist16, 2 * (size_t)kTopkBins * sizeof(unsigned int)));
@@ -697,6 +778,7 @@ int tri_shutdown(void) {
         cudaFree(S.d_lse_out);
         cudaFreeHost(S.h_lse_out);
         cudaFree(S.d_mom_done);
+        cudaFree(S.d_post_done);
         cudaFreeHost(S.h_counters);
         cudaFree(S.d_topk);
         cudaFree(S.d_hist16);
@@ -707,11 +789,15 @@ int tri_shutdown(void) {
         for (int b = 0; b < 2; ++b) {
             if (S.h_tidx[b]) cudaFreeHost(S.h_tidx[b]);
             if (S.h_tval[b]) cudaFreeHost(S.h_tval[b]);
+            if (S.d_post_idx[b]) cudaFree(S.d_post_idx[b]);
+            if (S.h_post_idx[b]) cudaFreeHost(S.h_post_idx[b]);
         }
         for (auto& ev : S.ev) cudaEventDestroy(ev);
         cudaEventDestroy(S.copied);
         cudaEventDestroy(S.done);
     }
+    for (int b = 0; b < 2; ++b)
+        if (g.h_post_last[b]) cudaFreeHost(g.h_post_last[b]);
     cudaStreamDestroy(g.copy_stream);
     cudaStreamDestroy(g.stream);
     g = Ctx{};
@@ -747,6 +833,69 @@ int tri_last_moments(double s2[2]) {
     if (!s2) return fail(TRI_EINVAL, "NULL argument");
     s2[0] = g.last_s2[0];
     s2[1] = g.last_s2[1];
+    return TRI_OK;
+}
+
+// Grow the index buffers of every slot (and the landing zone of the last result) to K per
+// branch.  The evaluations in flight finish first; the indices they already returned move over.
+static int grow_posterior(int64_t K) {
+    CU(cudaDeviceSynchronize());
+    auto grow_host = [&](int64_t*& p) -> int {
+        int64_t* q = nullptr;
+        CU(cudaMallocHost(&q, (size_t)K * sizeof(int64_t)));
+        if (p) {
+            std::memcpy(q, p, (size_t)g.post_cap * sizeof(int64_t));
+            cudaFreeHost(p);
+        }
+        p = q;
+        return TRI_OK;
+    };
+    for (int i = 0; i < kSlots; ++i) {
+        Slot& S = g.slots[i];
+        for (int b = 0; b < 2; ++b) {
+            if (S.d_post_idx[b]) cudaFree(S.d_post_idx[b]);
+            S.d_post_idx[b] = nullptr;
+            CU(cudaMalloc(&S.d_post_idx[b], (size_t)K * sizeof(int64_t)));
+            int rc = grow_host(S.h_post_idx[b]);
+            if (rc) return rc;
+        }
+    }
+    for (int b = 0; b < 2; ++b) {
+        int rc = grow_host(g.h_post_last[b]);
+        if (rc) return rc;
+    }
+    g.post_cap = K;
+    return TRI_OK;
+}
+
+int tri_set_posterior(int64_t K, uint64_t seed, uint64_t stream) {
+    int rc = need_ready(false);
+    if (rc) return rc;
+    if (K < 0 || K > TRI_MAX_POSTERIOR)
+        return fail(TRI_EINVAL, "posterior sample count K must be in [0, TRI_MAX_POSTERIOR]");
+    CU(cudaSetDevice(g.device));
+    if (K > g.post_cap) {
+        rc = grow_posterior(K);
+        if (rc) return rc;
+    }
+    g.post_K = K;
+    g.post_seed = seed;
+    g.post_stream = stream;
+    return TRI_OK;
+}
+
+int tri_last_posterior(int32_t branch, int64_t* idx, int64_t cap, int64_t* n, double* total) {
+    int rc = need_ready(false);
+    if (rc) return rc;
+    if (!n || !total || (!idx && cap > 0)) return fail(TRI_EINVAL, "NULL argument");
+    if (branch < 0 || branch > 1 || (g.last_branches > 0 && branch >= g.last_branches))
+        return fail(TRI_EINVAL, "bad branch");
+    const double T = g.last_post_T[branch];
+    const int64_t k = g.last_post_K > 0 && T > 0.0 && std::isfinite(T) ? g.last_post_K : 0;
+    if (cap < k) return fail(TRI_EINVAL, "cap is smaller than the posterior sample count");
+    if (k) std::memcpy(idx, g.h_post_last[branch], (size_t)k * sizeof(int64_t));
+    *n = k;
+    *total = T;
     return TRI_OK;
 }
 
@@ -1160,6 +1309,12 @@ int tri_wait(int64_t ticket, tri_result* out) {
     g.last = S;
     g.last_s2[0] = S->s2[0];
     g.last_s2[1] = S->s2[1];
+    g.last_branches = S->branches;
+    g.last_post_K = S->post_K;
+    for (int b = 0; b < 2; ++b) {
+        g.last_post_T[b] = S->post_T[b];
+        if (S->post_K > 0) std::swap(S->h_post_idx[b], g.h_post_last[b]);
+    }
     if (S->host && S->N > 0) {   // per-draw outputs (parity runs): copied now, synchronously
         for (int b = 0; b < S->branches; ++b) {
             if (S->d_out_lnl[b])

@@ -1347,6 +1347,173 @@ __global__ void __launch_bounds__(kMomThreads) moments_kernel(MomentsArgs M) {
     if (threadIdx.x == 0) *M.done = 0u;
 }
 
+// ---- posterior samples: systematic importance resampling (tri_set_posterior) -------------------
+// Weights w_i = exp(x_i - m) with x_i = lnL_i + lnprior_i formed as lnl_kernel's epilogue forms it
+// and m the branch's maximum from finalize_kernel (0 where x_i is not finite).  C_i is the
+// inclusive prefix sum of w in draw order, T = C_{N-1}, u_k = (U + k) * (T / K) for k < K, and
+// sample k is draw min{i : C_i > u_k}; positions at or above T go to the last draw at which C
+// increases (the last draw of positive weight, unless rounding absorbed its weight).
+//
+// The draws are cut into tiles of kPostTile = 256 threads x 16 contiguous draws, independent of
+// the SM count.  Inside a tile every sum is a serial chain: over a thread's 16 draws, over the 32
+// thread totals of a warp, over the 8 warp totals; posterior_sums_kernel chains the tile totals in
+// tile order.  So the last prefix a thread computes is, bit for bit, the start the next thread
+// (or tile) computes, and the intervals [C_{i-1}, C_i) tile [0, T) with neither gap nor overlap:
+// posterior_select_kernel writes every idx[k] exactly once, without atomics.
+constexpr int kPostThreads = 256;
+constexpr int kPostPer = 16;
+constexpr int64_t kPostTile = (int64_t)kPostThreads * kPostPer;
+
+struct PosteriorArgs {
+    const double* lnl[2];         // per-draw lnL of branch 0 / 1 (-inf where not evaluated)
+    Col lnprior;                  // ptr nullptr: none
+    int64_t N;
+    int64_t tiles;                // ceil(N / kPostTile) = gridDim.x
+    const LsePartial* lse;        // [branches] evidence records of finalize_kernel
+    double* tile_sum;             // [2][tiles]
+    double* tile_off;             // [2][tiles + 1]: exclusive offsets, then T
+    unsigned int* done;           // [2] block counters, 0 between launches
+    double* total;                // [branches] T (+inf: a weight is +inf; 0: none finite)
+    int64_t* idx[2];              // [K] sample -> draw, per branch
+    int64_t K;
+    unsigned long long seed, stream;
+};
+
+__device__ __forceinline__ unsigned long long splitmix64(unsigned long long x) {
+    x += 0x9E3779B97F4A7C15ull;
+    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+    return x ^ (x >> 31);
+}
+
+// U in [0, 1): _numerics.posterior_uniform(seed, stream, salt), bit for bit
+__device__ __forceinline__ double posterior_uniform(unsigned long long seed,
+                                                    unsigned long long stream,
+                                                    unsigned long long salt) {
+    unsigned long long h = splitmix64(seed);
+    h = splitmix64(h ^ stream);
+    h = splitmix64(h ^ salt);
+    return (double)(h >> 11) * 0x1.0p-53;
+}
+
+// This thread's 16 inclusive prefix sums l[] (serial, from 0) and its start in the tile,
+// start = Wb + E (E: serial chain of the warp's earlier thread totals, Wb: of the block's earlier
+// warp totals); the tile-local C of draw j is start-sum Wb + (E + l[j]).  Returns the tile total.
+__device__ __forceinline__ double post_tile_scan(const PosteriorArgs& P, int b, int64_t tile,
+                                                 double m, bool live, double (&l)[kPostPer],
+                                                 double& wb, double& e, double* sh_warp) {
+    const double* lnl = b ? P.lnl[1] : P.lnl[0];   // (constant indices: no stack copy)
+    const int64_t base = tile * kPostTile + (int64_t)threadIdx.x * kPostPer;
+    double acc = 0.0;
+#pragma unroll
+    for (int j = 0; j < kPostPer; ++j) {
+        const int64_t i = base + j;
+        double w = 0.0;
+        if (live && i < P.N) {
+            double x = lnl[i];
+            if (P.lnprior.p) x += P.lnprior.at(i);
+            if (isfinite(x)) w = exp(x - m);
+        }
+        acc += w;
+        l[j] = acc;
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double chain = 0.0;
+    e = 0.0;
+    for (int q = 0; q < 32; ++q) {
+        const double t = __shfl_sync(0xffffffffu, acc, q);
+        if (q == lane) e = chain;
+        chain += t;
+    }
+    if (lane == 0) sh_warp[warp] = chain;
+    __syncthreads();
+    double tot = 0.0;
+    wb = 0.0;
+    for (int q = 0; q < kPostThreads / 32; ++q) {
+        if (q == warp) wb = tot;
+        tot += sh_warp[q];
+    }
+    __syncthreads();
+    return tot;
+}
+
+__device__ __forceinline__ bool post_empty(const LsePartial& r) {
+    return r.n_posinf > 0 || r.n_finite == 0;
+}
+
+// grid (tiles, branches): tile totals; the last block of a branch chains them into the offsets
+// and T, then resets its counter.  The block stages the totals in shared memory, 256 at a time,
+// so that the serial chain of thread 0 does not wait on one L2 load per tile.
+__global__ void __launch_bounds__(kPostThreads) posterior_sums_kernel(PosteriorArgs P) {
+    __shared__ double sh_warp[kPostThreads / 32];
+    __shared__ double sh_tot[kPostThreads];
+    __shared__ bool last;
+    const int b = blockIdx.y;
+    const LsePartial r = P.lse[b];
+    double l[kPostPer], wb, e;
+    const double tot = post_tile_scan(P, b, blockIdx.x, r.m, !post_empty(r), l, wb, e, sh_warp);
+    if (threadIdx.x == 0) P.tile_sum[(size_t)b * P.tiles + blockIdx.x] = tot;
+    __threadfence();
+    if (threadIdx.x == 0) last = atomicAdd(P.done + b, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;   // (uniform over the block)
+    __threadfence();
+    const double* ts = P.tile_sum + (size_t)b * P.tiles;
+    double* off = P.tile_off + (size_t)b * (P.tiles + 1);
+    double o = 0.0;   // (thread 0's)
+    for (int64_t base = 0; base < P.tiles; base += kPostThreads) {
+        const int64_t t = base + threadIdx.x;
+        sh_tot[threadIdx.x] = t < P.tiles ? __ldcg(ts + t) : 0.0;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            const int n = (int)(P.tiles - base < kPostThreads ? P.tiles - base : kPostThreads);
+            for (int q = 0; q < n; ++q) {
+                off[base + q] = o;
+                o += sh_tot[q];
+            }
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x != 0) return;
+    off[P.tiles] = o;
+    P.total[b] = r.n_posinf > 0 ? INFINITY : r.n_finite == 0 ? 0.0 : o;
+    P.done[b] = 0u;
+}
+
+// number of k in [0, K) with (U + k) * step < c (u_k is non-decreasing in k)
+__device__ __forceinline__ int64_t post_count(double c, double U, double step, int64_t K) {
+    const double g = floor(c / step - U);
+    int64_t k = g > 0.0 ? (g < (double)K ? (int64_t)g : K) : 0;
+    while (k < K && (U + (double)k) * step < c) ++k;
+    while (k > 0 && (U + (double)(k - 1)) * step >= c) --k;
+    return k;
+}
+
+// grid (tiles, branches): each draw writes the samples whose u_k falls in [C_{i-1}, C_i)
+__global__ void __launch_bounds__(kPostThreads) posterior_select_kernel(PosteriorArgs P) {
+    __shared__ double sh_warp[kPostThreads / 32];
+    const int b = blockIdx.y;
+    const double T = P.total[b];
+    if (!(T > 0.0) || !isfinite(T)) return;   // empty posterior (uniform over the block)
+    double l[kPostPer], wb, e;
+    post_tile_scan(P, b, blockIdx.x, P.lse[b].m, true, l, wb, e, sh_warp);
+    const double o = P.tile_off[(size_t)b * (P.tiles + 1) + blockIdx.x];
+    const double U = posterior_uniform(P.seed, P.stream, (unsigned long long)b);
+    const double step = T / (double)P.K;
+    int64_t* idx = b ? P.idx[1] : P.idx[0];
+    const int64_t base = (int64_t)blockIdx.x * kPostTile + (int64_t)threadIdx.x * kPostPer;
+    double lo = o + (wb + e);
+#pragma unroll
+    for (int j = 0; j < kPostPer; ++j) {
+        const double hi = o + (wb + (e + l[j]));
+        if (hi > lo) {
+            const int64_t k1 = hi == T ? P.K : post_count(hi, U, step, P.K);
+            for (int64_t k = post_count(lo, U, step, P.K); k < k1; ++k) idx[k] = base + j;
+        }
+        lo = hi;
+    }
+}
+
 // ---- standalone log-mean-exp of an array (tri_log_mean_exp, _numerics.py:12-51) ----------------
 constexpr int kLseThreads = 256;
 

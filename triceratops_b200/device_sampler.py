@@ -266,14 +266,23 @@ def _take_rows(columns, idx, dev):
 
 
 def _table(lb, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, rps=None,
-           masses=None, radii=None, fluxratios=None):
-    """This rank's half of a result dictionary: the rows of its best local draws, registered
-    for the merge across ranks (_finished)."""
+           masses=None, radii=None, fluxratios=None, post=None, branch=0):
+    """This rank's half of a result dictionary: the rows of its best local draws (and of its
+    posterior samples, post = (K, seed, stream) of the call), registered for the merge across
+    ranks (_finished)."""
+    cols = dict(M_s=M_host, R_s=R_host, u1=u1, u2=u2, P=P, mtot=mtot, inc=incs, ecc=eccs,
+                argp=argps, R_p=rps, M_EB=masses, R_EB=radii, fluxratio_EB=fluxratios,
+                fluxratio_comp=cfr if torch.is_tensor(cfr) else None)
     idx = torch.as_tensor(np.asarray(lb.idx, dtype=np.int64), device=dev)
-    got = _take_rows(dict(M_s=M_host, R_s=R_host, u1=u1, u2=u2, P=P, mtot=mtot, inc=incs, ecc=eccs,
-                          argp=argps, R_p=rps, M_EB=masses, R_EB=radii, fluxratio_EB=fluxratios,
-                          fluxratio_comp=cfr if torch.is_tensor(cfr) else None), idx, dev)
-    return _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS)
+    got = _take_rows(cols, idx, dev)
+    ptab = None
+    if post is not None and lb.res.post_idx is not None:
+        pidx = np.asarray(lb.res.post_idx, dtype=np.int64)
+        ptab = ml.result_table(len(pidx), twin,
+                               **_take_rows(cols, torch.as_tensor(pidx, device=dev), dev))
+        ptab["draw"] = pidx + _dispatch.shard_bounds(lb.N)[0]
+    return _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS,
+                                   None if ptab is None else (post, branch, ptab))
 
 
 def _finished(exchange):
@@ -282,6 +291,7 @@ def _finished(exchange):
     out = ml.ScenarioResult(merged)
     out.n_pass, out.n_evaluated = n_pass, n_eval
     out.set_moments(exchange.lb.N, exchange.record, exchange.top)
+    out.posterior, out.post_total = exchange.posterior, exchange.post_total
     return out
 
 
@@ -295,16 +305,18 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
     cfr = c.get("cfr", 0.0)
     common = dict(P_orb=P, inc=c["inc"], ecc=c["ecc"], argp=c["argp"], mtot=c["mtot"],
                   rhost=R_host, u1=u1, u2=u2, cfr=cfr, lnprior=c.get("lnprior"))
+    post = _dispatch._next_post()
     if "ebfr" not in c:
         p = _dispatch._submit(eng, "tp_tensors", n, dict(rp=c["body"], **common), c["mask"],
-                              is_host, N_SAMPLES)
+                              is_host, N_SAMPLES, post=post)
         state = []
 
         def prepare():
             if not state:
                 lb = _dispatch.gather_local(p.result(), N, eng)
                 state.append(_table(lb, dev, False, M_host, R_host, u1, u2, P, c["mtot"],
-                                    c["inc"], c["ecc"], c["argp"], cfr, rps=c["body"]))
+                                    c["inc"], c["ecc"], c["argp"], cfr, rps=c["body"],
+                                    post=post))
 
         def table():
             prepare()
@@ -313,16 +325,17 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
     kw = {"scalar_loop": True} if scalar_loop else {}
     p = _dispatch._submit(eng, "eb_tensors", n,
                           dict(reb=c["body"], ebfr=c["ebfr"], q=c["q"], **common), c["mask"],
-                          is_host, N_SAMPLES, **kw)
+                          is_host, N_SAMPLES, post=post, **kw)
     args = (M_host, R_host, u1, u2, P, c["mtot"], c["inc"], c["ecc"], c["argp"], cfr)
-    tkw = dict(masses=c["meb"], radii=c["body"], fluxratios=c["ebfr"])
+    tkw = dict(masses=c["meb"], radii=c["body"], fluxratios=c["ebfr"], post=post)
     state, done = [], {}
 
     def prepare():   # both branches at the first request, in a fixed order
         if not state:
             r0, r1 = p.result()
             state.append(_table(_dispatch.gather_local(r0, N, eng), dev, False, *args, **tkw))
-            state.append(_table(_dispatch.gather_local(r1, N, eng), dev, True, *args, **tkw))
+            state.append(_table(_dispatch.gather_local(r1, N, eng), dev, True, *args, **tkw,
+                                branch=1))
 
     def table(b):
         prepare()

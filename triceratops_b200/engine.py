@@ -67,7 +67,7 @@ class BranchResult:
     """One scenario branch: lnZ pieces + optional per-draw arrays."""
     __slots__ = ("lnZ", "m", "s", "n_finite", "n_posinf", "n_pass", "n_stamps", "n_interior",
                  "n_limb", "lnL", "mask", "N", "top_idx", "top_lnL", "n_evaluated", "branch",
-                 "s2")
+                 "s2", "post_idx", "post_total")
 
     def __init__(self, r, N, lnL, mask, top=None, branch=0):
         self.lnZ, self.m, self.s = r.lnZ, r.m, r.s
@@ -77,6 +77,10 @@ class BranchResult:
         self.lnL, self.mask, self.N = lnL, mask, N
         self.branch = branch
         self.s2 = None       # second moment of the weights (Engine.set_moments), set on wait
+        # posterior samples (Engine.set_posterior), set on wait: int64 [K] draw indices in
+        # ascending order ([0] when the posterior is empty) and T, the sum of the weights
+        # relative to exp(m); None when off
+        self.post_idx = self.post_total = None
         if top is not None:
             self.top_idx, self.top_lnL = top[0][:r.n_top], top[1][:r.n_top]
             self.n_evaluated = r.n_evaluated
@@ -103,6 +107,7 @@ class Pending:
         self._engine, self._ticket, self._rr, self._nb = engine, ticket, rr, n_branches
         self._keep, self._build, self._n_best = keep, build, n_best
         self._moments = engine._moments     # (tri_set_moments is captured per submission)
+        self._post_K = engine._post_K       # (and so is tri_set_posterior)
         self._out = None
 
     def done(self):
@@ -129,6 +134,14 @@ class Pending:
                 _cabi.check(eng.lib.tri_last_moments(s2))
                 for b, br in enumerate(out):
                     br.s2 = s2[b]
+            if self._post_K > 0:
+                for b, br in enumerate(out):
+                    idx = np.empty(self._post_K, dtype=np.int64)
+                    n, T = ctypes.c_int64(), ctypes.c_double()
+                    _cabi.check(eng.lib.tri_last_posterior(
+                        b, idx.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), idx.size,
+                        ctypes.byref(n), ctypes.byref(T)))
+                    br.post_idx, br.post_total = idx[:n.value], T.value
             # fewer finite draws than the table has rows: the caller pads the table from the
             # full lnL array, which is only reachable until the next evaluation completes
             for b, br in enumerate(out):
@@ -138,6 +151,9 @@ class Pending:
             self._keep = None
             self._out = out[0] if self._nb == 1 else tuple(out)
         return self._out
+
+
+_U64 = (1 << 64) - 1
 
 
 def combine_lse(parts, N_total):
@@ -185,6 +201,7 @@ class Engine:
         self._side_streams = None
         self._side_turn = 0
         self._moments = False
+        self._post_K, self._post_seed = 0, 0
 
     @_locked
     def _make_room(self):
@@ -305,11 +322,12 @@ class Engine:
     @_locked
     def submit_tp(self, N, rp, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr, lnprior=None,
                   extra_mask=None, companion_is_host=False, want_lnL=True, want_mask=False,
-                  n_best=0, lightcurve=None):
+                  n_best=0, lightcurve=None, post_stream=0):
         """Queue a TP-type evaluation (tri_submit_tp) and return its Pending: the column copies
         overlap the kernels of the call submitted before.  `eval_tp` is submit + result().
         `lightcurve` = (time, flux, sigma, exptime, nsamples) makes that the current light
-        curve in the same critical section (callers in several threads)."""
+        curve in the same critical section (callers in several threads).  `post_stream`: the
+        stream of the posterior samples' U (set_posterior)."""
         N = int(N)
         if lightcurve is not None:
             self.set_lightcurve(*lightcurve)
@@ -326,6 +344,7 @@ class Engine:
         r, lnL, mask, top = self._result(N, want_lnL, want_mask, n_best)
         rr = (tri_result * 1)(r)
         ticket = ctypes.c_int64()
+        self._arm_posterior(post_stream)
         _cabi.check(self.lib.tri_submit_tp(ctypes.byref(a), rr, ctypes.byref(ticket)))
         keep, self._keep = self._keep + [a, lnL, mask, top], []
 
@@ -339,7 +358,7 @@ class Engine:
     @_locked
     def submit_eb(self, N, reb, ebfr, q, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr,
                   lnprior=None, extra_mask=None, companion_is_host=False, want_lnL=True,
-                  want_mask=False, n_best=0, lightcurve=None, scalar_loop=False):
+                  want_mask=False, n_best=0, lightcurve=None, scalar_loop=False, post_stream=0):
         """EB-type counterpart of submit_tp.  scalar_loop=True evaluates with the semantics of
         the reference's parallel=False loops (see tri_eb_args.scalar_loop)."""
         N = int(N)
@@ -363,6 +382,7 @@ class Engine:
             rr[b] = r
             outs.append((lnL, mask, top))
         ticket = ctypes.c_int64()
+        self._arm_posterior(post_stream)
         _cabi.check(self.lib.tri_submit_eb(ctypes.byref(a), rr, ctypes.byref(ticket)))
         keep, self._keep = self._keep + [a, outs], []
 
@@ -421,7 +441,7 @@ class Engine:
 
     @_locked
     def _submit_tensors(self, kind, N, cols, extra_mask, companion_is_host, n_best,
-                        lightcurve=None, scalar_loop=False):
+                        lightcurve=None, scalar_loop=False, post_stream=0):
         import torch
         N = int(N)
         if lightcurve is not None:
@@ -458,6 +478,7 @@ class Engine:
         stream = side.cuda_stream
         fn = self.lib.tri_submit_tp_dev if kind == "tp" else self.lib.tri_submit_eb_dev
         ticket = ctypes.c_int64()
+        self._arm_posterior(post_stream)
         _cabi.check(fn(ctypes.byref(a), rr, ctypes.c_void_p(stream), ctypes.byref(ticket)))
         keep.append(a)
 
@@ -469,17 +490,17 @@ class Engine:
         return p
 
     def submit_tp_tensors(self, N, cols, extra_mask=None, companion_is_host=False, n_best=100,
-                          lightcurve=None):
+                          lightcurve=None, post_stream=0):
         """tri_submit_tp_dev on torch CUDA tensors (columns: rp, P_orb, inc, ecc, argp, mtot,
         rhost, u1, u2, cfr, lnprior; tensors of N values or scalars), queued on torch's current
         stream behind the kernels that produce them.  Returns a Pending."""
         return self._submit_tensors("tp", N, cols, extra_mask, companion_is_host, n_best,
-                                    lightcurve)
+                                    lightcurve, post_stream=post_stream)
 
     def submit_eb_tensors(self, N, cols, extra_mask=None, companion_is_host=False, n_best=100,
-                          lightcurve=None, scalar_loop=False):
+                          lightcurve=None, scalar_loop=False, post_stream=0):
         return self._submit_tensors("eb", N, cols, extra_mask, companion_is_host, n_best,
-                                    lightcurve, scalar_loop)
+                                    lightcurve, scalar_loop, post_stream)
 
     def eval_tp_tensors(self, *args, **kw):
         return self.submit_tp_tensors(*args, **kw).result()
@@ -574,6 +595,21 @@ class Engine:
         evaluations submitted while it is on, None otherwise."""
         _cabi.check(self.lib.tri_set_moments(int(bool(on))))
         self._moments = bool(on)
+
+    @_locked
+    def set_posterior(self, K, seed=0):
+        """K posterior samples per branch of every evaluation submitted while K > 0
+        (tri_set_posterior): BranchResult.post_idx / post_total.  The third part of the hash
+        that gives U, the stream, is passed with each submission (`post_stream`)."""
+        K, seed = int(K), int(seed) & _U64
+        _cabi.check(self.lib.tri_set_posterior(K, seed, 0))
+        self._post_K, self._post_seed = K, seed
+
+    def _arm_posterior(self, post_stream):
+        """Hand the submission's stream to tri_set_posterior (lock held, K > 0 only)."""
+        if self._post_K > 0:
+            _cabi.check(self.lib.tri_set_posterior(self._post_K, self._post_seed,
+                                                   int(post_stream) & _U64))
 
     @_locked
     def fp64_peak(self):

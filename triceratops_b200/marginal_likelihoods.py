@@ -308,6 +308,11 @@ class ScenarioResult(dict):
     # rows: what calc_probs merges when it refines a scenario with more draws
     record = None
     top = None
+    # inside `triceratops_b200.posterior_samples(K)`: the K posterior samples as a table (the
+    # keys of RESULT_KEYS plus `draw`, the global draw index; 0 rows when the posterior is
+    # empty) and their total weight relative to exp(record[0]); None otherwise
+    posterior = None
+    post_total = None
 
     def set_moments(self, N, record, top):
         """Attach the branch's evidence record; the error fields when it carries s2."""
@@ -330,6 +335,15 @@ def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, *
     out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
     out.set_moments(br.N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
                     (br.vals, np.asarray(idx)[:len(br.vals)]))
+    if br.post_idx is not None:
+        p = np.asarray(br.post_idx, dtype=np.int64)
+        rows = {k: v[p] for k, v in body.items()}
+        out.posterior = result_table(
+            len(p), twin, _take(M_host, p), _take(R_host, p), _take(u1, p), _take(u2, p),
+            _take(P, p), _take(mtot, p), incs[p], eccs[p], argps[p],
+            fluxratio_comp=_take(cfr, p) if np.ndim(cfr) else None, **rows)
+        out.posterior["draw"] = p
+        out.post_total = br.post_total
     return out
 
 

@@ -19,11 +19,12 @@ import sys
 import warnings
 
 import numpy as np
-from pandas import DataFrame
+from pandas import DataFrame, concat
 from scipy.special import ndtr
 
 from . import _bufpool, _dispatch
-from ._numerics import _normalize_probabilities, mc_error, probability_errors
+from ._numerics import (_normalize_probabilities, mc_error, merge_posteriors,
+                        probability_errors)
 from .funcs import renorm_flux
 from .marginal_likelihoods import (RESULT_KEYS, ScenarioResult, lnZ_BEB, lnZ_BTP, lnZ_DEB,
                                    lnZ_DTP, lnZ_PEB, lnZ_PTP, lnZ_SEB, lnZ_STP, lnZ_TEB, lnZ_TTP)
@@ -138,7 +139,8 @@ class target:
                    verbose: int = 1, flatpriors: bool = False,
                    exptime: float = 0.00139, nsamples: int = 20,
                    molusc_file: str = None, mc_errors: bool = False,
-                   fpp_err_target: float = None, N_max: int = None):
+                   fpp_err_target: float = None, N_max: int = None,
+                   posterior_samples: int = None, posterior_seed: int = 0):
         """Relative probability of every scenario, FPP and NFPP (triceratops.py:673-1485).
 
         Extensions of the reference's arguments: `flux_err_0` may hold one error per time stamp
@@ -160,7 +162,24 @@ class target:
         as one more disjoint slice.  Rounds stop when FPP_err <= fpp_err_target or no
         contributing call can grow.  Host sampler: the new draws continue numpy's global
         generator; device sampler: each round is a new scenario call (a fresh Philox stream).
-        Refinement needs all draws on this process (no draw sharding over a process group)."""
+        Refinement needs all draws on this process (no draw sharding over a process group).
+
+        Posterior samples (not in the reference): `posterior_samples=K` draws K samples from the
+        posterior of every scenario row by systematic importance resampling of its prior draws
+        (weights exp(lnL + lnprior), on the GPU) and sets `self.posterior`, a long-format
+        DataFrame: one block of K rows per scenario row whose posterior is not empty, with the
+        columns ID, scenario, row (of `probs`), draw (the prior draw's index) and the parameter
+        columns of `probs` plus u1, u2, fluxratio_EB and fluxratio_comp.  Without it
+        `self.posterior` is None.  The samples depend on `posterior_seed` and the row (and on
+        the round under fpp_err_target, whose rounds merge their samples); lnZ, probs, FPP,
+        NFPP, the best-draw tables and numpy's generator are the same bits with and without
+        them.  At an effective sample size of a few, the K samples hold few distinct draws."""
+        post_K = None
+        if posterior_samples is not None:
+            post_K = _dispatch.check_posterior_K(posterior_samples)
+            if isinstance(posterior_seed, bool) or not isinstance(posterior_seed,
+                                                                  (int, np.integer)):
+                raise ValueError("posterior_seed must be an integer")
         if fpp_err_target is not None:
             if not (np.isfinite(fpp_err_target) and fpp_err_target > 0):
                 raise ValueError("fpp_err_target must be positive and finite")
@@ -251,7 +270,7 @@ class target:
                     lnZ[j] = -np.inf
                 return
             calls.append((rows, fn))
-            waiting.append((rows, chain.run(functools.partial(fn, N))))
+            waiting.append((rows, chain.run(functools.partial(_in_stream, fn, rows[0], N))))
             settle(_PIPELINE_DEPTH)
 
         def say(msg):
@@ -272,8 +291,10 @@ class target:
         sys.setswitchinterval(_dispatch.gil_switch_interval())
         _bufpool.note_call()       # (page-locked column buffers from a process's second call on)
         moments = _dispatch.mc_errors() if mc_errors else contextlib.nullcontext()
+        post = (lambda: _dispatch.posterior_samples(post_K, posterior_seed)) if post_K else \
+            contextlib.nullcontext
         try:
-            with moments, _dispatch.deferring():
+            with moments, post(), _dispatch.deferring():
                 for i, ID in enumerate(filtered["ID"].values if not follower else ()):
                     star = {c: filtered[c].values[i] for c in _STAR_COLUMNS}
                     flux, flux_err = renorm_flux(flux_0, flux_err_0, star["fluxratio"])
@@ -347,26 +368,33 @@ class target:
                 if not ok:
                     _dispatch.close_group()
         err = None
+        posterior = None
         try:
             if follower:
                 with _dispatch.mc_errors() if mc_errors else contextlib.nullcontext():
-                    targets, star_num, scenarios, best, lnZ, err = group.follow(eng)
+                    targets, star_num, scenarios, best, lnZ, err, posterior = group.follow(eng)
             elif group is not None:
                 group.exchange()
                 for rows, parts in held:
                     fill(rows, parts)
                 if mc_errors:
                     err = _refine(calls, row_results, lnZ, best, None, None)
+                if post_K:
+                    posterior = _posterior_frame(targets, scenarios, row_results)
                 if group.scatter:
-                    group.publish((targets, star_num, scenarios, best, lnZ, err))
+                    group.publish((targets, star_num, scenarios, best, lnZ, err, posterior))
         finally:
             self.collectives = None if group is None else {
                 "record_exchanges": group.collectives, "scatters": group.scatters}
             _dispatch.close_group()
 
         if mc_errors and group is None:
-            with _dispatch.mc_errors():
-                err = _refine(calls, row_results, lnZ, best, fpp_err_target, N_max)
+            with _dispatch.mc_errors(), post():
+                err = _refine(calls, row_results, lnZ, best, fpp_err_target, N_max,
+                              (post_K, posterior_seed) if post_K else None)
+        if post_K and group is None:
+            posterior = _posterior_frame(targets, scenarios, row_results)
+        self.posterior = posterior
         relative_probs, status = _normalize_probabilities(lnZ)
         if status == 'anomaly':
             warnings.warn(
@@ -407,6 +435,36 @@ class target:
         return
 
 
+_POSTERIOR_COLUMNS = (("M_s", "M_s"), ("R_s", "R_s"), ("P_orb", "P_orb"), ("inc", "inc"),
+                      ("b", "b"), ("ecc", "ecc"), ("w", "argp"), ("R_p", "R_p"),
+                      ("M_EB", "M_EB"), ("R_EB", "R_EB"), ("u1", "u1"), ("u2", "u2"),
+                      ("fluxratio_EB", "fluxratio_EB"), ("fluxratio_comp", "fluxratio_comp"))
+
+
+def _posterior_frame(targets, scenarios, row_results):
+    """calc_probs' `posterior`: the rows' posterior tables stacked in row order."""
+    blocks = []
+    for j, res in enumerate(row_results):
+        tab = None if res is None else res.posterior
+        if tab is None or not len(tab["draw"]):
+            continue
+        n = len(tab["draw"])
+        cols = {"ID": np.full(n, targets[j]), "scenario": np.full(n, scenarios[j]),
+                "row": np.full(n, j), "draw": np.asarray(tab["draw"], dtype=np.int64)}
+        cols.update({name: np.asarray(tab[key]) for name, key in _POSTERIOR_COLUMNS})
+        blocks.append(DataFrame(cols))
+    if not blocks:
+        return DataFrame(columns=["ID", "scenario", "row", "draw"]
+                         + [name for name, _ in _POSTERIOR_COLUMNS])
+    return concat(blocks, ignore_index=True)
+
+
+def _in_stream(make, stream, n):
+    """One scenario call of n draws whose posterior samples use `stream`."""
+    with _dispatch.call_stream(stream):
+        return make(n)
+
+
 def _bind(fn, *args, **kw):
     """One scenario call as a function of its number of draws: fn(*args, N=n, **kw)."""
     def make(n):
@@ -434,7 +492,7 @@ def _row_errors(calls, lnZ):
                 NFPP_err=nfpp_err), contrib
 
 
-def _merge_round(old, new, offset):
+def _merge_round(old, new, offset, post=None):
     """One branch's result over the draws of `old` followed by `new` (drawn after them: its
     indices start at `offset`), merged like the records of two ranks (_dispatch._merge_records):
     lnZ over all draws, the best-draw table the top 100 of both, each row from the round that
@@ -458,16 +516,28 @@ def _merge_round(old, new, offset):
     out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
     out.set_moments(N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
                     (br.vals, br.idx[:k]))
+    if post is not None and old.posterior is not None and new.posterior is not None:
+        # post = (K, seed, stream of the new round, branch): merged like two slices of draws
+        tabs = (old.posterior, {**new.posterior, "draw": new.posterior["draw"] + offset})
+        idx, _, W = merge_posteriors(
+            [(r.record[0], r.post_total, t["draw"]) for r, t in zip((old, new), tabs)], *post)
+        draws = np.concatenate([t["draw"] for t in tabs])
+        pos = np.searchsorted(draws, idx)
+        out.posterior = {key: np.concatenate([np.asarray(t[key]) for t in tabs])[pos]
+                         for key in tabs[0] if key != "draw"}
+        out.posterior["draw"] = idx
+        out.post_total = W
     return out
 
 
-def _refine(calls, row_results, lnZ, best, target, N_max):
+def _refine(calls, row_results, lnZ, best, target, N_max, post=None):
     """Error bars of calc_probs; with `target`, refinement rounds until FPP_err <= target or no
     call that contributes to Var(FPP) can grow (N_max draws per call).  Updates lnZ and best in
     place for the refined rows; returns the error fields."""
     state = [dict(rows=rows, make=make, N=int(row_results[rows[0]].N),
                   cur=[row_results[j] for j in rows]) for rows, make in calls]
     err, contrib = _row_errors(state, lnZ)
+    rnd = 0
     while target is not None and np.isfinite(err["FPP_err"]) and err["FPP_err"] > target:
         total, acc, picked = contrib.sum(), 0.0, []
         for ci in np.argsort(-contrib, kind="stable"):
@@ -478,12 +548,16 @@ def _refine(calls, row_results, lnZ, best, target, N_max):
                 acc += contrib[ci]
         if not picked:
             break
+        rnd += 1
         for ci in picked:
             c = state[ci]
             n_new = min(c["N"], N_max - c["N"])
-            out = c["make"](n_new)
+            stream = c["rows"][0] + (rnd << 32)     # (round 0 used the row itself)
+            out = _in_stream(c["make"], stream, n_new)
             parts = out if isinstance(out, tuple) else (out,)
-            c["cur"] = [_merge_round(old, new, c["N"]) for old, new in zip(c["cur"], parts)]
+            c["cur"] = [_merge_round(old, new, c["N"],
+                                     None if post is None else (*post, stream, b))
+                        for b, (old, new) in enumerate(zip(c["cur"], parts))]
             c["N"] += n_new
             for j, res in zip(c["rows"], c["cur"]):
                 lnZ[j] = res["lnZ"]
