@@ -281,7 +281,25 @@ typedef struct {
            *o_cfr, *o_lnprior, *o_mhost, *o_meb;
     uint8_t* o_mask;
     int32_t* err_flag;     /* set to 1 if a limb-darkening node lies beyond the grid */
+    /* importance proposal (appended: the offsets above are unchanged).  Each tuned prior
+     * dimension ("slot": 0 P when P_lo < P_hi, 1 the diluter's uniform -- q_comp or the TRILEGAL
+     * index, not MOLUSC rows --, 2 R_p (TP) or q (EB), 3 inc, 4 ecc (EB only), 5 argp) is drawn
+     * as its prior transform of v instead of the uniform u.  A coin c from a counter block of its
+     * own picks the branch of the defensive mixture q(v) = alpha + (1 - alpha) prod_d h_d(v_d):
+     * c < alpha, v = u (a prior draw); otherwise v = H_d^-1(u), H_d the piecewise-linear CDF of
+     * h_d.  The kernel adds -ln q(v) = -log1p((1 - alpha) expm1(s)), s = sum_d ln h_d(v_d), to
+     * o_lnprior (after the prior's clipping; a scenario without a companion prior then writes
+     * one).  Identity tables (C_b = b / B, ln h = 0) give the columns of prop = NULL bit for bit
+     * and a delta of exactly 0. */
+    const double* prop;    /* NULL: the prior.  Else per slot, 2 B + 1 doubles: the knots
+                            * C[0..B] of H (C[0] = 0, C[B] = 1), then ln h[0..B-1] */
+    int32_t prop_bins;     /* B, a power of two */
+    double prop_alpha;     /* alpha in (0, 1] */
+    double* o_coords;      /* optional [TRI_PROP_SLOTS][n]: the v each slot used (the raw
+                            * uniform without a proposal), NaN for slots the scenario does not
+                            * draw */
 } tri_sampler_args;
+#define TRI_PROP_SLOTS 6
 
 /* Queue the sampler kernel on `stream` (NULL = the CUDA default stream); does not wait. */
 int tri_dev_sample(const tri_sampler_args* args, void* stream);

@@ -81,6 +81,25 @@ def posterior_samples(K, seed=0):
     return _dispatch.posterior_samples(K, seed)
 
 
+def importance_proposal(p):
+    """Context manager: device-sampler lnZ_* calls made inside it draw their tuned prior
+    dimensions from `p`, a device_sampler.Proposal (the defensive mixture of the prior and a
+    fitted product of binned marginals, _numerics.fit_proposal), and weight each draw by
+    L prior / q: lnZ stays an unbiased evidence.  Outside it nothing changes.  A host-sampler
+    lnZ_* call inside it raises ValueError.  calc_probs(proposal="adaptive") uses it."""
+    from . import device_sampler
+    return device_sampler.importance_proposal(p)
+
+
+def record_coords():
+    """Context manager: device-sampler lnZ_* calls made inside it that also draw posterior
+    samples (posterior_samples) set each result's `post_coords`, the samples' coordinates in
+    the sampler's unit cube ([K, 6], one column per slot of tri_sampler_args.prop, NaN where
+    the scenario does not draw that slot): what a proposal is fitted to."""
+    from . import device_sampler
+    return device_sampler.record_coords()
+
+
 def set_sampler(mode="host", seed=None):
     """Where the prior draws are made.
 

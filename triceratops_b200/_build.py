@@ -8,7 +8,7 @@ CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libtriceratops_b200.so")
 HOST_SO_PATH = os.path.join(CSRC, "libtriceratops_host.so")   # prior-draw helpers (host_*.c)
 SOURCES = ["tri_cabi.cu"]
-HEADERS = ["tri_kernels.cuh", "tri_model.cuh", os.path.join("..", "..", "include", "triceratops_b200.h")]
+HEADERS = ["tri_kernels.cuh", "tri_model.cuh", "tri_sampler.cuh", os.path.join("..", "..", "include", "triceratops_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -17,6 +17,7 @@ TRI_OK, TRI_ECUDA, TRI_EINVAL, TRI_ESTATE, TRI_ENODEVICE = 0, -1, -2, -3, -4
 TRI_MAX_INFLIGHT = 4     # include/triceratops_b200.h
 TRI_MAX_CADENCES = 8     # include/triceratops_b200.h
 TRI_MAX_POSTERIOR = 1 << 20   # include/triceratops_b200.h
+TRI_PROP_SLOTS = 6       # include/triceratops_b200.h
 
 
 class TriError(RuntimeError):
@@ -96,7 +97,9 @@ class tri_sampler_args(ctypes.Structure):
         + [("o_" + n, ctypes.c_void_p) for n in ("body", "ebfr", "q", "P", "inc", "ecc", "argp",
                                                  "mtot", "rhost", "u1", "u2", "cfr", "lnprior",
                                                  "mhost", "meb")]
-        + [("o_mask", ctypes.c_void_p), ("err_flag", ctypes.c_void_p)])
+        + [("o_mask", ctypes.c_void_p), ("err_flag", ctypes.c_void_p),
+           ("prop", ctypes.c_void_p), ("prop_bins", ctypes.c_int32),
+           ("prop_alpha", ctypes.c_double), ("o_coords", ctypes.c_void_p)])
 
 
 # every symbol include/triceratops_b200.h declares

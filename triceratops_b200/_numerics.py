@@ -207,3 +207,128 @@ def merge_posteriors(parts, K, seed, stream, branch=0):
         pos = np.floor((np.arange(cr) + U) * (len(idx) / cr)).astype(np.int64)
         out.append(idx[np.minimum(pos, len(idx) - 1)])
     return np.concatenate(out), m, W
+
+
+# ---- adaptive importance sampling: proposal tables ----------------------------------------------
+# The device sampler draws each tuned prior dimension ("slot", tri_sampler_args.prop) as its
+# inverse prior CDF of a coordinate v in [0, 1).  A proposal replaces the uniform v of each slot
+# d by a piecewise-constant density h_d on B equal bins inside the defensive mixture
+# q(v) = alpha + (1 - alpha) prod_d h_d(v_d); the importance weight of a draw is then L pi / q(v),
+# and q >= alpha bounds it by L pi / alpha.  Tables per slot: the B + 1 knots C of h's
+# piecewise-linear CDF (C_0 = 0, C_B = 1), then B values of ln h.
+PROP_SLOTS = 6
+PROP_BINS = 1024          # B
+PROP_ALPHA = 0.1          # weight of the prior in the mixture
+_BELOW_ONE = np.nextafter(1.0, 0.0)
+_KDE_FLOOR = 1e-6         # share of a flat density in each fitted h: every bin stays positive
+
+
+def identity_tables(B=PROP_BINS):
+    """Tables of the prior for every slot: C_b = b / B, ln h = 0 (exact for a power-of-two B)."""
+    one = np.concatenate([np.arange(B + 1, dtype=np.float64) / B, np.zeros(B)])
+    return np.tile(one, (PROP_SLOTS, 1))
+
+
+def _slot_table(h):
+    """(2 B + 1) table of a density h over B bins (h > 0, mean 1)."""
+    B = h.size
+    C = np.concatenate([[0.0], np.cumsum(h / B)])
+    C[-1] = 1.0
+    return np.concatenate([C, np.log(h)])
+
+
+def _kde_bins(x, w, B):
+    """Gaussian KDE of points x in [0, 1] with weights w (sum 1), reflected at 0 and 1, as a
+    density on B equal bins (mean 1).  Bandwidth: Scott's rule over the distinct points,
+    sigma n^(-1/5), at least 8 bins.  The points are placed at the centres of 4 B sub-bins (at
+    most 1/64 of the bandwidth away) so that the bin masses are one convolution."""
+    from scipy.signal import fftconvolve
+    from scipy.special import ndtr
+    n = x.size
+    mu = float(np.sum(w * x))
+    sd = float(np.sqrt(max(np.sum(w * (x - mu) ** 2), 0.0)))
+    bw = max(sd * n ** -0.2, 8.0 / B)
+    R = 4 * B
+    hist = np.bincount(np.minimum((x * R).astype(np.int64), R - 1), weights=w, minlength=R)
+    ext = np.concatenate([hist[::-1], hist, hist[::-1]])    # mirror images at 0 and 1
+    # CDF at edge b / B: sum_k ext[k] Phi((4 b + R - k - 1/2) / (R bw)), a full convolution
+    g = ndtr((np.arange(-2 * R, 2 * R + 1) - 0.5) / (R * bw))
+    F = fftconvolve(ext, g)[3 * R + 4 * np.arange(B + 1)]
+    mass = np.maximum(np.diff(F), 0.0)
+    h = mass * (B / mass.sum())
+    h = (1.0 - _KDE_FLOOR) * h + _KDE_FLOOR
+    return h * (B / h.sum())
+
+
+def fit_proposal(coords, slots, B=PROP_BINS, alpha=PROP_ALPHA):
+    """Proposal tables ([PROP_SLOTS, 2 B + 1]) fitted to K resampled posterior rows `coords`
+    ([K, PROP_SLOTS], the v of each slot; rows of a systematic resample repeat draws).  The
+    distinct rows are weighted by their multiplicity; each slot in `slots` gets the binned
+    reflected-KDE density of its coordinates, every other slot the identity table.  An empty
+    posterior (no rows, or rows that are not finite in a fitted slot) gives identity tables.
+    `alpha` enters only the kernel's mixture (kept here for the signature of the schedule)."""
+    del alpha
+    tab = identity_tables(B)
+    coords = np.asarray(coords, dtype=np.float64).reshape(-1, PROP_SLOTS)
+    slots = [int(d) for d in slots]
+    if not coords.shape[0] or not slots or not np.all(np.isfinite(coords[:, slots])):
+        return tab
+    rows, counts = np.unique(coords[:, slots], axis=0, return_counts=True)
+    w = counts / counts.sum()
+    for j, d in enumerate(slots):
+        tab[d] = _slot_table(_kde_bins(np.clip(rows[:, j], 0.0, 1.0), w, B))
+    return tab
+
+
+def proposal_inverse(tab, u, mix):
+    """Numpy mirror of the kernel's map of one slot: (v, b) for uniforms u; `mix` True off the
+    prior branch of the mixture (v = H^-1(u)), False on it (v = u)."""
+    tab = np.asarray(tab, dtype=np.float64)
+    B = (tab.size - 1) // 2
+    C, lnh = tab[:B + 1], tab[B + 1:]
+    u = np.asarray(u, dtype=np.float64)
+    mix = np.broadcast_to(np.asarray(mix, dtype=bool), u.shape)
+    b_mix = np.clip(np.searchsorted(C, u, side="right") - 1, 0, B - 1)
+    v_mix = np.minimum((b_mix + (u - C[b_mix]) / (np.exp(lnh[b_mix]) / B)) / B, _BELOW_ONE)
+    b_pri = np.minimum((u * B).astype(np.int64), B - 1)
+    return np.where(mix, v_mix, u), np.where(mix, b_mix, b_pri)
+
+
+def proposal_lnq(tabs, v, slots, alpha=PROP_ALPHA, bins=None):
+    """ln q(v) of the mixture for coordinates v ([n, PROP_SLOTS]) over the tuned `slots`: s = sum
+    of ln h_d at the bin of v_d (floor(v_d B), or the given `bins` [n, PROP_SLOTS]), ln q =
+    log1p((1 - alpha) expm1(s)); what the kernel subtracts from lnprior."""
+    tabs = np.asarray(tabs, dtype=np.float64)
+    B = (tabs.shape[1] - 1) // 2
+    v = np.atleast_2d(np.asarray(v, dtype=np.float64))
+    s = np.zeros(v.shape[0])
+    for d in slots:
+        b = (np.minimum((v[:, d] * B).astype(np.int64), B - 1) if bins is None
+             else np.asarray(bins)[:, d])
+        s = s + tabs[d, B + 1 + b]
+    return np.log1p((1.0 - alpha) * np.expm1(s))
+
+
+def pooled_posterior(branches, K, seed, stream):
+    """The K posterior rows of one scenario call for fitting its proposal: for an EB-type call,
+    the mixture of its two branches' posteriors (disjoint masks over the same draws), with the
+    K rows allocated between them by evidence (merge_posteriors, the branches as two slices).
+    branches: (m, T, coords [K_b, PROP_SLOTS]) per branch.  Returns [k, PROP_SLOTS] rows (k = 0
+    when the posterior is empty or a weight is +inf)."""
+    if len(branches) == 1:
+        m, T, c = branches[0]
+        if not (np.isfinite(T) and T > 0) or c is None:
+            return np.zeros((0, PROP_SLOTS))
+        return np.asarray(c, dtype=np.float64).reshape(-1, PROP_SLOTS)
+    if any(c is None for _, _, c in branches):
+        return np.zeros((0, PROP_SLOTS))
+    parts, rows, off = [], [], 0
+    for m, T, c in branches:
+        c = np.asarray(c, dtype=np.float64).reshape(-1, PROP_SLOTS)
+        parts.append((m, T, off + np.arange(len(c), dtype=np.int64)))
+        rows.append(c)
+        off += len(c)
+    idx, _, W = merge_posteriors(parts, K, seed, stream)
+    if idx is None or not len(idx) or not np.isfinite(W):
+        return np.zeros((0, PROP_SLOTS))
+    return np.concatenate(rows)[idx]

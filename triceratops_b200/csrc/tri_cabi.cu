@@ -1539,6 +1539,10 @@ int tri_dev_sample(const tri_sampler_args* a, void* stream) {
         (a->host == 1 && (!a->ldc_u1 || !a->ldc_u2 || !a->err_flag)) ||
         (a->prior_mode != 0 && (!a->cc_sep || !a->cc_con || a->cc_n < 1)))
         return fail(TRI_EINVAL, "a table the scenario needs is NULL");
+    if (a->prop && (a->prop_bins < 1 || (a->prop_bins & (a->prop_bins - 1)) != 0 ||
+                    !(a->prop_alpha > 0.0 && a->prop_alpha <= 1.0) || !a->o_lnprior))
+        return fail(TRI_EINVAL, "a proposal needs a power-of-two bin count, alpha in (0, 1] "
+                                "and the lnprior column");
     CU(cudaSetDevice(g.device));
     cudaStream_t s = (cudaStream_t)stream;
     int blocks = (int)std::min<int64_t>((a->n + 255) / 256, (int64_t)g.sm_count * 8);

@@ -198,12 +198,75 @@ __device__ __forceinline__ double clip_prior(double lnprior, double delta_mag) {
     return delta_mag > 0.0 ? -INFINITY : lnprior;
 }
 
+// ---- importance proposal (tri_sampler_args.prop) --------------------------------------------------
+// One tuned dimension (slot) maps the uniform u its inverse CDF would receive to the coordinate v
+// it receives instead.  Off the prior branch of the defensive mixture, v = H^-1(u) with H the
+// piecewise-linear CDF of the slot's binned density h (knots C[0..B], ln h[0..B-1]); on it, v = u.
+// Either way s gains ln h of v's bin -- the bin the search found, not one recomputed from v,
+// which rounding can put on a bin edge.  Identity tables (C_b = b / B, h = 1, B a power of two)
+// give v = u exactly on both branches and s = 0.
+struct Proposal {
+    const double* tab;   // NULL: the prior, nothing is changed
+    int B;
+    bool mix;            // off the prior branch
+    double s;            // sum over the tuned slots of ln h(v)
+    double* coords;      // optional: v of each slot, column-major [TRI_PROP_SLOTS][n]
+    int64_t n, i;
+};
+
+__device__ __forceinline__ double propose(Proposal& Q, int slot, double u) {
+    if (Q.tab == nullptr) {
+        if (Q.coords) Q.coords[slot * Q.n + Q.i] = u;
+        return u;
+    }
+    const int B = Q.B;
+    const double* __restrict__ C = Q.tab + (size_t)slot * (2 * B + 1);
+    const double* __restrict__ lnh = C + B + 1;
+    double v;
+    int b;
+    if (Q.mix) {
+        int lo = 0, hi = B - 1;          // largest b with C[b] <= u
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (__ldg(C + mid) <= u) lo = mid; else hi = mid - 1;
+        }
+        b = lo;
+        const double l = __ldg(lnh + b);
+        v = ((double)b + (u - __ldg(C + b)) / (exp(l) / (double)B)) / (double)B;
+        v = fmin(v, 0x1.fffffffffffffp-1);
+        Q.s += l;
+    } else {
+        v = u;
+        b = min((int)(v * (double)B), B - 1);
+        Q.s += __ldg(lnh + b);
+    }
+    if (Q.coords) Q.coords[slot * Q.n + Q.i] = v;
+    return v;
+}
+
 // ---- the kernel ----------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) sampler_kernel(tri_sampler_args A) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n;
          i += (int64_t)gridDim.x * blockDim.x) {
         Philox rng(A.seed, A.stream, (uint64_t)(A.index0 + i));
-        const double P = A.P_lo == A.P_hi ? A.P_lo : A.P_lo + (A.P_hi - A.P_lo) * rng.uniform();
+        Proposal Q;
+        Q.tab = A.prop;
+        Q.B = A.prop_bins;
+        Q.s = 0.0;
+        Q.mix = false;
+        Q.coords = A.o_coords;
+        Q.n = A.n;
+        Q.i = i;
+        if (A.prop) {
+            // the mixture's coin comes from a counter block of its own: the draw's main stream
+            // is consumed exactly as without a proposal
+            Philox coin(A.seed, A.stream, (uint64_t)(A.index0 + i));
+            coin.ctr[3] = 0x80000000u;
+            Q.mix = !(coin.uniform() < A.prop_alpha);
+        }
+        const double P = A.P_lo == A.P_hi
+                             ? A.P_lo
+                             : A.P_lo + (A.P_hi - A.P_lo) * propose(Q, 0, rng.uniform());
 
         // ---- the star that hosts the event, and the star that dilutes it
         double M_host = A.M_s, R_host = A.R_s, T_host = A.Teff, u1 = A.u1, u2 = A.u2;
@@ -211,7 +274,8 @@ __global__ void __launch_bounds__(256) sampler_kernel(tri_sampler_args A) {
         bool ok = true;
         int64_t idx = 0;
         if (A.diluter == 1) {            // unresolved bound companion (P*, S*)
-            const double q_comp = A.molusc_q ? A.molusc_q[i] : pl_inverse(A.qc_pl, rng.uniform());
+            const double q_comp = A.molusc_q ? A.molusc_q[i]
+                                              : pl_inverse(A.qc_pl, propose(Q, 1, rng.uniform()));
             ok = q_comp != 0.0;          // MOLUSC padding (marginal_likelihoods.py:464, :534)
             m_comp = q_comp * A.M_s;
             cfr = ok ? flux_ratio(A, m_comp, false) : 0.0;
@@ -231,7 +295,7 @@ __global__ void __launch_bounds__(256) sampler_kernel(tri_sampler_args A) {
                 }
             }
         } else if (A.diluter == 2) {     // chance-aligned background star (D*, B*)
-            idx = (int64_t)(rng.uniform() * (double)A.idx_hi);
+            idx = (int64_t)(propose(Q, 1, rng.uniform()) * (double)A.idx_hi);
             if (idx >= A.idx_hi) idx = A.idx_hi - 1;
             cfr = __ldg(A.bg_fr_tess + idx);
             if (A.host == 2) {           // the background star hosts the event (B*)
@@ -247,19 +311,19 @@ __global__ void __launch_bounds__(256) sampler_kernel(tri_sampler_args A) {
         // ---- the transiting / eclipsing body
         double body, ebfr = 0.0, q = 0.0, mtot, inc, ecc, argp, m_eb = 0.0;
         if (A.kind == 0) {
-            const double x = rng.uniform();
+            const double x = propose(Q, 2, rng.uniform());
             body = A.flatpriors ? x / (1.0 / 19.5) + 0.5
                                 : pl_inverse(M_host > 0.45 ? A.rp_hi : A.rp_lo, x);
-            inc = acos(1.0 - rng.uniform()) * (180.0 / kPi);
+            inc = acos(1.0 - propose(Q, 3, rng.uniform())) * (180.0 / kPi);
             const double ga = rng.gamma(0.867), gb = rng.gamma(3.030);
             ecc = ga / (ga + gb);
-            argp = rng.uniform() * 360.0;
+            argp = propose(Q, 5, rng.uniform()) * 360.0;
             mtot = M_host;
         } else {
-            inc = acos(1.0 - rng.uniform()) * (180.0 / kPi);
-            q = pl_inverse(A.q_pl, rng.uniform());
-            ecc = pow(rng.uniform(), 1.0 / A.ecc_expo);
-            argp = rng.uniform() * 360.0;
+            inc = acos(1.0 - propose(Q, 3, rng.uniform())) * (180.0 / kPi);
+            q = pl_inverse(A.q_pl, propose(Q, 2, rng.uniform()));
+            ecc = pow(propose(Q, 4, rng.uniform()), 1.0 / A.ecc_expo);
+            argp = propose(Q, 5, rng.uniform()) * 360.0;
             m_eb = q * M_host;
             double T_eb;
             star_of_mass(A, m_eb, R_host, T_host, body, T_eb);
@@ -304,6 +368,9 @@ __global__ void __launch_bounds__(256) sampler_kernel(tri_sampler_args A) {
                 : A.bg_const_prior;
             lnprior = clip_prior(lp, dmag);
         }
+        // importance weight of the proposal: lnprior - ln q(v), q = alpha + (1 - alpha) e^s
+        // (exactly 0 for s = 0), after the clipping, which is part of the prior
+        if (A.prop) lnprior -= log1p((1.0 - A.prop_alpha) * expm1(Q.s));
 
         A.o_body[i] = body;
         A.o_P[i] = P;

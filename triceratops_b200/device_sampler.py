@@ -22,6 +22,7 @@ on (seed, scenario call number, GLOBAL draw index) only: under a process group e
 its own N/G draws and the union is the same sample whatever the number of ranks; an unseeded run
 agrees on one seed first (rank 0's entropy).
 """
+import contextlib
 import ctypes
 import math
 import os
@@ -29,7 +30,7 @@ import os
 import numpy as np
 import torch
 
-from . import _cabi, _dispatch, funcs, priors
+from . import _cabi, _dispatch, _numerics, funcs, priors
 from . import marginal_likelihoods as ml
 from ._cabi import tri_bound_prior, tri_powerlaw, tri_sampler_args, tri_spline
 from ._ldc import grid_for
@@ -44,6 +45,62 @@ _cache = {}
 def seed(value):
     _state["seed"] = value
     _state["calls"] = 0
+
+
+# ------------------------------------------------------------------------------- proposals
+class Proposal:
+    """An importance proposal of one scenario call: per slot of tri_sampler_args.prop the
+    knots of H_d and ln h_d (`tables`, [TRI_PROP_SLOTS, 2 B + 1]; _numerics.fit_proposal), the
+    mixture weight `alpha` of the prior, and the tables' copy on each device they were used on."""
+
+    def __init__(self, tables, alpha=_numerics.PROP_ALPHA):
+        tables = np.ascontiguousarray(tables, dtype=np.float64)
+        B = (tables.shape[1] - 1) // 2
+        if (tables.shape != (_cabi.TRI_PROP_SLOTS, 2 * B + 1) or B < 1 or B & (B - 1)
+                or not np.all(np.isfinite(tables))):
+            raise ValueError("proposal tables must be finite, [%d, 2 B + 1] with B a power of two"
+                             % _cabi.TRI_PROP_SLOTS)
+        if not 0.0 < float(alpha) <= 1.0:
+            raise ValueError("alpha must be in (0, 1]")
+        self.tables, self.bins, self.alpha = tables, B, float(alpha)
+        self._dev = {}
+
+    @classmethod
+    def identity(cls, B=_numerics.PROP_BINS, alpha=_numerics.PROP_ALPHA):
+        """The prior as a proposal: the columns of a call without one, bit for bit."""
+        return cls(_numerics.identity_tables(B), alpha)
+
+    def device_tables(self, dev):
+        key = str(dev)
+        if key not in self._dev:      # (a stream-ordered copy on the current stream)
+            self._dev[key] = _t(self.tables, dev)
+        return self._dev[key]
+
+
+_prop = {"proposal": None, "record": 0}
+
+
+@contextlib.contextmanager
+def importance_proposal(p):
+    """Device-sampler lnZ_* calls made inside draw from Proposal `p` (None: the prior)."""
+    if p is not None and not isinstance(p, Proposal):
+        raise ValueError("importance_proposal takes a device_sampler.Proposal or None")
+    prev, _prop["proposal"] = _prop["proposal"], p
+    try:
+        yield
+    finally:
+        _prop["proposal"] = prev
+
+
+@contextlib.contextmanager
+def record_coords():
+    """Device-sampler lnZ_* calls made inside that also draw posterior samples set
+    ScenarioResult.post_coords, the samples' proposal coordinates ([K, TRI_PROP_SLOTS])."""
+    _prop["record"] += 1
+    try:
+        yield
+    finally:
+        _prop["record"] -= 1
 
 
 def _device():
@@ -229,11 +286,21 @@ def _sample(time, flux, sigma, exptime, nsamples, N, kind, host, diluter, P_orb,
         want |= {"rhost", "u1", "u2", "mhost"}
     if diluter != 0:
         want |= {"cfr"}
-    if A.prior_mode:
+    prop = _prop["proposal"]
+    if A.prior_mode or prop is not None:
         want |= {"lnprior"}
     cols = {k: torch.empty(max(n, 1), dtype=F64, device=dev)[:n] for k in _OUT if k in want}
     for k, v in cols.items():
         setattr(A, "o_" + k, v.data_ptr())
+    if prop is not None:
+        tab = prop.device_tables(dev)
+        keep.append(tab)
+        A.prop, A.prop_bins, A.prop_alpha = tab.data_ptr(), prop.bins, prop.alpha
+    coords = None
+    if _prop["record"] and _dispatch._post is not None:
+        # the coordinates of the posterior samples (slots the scenario does not draw stay NaN)
+        coords = torch.full((_cabi.TRI_PROP_SLOTS, max(n, 1)), math.nan, dtype=F64, device=dev)
+        A.o_coords = coords.data_ptr()
     mask = None
     if (diluter == 1) or host == 2:
         mask = torch.empty(max(n, 1), dtype=torch.uint8, device=dev)[:n]
@@ -246,6 +313,7 @@ def _sample(time, flux, sigma, exptime, nsamples, N, kind, host, diluter, P_orb,
             raise ValueError("can only convert an array of size 1 to a Python scalar")
     cols["mask"] = mask
     cols["_keep"] = keep
+    cols["_coords"] = coords
     return eng, dev, n, cols, A.P_lo if A.P_lo == A.P_hi else cols["P"]
 
 
@@ -266,7 +334,7 @@ def _take_rows(columns, idx, dev):
 
 
 def _table(lb, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, rps=None,
-           masses=None, radii=None, fluxratios=None, post=None, branch=0):
+           masses=None, radii=None, fluxratios=None, post=None, branch=0, coords=None):
     """This rank's half of a result dictionary: the rows of its best local draws (and of its
     posterior samples, post = (K, seed, stream) of the call), registered for the merge across
     ranks (_finished)."""
@@ -275,14 +343,20 @@ def _table(lb, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cf
                 fluxratio_comp=cfr if torch.is_tensor(cfr) else None)
     idx = torch.as_tensor(np.asarray(lb.idx, dtype=np.int64), device=dev)
     got = _take_rows(cols, idx, dev)
-    ptab = None
+    ptab = pcoords = None
     if post is not None and lb.res.post_idx is not None:
         pidx = np.asarray(lb.res.post_idx, dtype=np.int64)
-        ptab = ml.result_table(len(pidx), twin,
-                               **_take_rows(cols, torch.as_tensor(pidx, device=dev), dev))
+        tidx = torch.as_tensor(pidx, device=dev)
+        ptab = ml.result_table(len(pidx), twin, **_take_rows(cols, tidx, dev))
         ptab["draw"] = pidx + _dispatch.shard_bounds(lb.N)[0]
-    return _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS,
-                                   None if ptab is None else (post, branch, ptab))
+        if coords is not None and _dispatch._dist() is None:
+            # gathered on the device by posterior index, one copy (as _take_rows)
+            pcoords = coords[:, tidx].T.contiguous().cpu().numpy() if len(pidx) else \
+                np.zeros((0, _cabi.TRI_PROP_SLOTS))
+    ex = _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS,
+                                 None if ptab is None else (post, branch, ptab))
+    ex.post_coords = pcoords
+    return ex
 
 
 def _finished(exchange):
@@ -292,6 +366,7 @@ def _finished(exchange):
     out.n_pass, out.n_evaluated = n_pass, n_eval
     out.set_moments(exchange.lb.N, exchange.record, exchange.top)
     out.posterior, out.post_total = exchange.posterior, exchange.post_total
+    out.post_coords = exchange.post_coords
     return out
 
 
@@ -316,7 +391,7 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
                 lb = _dispatch.gather_local(p.result(), N, eng)
                 state.append(_table(lb, dev, False, M_host, R_host, u1, u2, P, c["mtot"],
                                     c["inc"], c["ecc"], c["argp"], cfr, rps=c["body"],
-                                    post=post))
+                                    post=post, coords=c["_coords"]))
 
         def table():
             prepare()
@@ -327,7 +402,8 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
                           dict(reb=c["body"], ebfr=c["ebfr"], q=c["q"], **common), c["mask"],
                           is_host, N_SAMPLES, post=post, **kw)
     args = (M_host, R_host, u1, u2, P, c["mtot"], c["inc"], c["ecc"], c["argp"], cfr)
-    tkw = dict(masses=c["meb"], radii=c["body"], fluxratios=c["ebfr"], post=post)
+    tkw = dict(masses=c["meb"], radii=c["body"], fluxratios=c["ebfr"], post=post,
+               coords=c["_coords"])
     state, done = [], {}
 
     def prepare():   # both branches at the first request, in a fixed order

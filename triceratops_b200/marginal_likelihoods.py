@@ -22,6 +22,7 @@ branches (marginal_likelihoods.py:316-319) -- and is reproduced by the engine's 
 TP-type scenarios give the same numbers either way.
 """
 import functools
+import sys
 
 import numpy as np
 from pandas import read_csv
@@ -52,6 +53,10 @@ def _device_sampler_twin(fn):
         if _sampler_mode() == "device":
             from . import device_sampler
             return getattr(device_sampler, fn.__name__)(*args, **kwargs)
+        ds = sys.modules.get(__package__ + ".device_sampler")
+        if ds is not None and ds._prop["proposal"] is not None:
+            raise ValueError("importance proposals draw on the device sampler only "
+                             "(set_sampler('device'))")
         return fn(*args, **kwargs)
     return call
 
@@ -313,6 +318,10 @@ class ScenarioResult(dict):
     # empty) and their total weight relative to exp(record[0]); None otherwise
     posterior = None
     post_total = None
+    # inside `triceratops_b200.record_coords()` (device sampler, with posterior samples): the
+    # samples' coordinates in the sampler's unit cube, [K, 6] (NaN in slots the scenario does
+    # not draw); None otherwise
+    post_coords = None
 
     def set_moments(self, N, record, top):
         """Attach the branch's evidence record; the error fields when it carries s2."""

@@ -140,7 +140,8 @@ class target:
                    exptime: float = 0.00139, nsamples: int = 20,
                    molusc_file: str = None, mc_errors: bool = False,
                    fpp_err_target: float = None, N_max: int = None,
-                   posterior_samples: int = None, posterior_seed: int = 0):
+                   posterior_samples: int = None, posterior_seed: int = 0,
+                   proposal: str = "prior"):
         """Relative probability of every scenario, FPP and NFPP (triceratops.py:673-1485).
 
         Extensions of the reference's arguments: `flux_err_0` may hold one error per time stamp
@@ -173,7 +174,38 @@ class target:
         `self.posterior` is None.  The samples depend on `posterior_seed` and the row (and on
         the round under fpp_err_target, whose rounds merge their samples); lnZ, probs, FPP,
         NFPP, the best-draw tables and numpy's generator are the same bits with and without
-        them.  At an effective sample size of a few, the K samples hold few distinct draws."""
+        them.  At an effective sample size of a few, the K samples hold few distinct draws.
+
+        Adaptive importance sampling (not in the reference; device sampler only):
+        `proposal="adaptive"` draws every scenario call's final N draws from a proposal fitted
+        to its own pilot posteriors instead of from the prior.  Stage 1 runs N_pilot = max(N //
+        8, 10 000) prior draws per call and resamples 4096 posterior samples; a proposal is
+        fitted to their coordinates (_numerics.fit_proposal: per tuned prior dimension a
+        binned reflected KDE, inside a defensive mixture with the prior of weight 0.1); stage 2
+        runs N_pilot draws from it and refits; the final round runs N draws from the stage-2
+        proposal with weights L prior / q; the pilots resample with `posterior_seed`, which
+        therefore also fixes the final draws.  Only the final round enters lnZ, probs, FPP, NFPP,
+        the best-draw tables, the error bars (mc_errors) and the posterior samples; each
+        proposal depends on earlier rounds only, so the evidences stay unbiased.  `N_pilot`
+        holds the pilot draws per call and stage (None with the default "prior", which runs
+        exactly the plain prior sampling).  "adaptive" raises ValueError on the host sampler,
+        with draws sharded over a process group and with fpp_err_target."""
+        if proposal not in ("prior", "adaptive"):
+            raise ValueError("proposal must be 'prior' or 'adaptive', got %r" % (proposal,))
+        adaptive = proposal == "adaptive"
+        if adaptive:
+            from . import marginal_likelihoods as _mlm
+            if _mlm._sampler_mode() != "device":
+                raise ValueError("proposal='adaptive' draws on the device sampler only; the host "
+                                 "sampler keeps numpy-exact parity with the reference "
+                                 "(set_sampler('device'))")
+            if _dispatch._dist() is not None:
+                raise ValueError("proposal='adaptive' fits its proposals on one process: it "
+                                 "cannot be combined with draws sharded over a process group "
+                                 "(vet whole targets per rank instead, batch.vet_many)")
+            if fpp_err_target is not None:
+                raise ValueError("proposal='adaptive' cannot be combined with fpp_err_target")
+        N_pilot = max(int(N) // 8, _PILOT_MIN) if adaptive else None
         post_K = None
         if posterior_samples is not None:
             post_K = _dispatch.check_posterior_K(posterior_samples)
@@ -270,7 +302,8 @@ class target:
                     lnZ[j] = -np.inf
                 return
             calls.append((rows, fn))
-            waiting.append((rows, chain.run(functools.partial(_in_stream, fn, rows[0], N))))
+            waiting.append((rows, chain.run(functools.partial(_in_stream, fn, rows[0],
+                                                              N_pilot if adaptive else N))))
             settle(_PIPELINE_DEPTH)
 
         def say(msg):
@@ -293,8 +326,9 @@ class target:
         moments = _dispatch.mc_errors() if mc_errors else contextlib.nullcontext()
         post = (lambda: _dispatch.posterior_samples(post_K, posterior_seed)) if post_K else \
             contextlib.nullcontext
+        first = _pilot(posterior_seed) if adaptive else post()
         try:
-            with moments, post(), _dispatch.deferring():
+            with moments, first, _dispatch.deferring():
                 for i, ID in enumerate(filtered["ID"].values if not follower else ()):
                     star = {c: filtered[c].values[i] for c in _STAR_COLUMNS}
                     flux, flux_err = renorm_flux(flux_0, flux_err_0, star["fluxratio"])
@@ -388,6 +422,9 @@ class target:
                 "record_exchanges": group.collectives, "scatters": group.scatters}
             _dispatch.close_group()
 
+        if adaptive:
+            with _dispatch.mc_errors() if mc_errors else contextlib.nullcontext():
+                _adapt(calls, row_results, lnZ, best, N, N_pilot, posterior_seed, post)
         if mc_errors and group is None:
             with _dispatch.mc_errors(), post():
                 err = _refine(calls, row_results, lnZ, best, fpp_err_target, N_max,
@@ -428,6 +465,7 @@ class target:
         self.FPP = 1 - (prob[0] + prob[3] + prob[9])
         self.NFPP = np.sum(prob[15:]) if len(prob) > 15 else 0.0
         self.lnZ_err = self.ess = self.N_draws = self.FPP_err = self.NFPP_err = None
+        self.N_pilot = N_pilot
         if err is not None:
             self.lnZ_err, self.ess, self.N_draws = err["lnZ_err"], err["ess"], err["N"]
             self.FPP_err, self.NFPP_err = err["FPP_err"], err["NFPP_err"]
@@ -457,6 +495,69 @@ def _posterior_frame(targets, scenarios, row_results):
         return DataFrame(columns=["ID", "scenario", "row", "draw"]
                          + [name for name, _ in _POSTERIOR_COLUMNS])
     return concat(blocks, ignore_index=True)
+
+
+# adaptive importance sampling (calc_probs(proposal="adaptive"), DESIGN.md section 4g)
+_PILOT_MIN = 10_000       # N_pilot = max(N // 8, _PILOT_MIN) draws per call and stage
+_PILOT_K = 4096           # posterior samples a proposal is fitted to
+_STAGES = 2               # pilot stages before the final round
+
+
+@contextlib.contextmanager
+def _pilot(seed):
+    """A pilot round: K_pilot posterior samples per branch with their coordinates."""
+    from . import device_sampler
+    with _dispatch.posterior_samples(_PILOT_K, seed), device_sampler.record_coords():
+        yield
+
+
+def _fit_call(parts, seed, stream):
+    """Proposal of one scenario call from the pilot posteriors of its branches."""
+    from . import _numerics, device_sampler
+    rows = _numerics.pooled_posterior(
+        [(r.record[0], r.post_total, r.post_coords) for r in parts], _PILOT_K, seed, stream)
+    slots = [d for d in range(_numerics.PROP_SLOTS)
+             if rows.shape[0] and np.all(np.isfinite(rows[:, d]))]
+    return device_sampler.Proposal(_numerics.fit_proposal(rows, slots))
+
+
+def _round(calls, props, n, stage):
+    """One round of every scenario call, n draws from its proposal, a few calls in flight;
+    returns the results of each call (a tuple of its branches)."""
+    from . import device_sampler
+    out, waiting = [], collections.deque()
+
+    def settle(keep):
+        while len(waiting) > keep:
+            res = waiting.popleft()
+            out.append(tuple(_dispatch.resolve(r) for r in
+                             (res if isinstance(res, tuple) else (res,))))
+    with _dispatch.deferring():
+        for (rows, make), p in zip(calls, props):
+            with device_sampler.importance_proposal(p):
+                waiting.append(_in_stream(make, rows[0] + (stage << 32), n))
+            settle(_PIPELINE_DEPTH)
+        settle(0)
+    return out
+
+
+def _adapt(calls, row_results, lnZ, best, N, N_pilot, seed, post):
+    """The adaptive schedule after stage 1 (row_results hold its pilots): fit, _STAGES - 1 more
+    pilot rounds each refitted, then the final round of N draws, whose results replace the rows'
+    lnZ, best-draw rows and results."""
+    parts = [tuple(row_results[j] for j in rows) for rows, _ in calls]
+    for stage in range(1, _STAGES + 1):
+        props = [_fit_call(pt, seed, rows[0] + ((stage - 1) << 32))
+                 for (rows, _), pt in zip(calls, parts)]
+        final = stage == _STAGES
+        with post() if final else _pilot(seed):
+            parts = _round(calls, props, N if final else N_pilot, stage)
+    for (rows, _), pt in zip(calls, parts):
+        for j, res in zip(rows, pt):
+            for k in RESULT_KEYS:
+                best[k][j] = res[k][0]
+            lnZ[j] = res["lnZ"]
+            row_results[j] = res
 
 
 def _in_stream(make, stream, n):
