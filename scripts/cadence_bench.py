@@ -7,7 +7,7 @@ engine call's light curve then gets a second cadence group: the same folded curv
 timed alternately in one process, inputs resident in HBM, CUDA events around every step of
 12 engine calls (18 rows):
 
-  mixed   the two-group light curve on the segmented kernel (lnl_seg_kernel)
+  mixed   the two-group light curve on the segmented instantiation (lnl_kernel<*, true>)
   forced  the same stamps forced to one cadence (0.00139 d, 20): today's workaround
 
 model_points_per_s = 18 * N * sum_g(npts_g * nsamples_g) / step time.  This counts sub-exposure

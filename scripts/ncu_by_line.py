@@ -29,8 +29,8 @@ dis = subprocess.run(["nvdisasm", "-g", "-c", os.path.join(tmp, cubin)], capture
 lines, cur, inside = [], ("?", 0), False
 for ln in dis.splitlines():
     if ln.startswith("//---") and ".text." in ln:
-        # the production instantiation (lnl_kernel<false>) when the kernel is a template
-        inside = KERNEL in ln and "ILb1E" not in ln
+        # the production instantiation lnl_kernel<false, false> (no work counters, one cadence)
+        inside = KERNEL + "ILb0ELb0EE" in ln
         continue
     if not inside:
         continue

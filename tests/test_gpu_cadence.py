@@ -1,8 +1,8 @@
-"""Mixed-cadence light curves on the GPU (tri_set_lightcurve_cadence, lnl_seg_kernel): constant
-cadence arrays are the scalar call, chi^2 is additive over cadence groups on the lnL_*_p seam,
-the L2 seam agrees with the per-group oracle (tests/_cadence_oracle.py), simulated rows come
-back in the caller's order, the C ABI rejects bad cadences, and calc_probs runs on a mixed
-curve with both samplers."""
+"""Mixed-cadence light curves on the GPU (tri_set_lightcurve_cadence, the segmented
+instantiation lnl_kernel<*, true>): constant cadence arrays are the scalar call, chi^2 is additive
+over cadence groups on the lnL_*_p seam, the L2 seam agrees with the per-group oracle
+(tests/_cadence_oracle.py), simulated rows come back in the caller's order, the C ABI rejects bad
+cadences, and calc_probs runs on a mixed curve with both samplers."""
 import ctypes
 import os
 

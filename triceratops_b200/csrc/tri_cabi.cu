@@ -197,7 +197,7 @@ struct Ctx {
     int* d_perm = nullptr;   // sorted stamp -> caller's stamp
     size_t lc_cap = 0;
     LightCurve lc{};
-    CadenceTable cad{};   // n > 1: mixed cadence (lnl_seg_kernel), else n == 1
+    CadenceTable cad{};   // n > 1: mixed cadence (lnl_kernel<*, true>), else n == 1
     Slot slots[kSlots + 1];
     int64_t next_ticket = 1;
     Slot* last = nullptr;    // the call completed last (tri_last_timing, tri_fetch_lnl)
@@ -313,14 +313,16 @@ void finish_result(const LsePartial& r, int64_t N, tri_result* out) {
     else out->lnZ = r.m + std::log(r.s) - std::log((double)N);
 }
 
+// the light-curve instantiation for the current light curve and counting switch
+void (*lnl_instance())(LnlArgs) {
+    const bool seg = g.cad.n > 1;   // mixed cadence: the segmented instantiation
+    if (g.count_work) return seg ? lnl_kernel<true, true> : lnl_kernel<true, false>;
+    return seg ? lnl_kernel<false, true> : lnl_kernel<false, false>;
+}
+
 int launch_lnl(Slot& S, LnlArgs& A, cudaStream_t s) {
-    size_t smem = lnl_smem_bytes();
-    if (g.cad.n > 1) {   // mixed cadence: the segmented instantiation
-        A.cad = g.cad;
-        if (g.count_work) lnl_seg_kernel<true><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
-        else lnl_seg_kernel<false><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
-    } else if (g.count_work) lnl_kernel<true><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
-    else lnl_kernel<false><<<lnl_grid(), kLnlThreads, smem, s>>>(A);
+    if (g.cad.n > 1) A.cad = g.cad;
+    lnl_instance()<<<lnl_grid(), kLnlThreads, lnl_smem_bytes(), s>>>(A);
     S.launches += 1;
     CU(cudaGetLastError());
     return TRI_OK;
@@ -755,7 +757,8 @@ int tri_init(int device) {
     }
     // occupancy of the persistent light-curve kernel
     int bps = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, lnl_kernel<false>, kLnlThreads, 0));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, lnl_kernel<false, false>, kLnlThreads,
+                                                     0));
     g.lnl_blocks_per_sm = std::max(1, bps);
     g.lnl_smem = 0;
     g.ready = true;
@@ -1004,7 +1007,7 @@ static int set_lightcurve(const double* time, const double* flux, const double* 
     // stage the light curve in shared memory only when that costs no occupancy (of the
     // instantiation that will run)
     {
-        void (*kern)(LnlArgs) = g.cad.n > 1 ? lnl_seg_kernel<false> : lnl_kernel<false>;
+        void (*kern)(LnlArgs) = lnl_instance();
         int bps0 = 0, bps1 = 0;
         size_t need = (size_t)(3 * (size_t)npts + 1) * sizeof(double);
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps0, kern, kLnlThreads, 0));

@@ -222,7 +222,7 @@ constexpr int kTopkBins = 1 << 16;   // histogram over the leading 16 key bits (
 // ---- light curve + chi^2 ---------------------------------------------------------------------
 // Mixed cadence (tri_set_lightcurve_cadence): the stamps are sorted by (group, time) and group g
 // owns the sorted stamps [off[g], off[g+1]) of the one light curve (one prefix-sum array over
-// the concatenation).  Read by lnl_seg_kernel only; lnl_kernel's light curve has one cadence.
+// the concatenation).  Read by lnl_kernel<*, true> only; with one cadence the table is unused.
 constexpr int kMaxCadences = 8;   // TRI_MAX_CADENCES
 struct CadenceTable {
     int n;                           // groups
@@ -269,7 +269,7 @@ struct LnlArgs {
     const int* perm;         // sorted stamp j -> caller's stamp index
     int scalar_rule;         // 1: radius-ratio rules of the scalar simulate_EB_transit
                              // (likelihoods.py:121-123, :137) instead of the vectorised ones
-    CadenceTable cad;        // cadence groups (lnl_seg_kernel); lc.exptime is then the largest
+    CadenceTable cad;        // cadence groups (lnl_kernel<*, true>); lc.exptime is then the largest
                              // exposure of the groups, which transit_window's image check uses
 };
 
@@ -320,18 +320,41 @@ struct LnlShared {
     WarpDraw draw[kLnlWarps];
     LsePartial lse[kLnlWarps][2];
     unsigned long long cnt[kLnlWarps][4];   // diagnostic counters of the warp
-    double toff[kToffTable];
+    double toff[kLnlWarps][kToffTable];   // sub-exposure offsets: row 0 for the whole block
+                                          // with one cadence, else the warp's current group
     const double* time;
     const double* flux;
     const double* prefix;
     double lnorm;
 };
 
+// Per-draw state of the segmented instantiation: the transit window, found once and used by
+// every cadence group, the current group's stamps, and the sums over the groups.
+struct SegDraw {
+    double red = 0.0;       // per lane: chi^2 of the groups' window stamps
+    double pre_chi = 0.0;   // chi^2 of the groups' stamps outside the window
+    bool have_win = false;
+    double t_lo = 0.0, t_hi = 0.0, speed = 0.0;   // the window, max_projected_speed
+    int n_win = 0;          // the groups' window stamps
+    int g0, g1;             // the current group's stamps [g0, g1)
+};
+
 // kCount: also count the work classes of SURVEY.md 8(d) (window stamps, evaluated stamps,
 // interior and limb points) into A.counters -- the roofline accounting of bench.py and the
 // n_stamps / n_interior / n_limb diagnostics; the production instantiation leaves them out of
 // the hot loop.
-template <bool kCount>
+// kSeg: the light curve has several cadence groups (A.cad).  Per draw the orbit, limb and
+// dilution set-up, the transit window and (EB-type) the secondary pass run once, as with one
+// cadence; then each group in turn takes its stamp range inside the window (its own half
+// exposure), its own centre-probe radius and sub-exposure half-width in the warp's record, its
+// own sub-exposure offsets in the warp's row of S.toff, the round loop with its own sample
+// count, and the prefix terms of its stamps outside the window.  A compile-time switch, so that
+// the single-cadence instantiation carries none of the per-group bookkeeping.  Where the two are
+// written differently below for the same arithmetic (the pass index, where exptime is set, the
+// per-pass reductions, the segmented state in one SegDraw), the single-cadence form is the one
+// whose SASS is unchanged: which locals exist and where they are defined moves the compiler's
+// register assignment (DESIGN.md section 4h).
+template <bool kCount, bool kSeg>
 __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs A) {
     extern __shared__ double smem[];
     __shared__ LnlShared S;
@@ -356,12 +379,14 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
             S.time = A.lc.time; S.flux = A.lc.flux; S.prefix = A.lc.prefix;
         }
     }
-    // sub-exposure offsets of the observed light curve (the same for every draw)
-    const bool toff_tab = A.lc.nsamples < kToffTable;
-    if (toff_tab) {
+    // sub-exposure offsets of the observed light curve (the same for every draw) in row 0; with
+    // cadence groups every warp fills its own row per group instead, and toff_tab follows the
+    // group
+    bool toff_tab = A.lc.nsamples < kToffTable;
+    if (!kSeg && toff_tab) {
         const double inv = 1.0 / A.lc.nsamples;
         for (int is = threadIdx.x; is <= A.lc.nsamples; is += blockDim.x)
-            S.toff[is] = is ? A.lc.exptime * ((is - 0.5) * inv - 0.5) : 0.0;
+            S.toff[0][is] = is ? A.lc.exptime * ((is - 0.5) * inv - 0.5) : 0.0;
     }
     const int lane = threadIdx.x & 31;
     // (one warp per block: every shared-memory address is a compile-time constant)
@@ -379,6 +404,7 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
     const volatile LnlShared& VS = S;
     const int64_t n_front = A.count_dev ? (int64_t)A.count_dev[0] : A.count;
     const int64_t count = n_front + (A.count_dev ? (int64_t)A.count_dev[3] : 0);
+    constexpr int kPass1 = kSeg ? 0 : 1;   // the first pass over the observed light curve
 
 #pragma unroll 1
     for (;;) {
@@ -393,23 +419,33 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
         const int64_t i = item >> 1;
         const int twin = (int)(item & 1);
 
-        // Two passes through ONE copy of the model code: pass 0 (EB-type only) is the
+        // Passes through ONE copy of the model code: pass kPass1 - 1 (EB-type only) is the
         // 25-stamp secondary eclipse on [-0.05, 0.05] d with the roles swapped and no
-        // supersampling (likelihoods.py:417-423), reduced with a minimum; pass 1 is the
-        // observed light curve, reduced to chi^2.
+        // supersampling (likelihoods.py:417-423), reduced with a minimum; pass kPass1 + g is
+        // cadence group g of the observed light curve (the whole curve without kSeg), reduced to
+        // chi^2.
         double chi = 0.0;
+        SegDraw sg;   // kSeg only
         bool cut = false;
         int jlo = 0, jhi = 0;
         unsigned n_interior = 0, n_limb = 0;   // per lane, this draw
         unsigned n_skip = 0;                    // per lane: stamps the centre probe dismissed
 #pragma unroll 1
-        for (int pass = A.eb ? 0 : 1; pass < 2; ++pass) {
-            const bool primary = (pass == 1);
-            const int ns = primary ? A.lc.nsamples : 1;
+        for (int pass = A.eb ? kPass1 - 1 : kPass1; pass < kPass1 + (kSeg ? A.cad.n : 1); ++pass) {
+            const bool primary = pass >= kPass1;
+            const int grp = pass - kPass1;
+            const int ns = primary ? (kSeg ? A.cad.nsamples[grp] : A.lc.nsamples) : 1;
+            // (one cadence: set with the per-sample constants below)
+            double exptime = kSeg && primary ? A.cad.exptime[grp] : 0.0;
+            if constexpr (kSeg) {
+                sg.g0 = primary ? A.cad.off[grp] : 0;
+                sg.g1 = primary ? A.cad.off[grp + 1] : 25;
+            }
             bool probe;
-            {
+            if (!kSeg || grp <= 0) {
                 // ---- per-sample constants (every lane computes the same values); nothing of
-                // this block stays in registers across the stamp loop
+                // this block stays in registers across the stamp loop.  The cadence groups
+                // share them: with kSeg the block runs for the secondary and the first group.
                 const double P = A.P.at(i), e = A.ecc.at(i), argp = A.argp.at(i);
                 const double rhost = A.rhost.at(i);
                 const double a_rs = A.a.at(i) / (rhost * kRsun);          // likelihoods.py:343 / :409
@@ -453,38 +489,80 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                 orbit_setup(o, A.tab, k, P, a_rs, inc, e, w_rad);
                 Limb L;
                 limb_setup(L, A.u1.at(i), A.u2.at(i), k);
-                const double exptime = primary ? A.lc.exptime : 0.0;
-                if (primary) {
-                    // time stamps that can be in transit
-                    jlo = 0;
-                    jhi = npts;
-                    Window win;
-                    if (transit_window(o, A.tab, a_rs, P, A.lc, win)) {
-                        double half = 0.5 * A.lc.exptime;
-                        const double* tp = VS.time;
-                        jlo = lower_bound(tp, npts, win.t_lo - half);
-                        jhi = lower_bound(tp, npts, win.t_hi + half);
-                        if (jhi < jlo) jhi = jlo;
+                double skip_beyond;
+                if constexpr (!kSeg) {
+                    exptime = primary ? A.lc.exptime : 0.0;
+                    if (primary) {
+                        // time stamps that can be in transit
+                        jlo = 0;
+                        jhi = npts;
+                        Window win;
+                        if (transit_window(o, A.tab, a_rs, P, A.lc, win)) {
+                            double half = 0.5 * A.lc.exptime;
+                            const double* tp = VS.time;
+                            jlo = lower_bound(tp, npts, win.t_lo - half);
+                            jhi = lower_bound(tp, npts, win.t_hi + half);
+                            if (jhi < jlo) jhi = jlo;
+                        }
+                    } else {
+                        jlo = 0;
+                        jhi = 25;
                     }
-                } else {
-                    jlo = 0;
-                    jhi = 25;
+                    // centre probe (see max_projected_speed): only worth it with supersampling
+                    probe = primary && ns > 1 && !o.table_clamped;
+                    skip_beyond =
+                        1.0 + k + max_projected_speed(o, a_rs) * (0.5 * exptime) + 1e-9;
+                } else if (primary) {
+                    // one window for every group: the image check uses the largest exposure
+                    Window win;
+                    sg.have_win = transit_window(o, A.tab, a_rs, P, A.lc, win);
+                    sg.t_lo = win.t_lo;
+                    sg.t_hi = win.t_hi;
                 }
-                // centre probe (see max_projected_speed): only worth it with supersampling
-                probe = primary && ns > 1 && !o.table_clamped;
-                const double skip_beyond =
-                    1.0 + k + max_projected_speed(o, a_rs) * (0.5 * exptime) + 1e-9;
+                if constexpr (kSeg) sg.speed = max_projected_speed(o, a_rs);
                 __syncwarp();
                 if (lane == 0) {
                     wd.o = o;
                     wd.L = L;
-                    wd.skip_beyond = skip_beyond;
-                    // table_clamped orbits (e >= 0.95) always take the generic path
-                    wd.half_ma = o.table_clamped ? 1e30
-                                                 : o.n_rate * (0.5 * exptime) * (1.0 + 1e-9) + 1e-12;
+                    if constexpr (!kSeg) {
+                        wd.skip_beyond = skip_beyond;
+                        // table_clamped orbits (e >= 0.95) always take the generic path
+                        wd.half_ma = o.table_clamped
+                                         ? 1e30 : o.n_rate * (0.5 * exptime) * (1.0 + 1e-9) + 1e-12;
+                    }
                     wd.d1 = d1;
                     wd.d2 = d2;
                     wd.two_stage = two_stage;
+                }
+                __syncwarp();
+            }
+            if constexpr (kSeg) {
+                // ---- the group's stamp range, probe radius, sub-exposure half-width and offsets
+                jlo = sg.g0;
+                jhi = sg.g1;
+                const double half = 0.5 * exptime;
+                if (primary && sg.have_win) {
+                    if (sg.t_hi + half < A.cad.tmin[grp] || sg.t_lo - half > A.cad.tmax[grp]) {
+                        jhi = jlo;
+                    } else {
+                        const double* tp = VS.time;
+                        jlo = sg.g0 + lower_bound(tp + sg.g0, sg.g1 - sg.g0, sg.t_lo - half);
+                        jhi = sg.g0 + lower_bound(tp + sg.g0, sg.g1 - sg.g0, sg.t_hi + half);
+                        if (jhi < jlo) jhi = jlo;
+                    }
+                }
+                const bool clamped = vd.o.table_clamped;
+                probe = primary && ns > 1 && !clamped;
+                toff_tab = ns < kToffTable;
+                __syncwarp();   // every lane is done with the previous group's record and offsets
+                if (lane == 0) {
+                    wd.skip_beyond = 1.0 + vd.o.k + sg.speed * half + 1e-9;
+                    wd.half_ma = clamped ? 1e30 : vd.o.n_rate * half * (1.0 + 1e-9) + 1e-12;
+                }
+                if (primary && toff_tab) {
+                    const double inv = 1.0 / ns;
+                    for (int is = lane; is <= ns; is += 32)
+                        S.toff[warp][is] = is ? exptime * ((is - 0.5) * inv - 0.5) : 0.0;
                 }
                 __syncwarp();
             }
@@ -505,16 +583,21 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                     const unsigned bf = b & 0xffffu, bb = b >> 16;
                     jlo += bf ? (__ffs(bf) - 1) : 16;
                     jhi -= bb ? (__ffs(bb) - 1) : 16;
-                    if (jlo >= jhi) { jhi = jlo = (jlo < npts ? jlo : npts); break; }
+                    if (jlo >= jhi) {
+                        jhi = jlo = (jlo < (kSeg ? sg.g1 : npts) ? jlo : (kSeg ? sg.g1 : npts));
+                        break;
+                    }
                     if (bf && bb) break;
                 }
             }
             if (primary && A.model_out) {   // outside the window the model is exactly 1
                 double* row = A.model_out + (size_t)w * npts;
-                for (int j = lane; j < npts; j += 32)
+                for (int j = (kSeg ? sg.g0 : 0) + lane; j < (kSeg ? sg.g1 : npts); j += 32)
                     if (j < jlo || j >= jhi) row[A.perm[j]] = 1.0;
             }
-            double red = primary ? 0.0 : INFINITY;
+            // per lane: the pass's chi^2 (with kSeg sg.red, which runs on over the groups) or, on
+            // the secondary pass, its minimum
+            double red = primary && !kSeg ? 0.0 : INFINITY;
             // lane <-> time stamp, serial over sub-exposures.  Full rounds take 16 stamps from
             // the front of the window and 16 from its back: ingress and egress mirror each
             // other, so the two halves of the warp are in the same occultation case (limb or
@@ -561,13 +644,14 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
 #pragma unroll 1
                         for (int is = is_lo; is <= is_hi; ++is) {
                             // sub-exposure offset exptime ((is - 1/2)/ns - 1/2), tabulated per
-                            // block (the back half of a paired round runs its sub-exposures
-                            // backwards in time, the mirror image of the front half)
+                            // block (kSeg: per warp and group; the back half of a paired round
+                            // runs its sub-exposures backwards in time, the mirror image of the
+                            // front half)
                             const int iso = mirror ? ns + 1 - is : is;
                             double toff = 0.0;
                             if (primary)
-                                toff = toff_tab ? S.toff[iso]
-                                                : A.lc.exptime * ((iso - 0.5) / ns - 0.5);
+                                toff = toff_tab ? S.toff[kSeg ? warp : 0][iso]
+                                                : exptime * ((iso - 0.5) / ns - 0.5);
                             const double z = fast ? z_sub(vd.o, A.tab, so, toff)
                                                   : z_at(vd.o, A.tab, t + toff);
                             int cls = 0;   // work class of SURVEY.md 8(d): 1 interior, 2 limb-crossing
@@ -593,7 +677,8 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                         if (A.model_out) A.model_out[(size_t)w * npts + A.perm[j]] = md;
                         const double* fp = VS.flux;
                         const double rr = fp[j] - md;
-                        red = fma(A.lc.weight ? rr * __ldg(A.lc.weight + j) : rr, rr, red);
+                        double& sum = kSeg ? sg.red : red;
+                        sum = fma(A.lc.weight ? rr * __ldg(A.lc.weight + j) : rr, rr, sum);
                     } else {
                         red = fmin(red, m);
                     }
@@ -610,6 +695,10 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                 if (A.secdepth_out && lane == 0) A.secdepth_out[w] = sd;
                 cut = !twin && !(sd < 1.5 * A.lc.sigma);                 // :535-538
                 if (cut) break;
+            } else if constexpr (kSeg) {
+                const double* pre = VS.prefix;
+                sg.pre_chi += (pre[jlo] - pre[sg.g0]) + (pre[sg.g1] - pre[jhi]);
+                sg.n_win += jhi - jlo;
             } else {
                 chi = warp_sum(red);
             }
@@ -619,8 +708,12 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
         if (cut) {
             val = A.raw ? INFINITY : -INFINITY;
         } else {
-            const double* pre = VS.prefix;
-            chi += (pre[jlo] - pre[0]) + (pre[npts] - pre[jhi]);
+            if constexpr (kSeg) {
+                chi = warp_sum(sg.red) + sg.pre_chi;
+            } else {
+                const double* pre = VS.prefix;
+                chi += (pre[jlo] - pre[0]) + (pre[npts] - pre[jhi]);
+            }
             const double sigma = A.lc.sigma;
             const double half_chi2 = A.lc.weight ? 0.5 * chi              // weights carry 1/sigma_j^2
                                                  : 0.5 * (chi / (sigma * sigma));   // likelihoods.py:486
@@ -634,8 +727,8 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                 c_limb += __shfl_xor_sync(0xffffffffu, c_limb, o);
             }
             if (lane == 0 && !cut) {
-                S.cnt[warp][0] += (unsigned long long)(jhi - jlo);
-                S.cnt[warp][1] += (unsigned long long)(jhi - jlo) - c_skip;
+                S.cnt[warp][0] += (unsigned long long)(kSeg ? sg.n_win : jhi - jlo);
+                S.cnt[warp][1] += (unsigned long long)(kSeg ? sg.n_win : jhi - jlo) - c_skip;
                 S.cnt[warp][2] += c_int;
                 S.cnt[warp][3] += c_limb;
             }
@@ -668,332 +761,6 @@ __global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_kernel(LnlArgs
                 for (int wv = 0; wv < kLnlWarps; ++wv) v += S.cnt[wv][c];
                 if (v) atomicAdd(A.counters + c, v);
             }
-        }
-    }
-}
-
-// Segmented instantiation of lnl_kernel for a light curve with several cadence groups (A.cad).
-// A separate body, so that the single-cadence kernel above keeps its code.  Per draw: the orbit,
-// limb and dilution set-up, the transit window and (EB-type) the secondary pass 0 run once, as
-// there; then each group in turn takes its stamp range inside the window (its own half
-// exposure), its own centre-probe radius and sub-exposure half-width in the warp's record, its
-// own sub-exposure offsets in S.toff, the round loop with its own sample count, and the prefix
-// terms of its stamps outside the window.
-template <bool kCount>
-__global__ void __launch_bounds__(kLnlThreads, kLnlMinBlocks) lnl_seg_kernel(LnlArgs A) {
-    static_assert(kLnlWarps == 1, "S.toff is refilled per group: one warp per block");
-    extern __shared__ double smem[];
-    __shared__ LnlShared S;
-    if (A.lc.time == nullptr) return;
-    const int npts = A.lc.npts;
-    {
-        size_t need = (size_t)(3 * npts + 1) * sizeof(double);
-        unsigned dyn;
-        asm volatile("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn));
-        if (need <= dyn) {
-            double* st = smem;
-            double* sf = smem + npts;
-            double* sp = smem + 2 * npts;
-            for (int j = threadIdx.x; j < npts; j += blockDim.x) {
-                st[j] = A.lc.time[j];
-                sf[j] = A.lc.flux[j];
-            }
-            for (int j = threadIdx.x; j <= npts; j += blockDim.x) sp[j] = A.lc.prefix[j];
-            if (threadIdx.x == 0) { S.time = st; S.flux = sf; S.prefix = sp; }
-        } else if (threadIdx.x == 0) {
-            S.time = A.lc.time; S.flux = A.lc.flux; S.prefix = A.lc.prefix;
-        }
-    }
-    const int lane = threadIdx.x & 31;
-    constexpr int warp = 0;
-    if (lane == 0) {
-        S.lse[warp][0] = LsePartial{-INFINITY, 0.0, 0, 0};
-        S.lse[warp][1] = LsePartial{-INFINITY, 0.0, 0, 0};
-        for (int c = 0; c < 4; ++c) S.cnt[warp][c] = 0;
-    }
-    if (threadIdx.x == 0) S.lnorm = -0.5 * log(2.0 * kPi) - log(A.lc.sigma);
-    __syncthreads();
-    WarpDraw& wd = S.draw[warp];
-    const volatile WarpDraw& vd = S.draw[warp];
-    const volatile LnlShared& VS = S;
-    const int64_t n_front = A.count_dev ? (int64_t)A.count_dev[0] : A.count;
-    const int64_t count = n_front + (A.count_dev ? (int64_t)A.count_dev[3] : 0);
-    const int n_groups = A.cad.n;
-
-#pragma unroll 1
-    for (;;) {
-        unsigned long long w = 0;
-        if (lane == 0) w = atomicAdd(A.next, 1ull);
-        w = __shfl_sync(0xffffffffu, w, 0);
-        if ((int64_t)w >= count) break;
-        const int64_t slot = ((int64_t)w < n_front) ? (int64_t)w
-                                                    : A.items_cap - 1 - ((int64_t)w - n_front);
-        const int64_t item = !A.items ? (((int64_t)w << 1) | A.twin_uniform) : A.items[slot];
-        const int64_t i = item >> 1;
-        const int twin = (int)(item & 1);
-
-        // segment -1: the secondary eclipse (EB-type); segment g >= 0: cadence group g
-        double red = 0.0;          // per lane: chi^2 of the groups' window stamps
-        double pre_chi = 0.0;      // warp-uniform: the groups' stamps outside the window
-        bool cut = false;
-        bool have_win = false;
-        double t_lo = 0.0, t_hi = 0.0, speed = 0.0;
-        unsigned n_interior = 0, n_limb = 0, n_skip = 0;
-        int n_win = 0;
-#pragma unroll 1
-        for (int seg = A.eb ? -1 : 0; seg < n_groups; ++seg) {
-            const bool primary = seg >= 0;
-            const int ns = primary ? A.cad.nsamples[seg] : 1;
-            const double exptime = primary ? A.cad.exptime[seg] : 0.0;
-            const int g0 = primary ? A.cad.off[seg] : 0;
-            const int g1 = primary ? A.cad.off[seg + 1] : 25;
-            if (seg <= 0) {
-                // ---- per-sample constants, once per pass (as in lnl_kernel)
-                const double P = A.P.at(i), e = A.ecc.at(i), argp = A.argp.at(i);
-                const double rhost = A.rhost.at(i);
-                const double a_rs = A.a.at(i) / (rhost * kRsun);
-                const double inc = A.inc.at(i) * (kPi / 180.0);
-                const double cfr = A.cfr.at(i);
-                const double F_comp = cfr / (1.0 - cfr);
-                double k_pri, k_sec = 0.0, d1, d2, F_EB;
-                int two_stage;
-                if (!A.eb) {
-                    k_pri = A.body.at(i) * kRearth / (rhost * kRsun);
-                    two_stage = 0;
-                    d1 = 0.0;
-                    d2 = A.companion_is_host ? 1.0 / F_comp : F_comp / 1.0;
-                } else {
-                    const double reb = A.body.at(i);
-                    const double fr = A.ebfr.at(i);
-                    F_EB = fr / (1.0 - fr);
-                    k_pri = reb / rhost;
-                    if (!A.scalar_rule) {
-                        if ((k_pri - 1.0) < 1e-6) k_pri *= 0.999;
-                        k_sec = rhost / reb;
-                        if ((k_sec - 1.0) < 1e-6) k_sec *= 0.999;
-                    } else {
-                        if (fabs(k_pri - 1.0) < 1e-6) k_pri *= 0.999;
-                        k_sec = 1.0 / k_pri;
-                    }
-                    two_stage = 1;
-                    if (A.companion_is_host) {
-                        d1 = F_EB / F_comp;
-                        d2 = 1.0 / (F_comp + F_EB);
-                    } else {
-                        d1 = F_EB / 1.0;
-                        d2 = F_comp / (1.0 + F_EB);
-                    }
-                }
-                const double k = primary ? k_pri : k_sec;
-                const double w_rad = primary ? (90.0 - argp) * (kPi / 180.0)
-                                             : (90.0 - argp + 180.0) * (kPi / 180.0);
-                Orbit o;
-                orbit_setup(o, A.tab, k, P, a_rs, inc, e, w_rad);
-                Limb L;
-                limb_setup(L, A.u1.at(i), A.u2.at(i), k);
-                if (primary) {
-                    // one window for every group: the image check uses the largest exposure
-                    Window win;
-                    have_win = transit_window(o, A.tab, a_rs, P, A.lc, win);
-                    t_lo = win.t_lo;
-                    t_hi = win.t_hi;
-                }
-                speed = max_projected_speed(o, a_rs);
-                __syncwarp();
-                if (lane == 0) {
-                    wd.o = o;
-                    wd.L = L;
-                    wd.d1 = d1;
-                    wd.d2 = d2;
-                    wd.two_stage = two_stage;
-                }
-                __syncwarp();
-            }
-            // ---- this segment's stamp range, probe radius, sub-exposure half-width and offsets
-            int jlo = g0, jhi = g1;
-            const double half = 0.5 * exptime;
-            if (primary && have_win) {
-                if (t_hi + half < A.cad.tmin[seg] || t_lo - half > A.cad.tmax[seg]) {
-                    jhi = jlo;
-                } else {
-                    const double* tp = VS.time;
-                    jlo = g0 + lower_bound(tp + g0, g1 - g0, t_lo - half);
-                    jhi = g0 + lower_bound(tp + g0, g1 - g0, t_hi + half);
-                    if (jhi < jlo) jhi = jlo;
-                }
-            }
-            const bool clamped = vd.o.table_clamped;
-            const bool probe = primary && ns > 1 && !clamped;
-            const bool toff_tab = ns < kToffTable;
-            __syncwarp();   // every lane is done with the previous segment's record and offsets
-            if (lane == 0) {
-                wd.skip_beyond = 1.0 + vd.o.k + speed * half + 1e-9;
-                wd.half_ma = clamped ? 1e30 : vd.o.n_rate * half * (1.0 + 1e-9) + 1e-12;
-            }
-            if (primary && toff_tab) {
-                const double inv = 1.0 / ns;
-                for (int is = lane; is <= ns; is += 32)
-                    S.toff[is] = is ? exptime * ((is - 0.5) * inv - 0.5) : 0.0;
-            }
-            __syncwarp();
-            if (probe) {
-#pragma unroll 1
-                for (;;) {
-                    const bool back = lane >= 16;
-                    const int j = back ? jhi - 1 - (lane - 16) : jlo + lane;
-                    bool keep = false;
-                    if (j >= jlo && j < jhi) {
-                        const double* tp = VS.time;
-                        keep = !(fabs(z_at(vd.o, A.tab, tp[j])) > vd.skip_beyond);
-                    }
-                    const unsigned b = __ballot_sync(0xffffffffu, keep);
-                    const unsigned bf = b & 0xffffu, bb = b >> 16;
-                    jlo += bf ? (__ffs(bf) - 1) : 16;
-                    jhi -= bb ? (__ffs(bb) - 1) : 16;
-                    if (jlo >= jhi) { jhi = jlo = (jlo < g1 ? jlo : g1); break; }
-                    if (bf && bb) break;
-                }
-            }
-            if (primary && A.model_out) {   // outside the window the model is exactly 1
-                double* row = A.model_out + (size_t)w * npts;
-                for (int j = g0 + lane; j < g1; j += 32)
-                    if (j < jlo || j >= jhi) row[A.perm[j]] = 1.0;
-            }
-            double red_sec = INFINITY;
-            // the round structure of lnl_kernel: full rounds pair the front and the back of the
-            // range, the remainder shares sub-exposures between 2 or 4 lanes
-            const int n_full = (jhi - jlo) >> 5;
-            const int rem = (jhi - jlo) - 32 * n_full;
-#pragma unroll 1
-            for (int r = 0; r < n_full + (rem > 0 ? 1 : 0); ++r) {
-                int gsh = 0, j, sub = 0;
-                bool have = true;
-                bool mirror = false;
-                if (r < n_full) {
-                    mirror = lane >= 16;
-                    j = mirror ? jhi - 16 * r - 1 - (lane - 16) : jlo + 16 * r + lane;
-                } else {
-                    gsh = (primary && ns >= 4) ? (rem <= 8 ? 2 : (rem <= 16 ? 1 : 0)) : 0;
-                    j = jlo + 16 * n_full + (lane >> gsh);
-                    sub = lane & ((1 << gsh) - 1);
-                    have = (lane >> gsh) < rem;
-                }
-                double acc = 0.0;
-                if (have) {
-                    double t;
-                    if (primary) {
-                        const double* tp = VS.time;
-                        t = tp[j];
-                    } else {
-                        t = (j == 24) ? 0.05 : -0.05 + j * ((0.05 - -0.05) / 24.0);
-                    }
-                    const int is_lo = 1 + ((sub * ns) >> gsh), is_hi = ((sub + 1) * ns) >> gsh;
-                    StampOrbit so;
-                    bool fast;
-                    const double zc = stamp_centre(vd.o, A.tab, t, vd.half_ma, so, fast);
-                    if (probe && fabs(zc) > vd.skip_beyond) {
-                        acc = (double)(is_hi - is_lo + 1);
-                        if (kCount) n_skip += (sub == 0);
-                    } else {
-#pragma unroll 1
-                        for (int is = is_lo; is <= is_hi; ++is) {
-                            const int iso = mirror ? ns + 1 - is : is;
-                            double toff = 0.0;
-                            if (primary)
-                                toff = toff_tab ? S.toff[iso] : exptime * ((iso - 0.5) / ns - 0.5);
-                            const double z = fast ? z_sub(vd.o, A.tab, so, toff)
-                                                  : z_at(vd.o, A.tab, t + toff);
-                            int cls = 0;
-                            const double k = vd.o.k;
-                            acc += (z > 1.0 + k) ? 1.0 : occult_quad(z, k, vd.L, cls);
-                            if (kCount) {
-                                n_interior += (unsigned)(primary && cls == 1);
-                                n_limb += (unsigned)(primary && cls == 2);
-                            }
-                        }
-                    }
-                }
-                if (gsh) {
-                    acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-                    if (gsh == 2) acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-                }
-                if (have && sub == 0) {
-                    double m = acc / ns;
-                    if (primary) {
-                        if (vd.two_stage) m = (m + vd.d1) / (1.0 + vd.d1);
-                        const double d2 = vd.d2;
-                        const double md = (m + d2) / (1.0 + d2);
-                        if (A.model_out) A.model_out[(size_t)w * npts + A.perm[j]] = md;
-                        const double* fp = VS.flux;
-                        const double rr = fp[j] - md;
-                        red = fma(A.lc.weight ? rr * __ldg(A.lc.weight + j) : rr, rr, red);
-                    } else {
-                        red_sec = fmin(red_sec, m);
-                    }
-                }
-            }
-            if (!primary) {
-                double sec = warp_min(red_sec);
-                const double cfr = A.cfr.at(i), fr = A.ebfr.at(i);
-                const double F_comp = cfr / (1.0 - cfr), F_EB = fr / (1.0 - fr);
-                if (A.companion_is_host) sec = (sec + F_comp / F_EB) / (1.0 + F_comp / F_EB);
-                else sec = (sec + 1.0 / F_EB) / (1.0 + 1.0 / F_EB);
-                const double d2 = vd.d2;
-                const double sd = 1.0 - (sec + d2) / (1.0 + d2);
-                if (A.secdepth_out && lane == 0) A.secdepth_out[w] = sd;
-                cut = !twin && !(sd < 1.5 * A.lc.sigma);                 // :535-538
-                if (cut) break;
-            } else {
-                const double* pre = VS.prefix;
-                pre_chi += (pre[jlo] - pre[g0]) + (pre[g1] - pre[jhi]);
-                n_win += jhi - jlo;
-            }
-        }
-        double* outp = (twin && A.out_twin) ? A.out_twin : A.out;
-        double val;
-        if (cut) {
-            val = A.raw ? INFINITY : -INFINITY;
-        } else {
-            const double chi = warp_sum(red) + pre_chi;
-            const double sigma = A.lc.sigma;
-            const double half_chi2 = A.lc.weight ? 0.5 * chi
-                                                 : 0.5 * (chi / (sigma * sigma));
-            val = A.raw ? half_chi2 : S.lnorm - half_chi2;
-        }
-        if (kCount && A.counters) {
-            unsigned long long c_skip = n_skip, c_int = n_interior, c_limb = n_limb;
-            for (int o = 16; o > 0; o >>= 1) {
-                c_skip += __shfl_xor_sync(0xffffffffu, c_skip, o);
-                c_int += __shfl_xor_sync(0xffffffffu, c_int, o);
-                c_limb += __shfl_xor_sync(0xffffffffu, c_limb, o);
-            }
-            if (lane == 0 && !cut) {
-                S.cnt[warp][0] += (unsigned long long)n_win;
-                S.cnt[warp][1] += (unsigned long long)n_win - c_skip;
-                S.cnt[warp][2] += c_int;
-                S.cnt[warp][3] += c_limb;
-            }
-        }
-        if (lane == 0) {
-            outp[i] = val;
-            if (A.cval) A.cval[slot] = val;
-            if (A.lse_partials) {
-                double x = val;
-                if (A.lnprior.p) x += A.lnprior.at(i);
-                lse_push(S.lse[warp][twin], x);
-                if (A.hist16 && isfinite(val))
-                    atomicAdd(A.hist16 + twin * kTopkBins + (int)(topk_key(val) >> 48), 1u);
-            }
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (A.lse_partials) {
-            for (int b = 0; b < 2; ++b) A.lse_partials[(size_t)b * gridDim.x + blockIdx.x] = S.lse[0][b];
-        }
-        if (kCount && A.counters) {
-            for (int c = 0; c < 4; ++c)
-                if (S.cnt[0][c]) atomicAdd(A.counters + c, S.cnt[0][c]);
         }
     }
 }
