@@ -260,18 +260,61 @@ const void* via_pinned(Slot& S, const void* src, size_t bytes) {
     return hp;
 }
 
-// copy one host column to the slot's staging arena
-int stage(Slot& S, const tri_col& h, int64_t N, Col& d, cudaStream_t s) {
-    if (h.ptr == nullptr) {
-        d = Col{nullptr, 0};
-        return TRI_OK;
-    }
-    if (h.stride != 0 && h.stride != 1) return fail(TRI_EINVAL, "column stride must be 0 or 1");
-    size_t n = h.stride ? (size_t)N : 1;
+// copy one host column (if any) to the slot's staging arena: `c` then names the device copy
+int stage(Slot& S, tri_col& c, int64_t N, cudaStream_t s) {
+    if (c.ptr == nullptr) return TRI_OK;
+    size_t n = c.stride ? (size_t)N : 1;
     double* p = S.staging.take<double>(n);
-    CU(cudaMemcpyAsync(p, via_pinned(S, h.ptr, n * sizeof(double)), n * sizeof(double),
+    CU(cudaMemcpyAsync(p, via_pinned(S, c.ptr, n * sizeof(double)), n * sizeof(double),
                        cudaMemcpyHostToDevice, s));
-    d = Col{p, h.stride};
+    c.ptr = p;
+    return TRI_OK;
+}
+
+// One evaluation as the submission path sees it, whichever public layout it came in: 1 branch
+// (tri_tp_args) or 2 (tri_eb_args: the EB and EBx2P branches), body = rp or reb.  A TP-type
+// call has no ebfr and q (NULL) and scalar_loop 0.
+struct Call {
+    int branches;
+    int64_t N;
+    tri_col body, ebfr, q, P, inc, ecc, argp, mtot, rhost, u1, u2, cfr, lnprior;
+    const uint8_t* extra_mask;
+    int companion_is_host, scalar_loop;
+};
+
+// The adapters of the two public layouts (nullptr for a NULL argument).
+const Call* as_call(const tri_tp_args* a, Call& c) {
+    if (!a) return nullptr;
+    c = Call{1, a->N, a->rp, {}, {}, a->P_orb, a->inc, a->ecc, a->argp, a->mtot, a->rhost, a->u1,
+             a->u2, a->cfr, a->lnprior, a->extra_mask, a->companion_is_host, 0};
+    return &c;
+}
+
+const Call* as_call(const tri_eb_args* a, Call& c) {
+    if (!a) return nullptr;
+    c = Call{2, a->N, a->reb, a->ebfr, a->q, a->P_orb, a->inc, a->ecc, a->argp, a->mtot,
+             a->rhost, a->u1, a->u2, a->cfr, a->lnprior, a->extra_mask, a->companion_is_host,
+             a->scalar_loop};
+    return &c;
+}
+
+// The columns of a call in staging order, and which calls require each: `need` 1 every call,
+// 2 EB-type calls only, 0 none (lnprior is optional).
+struct CallCol {
+    tri_col Call::*col;
+    int need;
+};
+constexpr CallCol kCallCols[] = {
+    {&Call::body, 1}, {&Call::ebfr, 2}, {&Call::q, 2},     {&Call::P, 1},   {&Call::inc, 1},
+    {&Call::ecc, 1},  {&Call::argp, 1}, {&Call::mtot, 1},  {&Call::rhost, 1}, {&Call::u1, 1},
+    {&Call::u2, 1},   {&Call::cfr, 1},  {&Call::lnprior, 0}};
+
+// copy the call's host columns to the slot's staging arena: `c` then names the device copies
+int stage_call(Slot& S, Call& c, cudaStream_t s) {
+    for (const CallCol& k : kCallCols) {
+        int rc = stage(S, c.*k.col, c.N, s);
+        if (rc) return rc;
+    }
     return TRI_OK;
 }
 
@@ -280,7 +323,8 @@ int lnl_grid() { return g.sm_count * std::max(1, g.lnl_blocks_per_sm); }
 size_t lnl_smem_bytes() { return g.lnl_smem; }
 
 struct Scratch {
-    double *a = nullptr, *p = nullptr, *lnl = nullptr, *lnl_twin = nullptr, *cval = nullptr;
+    double *a = nullptr, *cval = nullptr;
+    double* lnl[2] = {nullptr, nullptr};   // per branch
     int64_t* items = nullptr;
     LsePartial* partials = nullptr;   // [2][lnl_grid()]
 };
@@ -292,10 +336,11 @@ int lse_blocks(int64_t N) {
 
 int64_t post_tiles(int64_t N) { return (N + kPostTile - 1) / kPostTile; }
 
-size_t scratch_bytes(int64_t N, bool eb) {
+// (sized for an EB-type call: a slot serves both kinds in turn)
+size_t scratch_bytes(int64_t N) {
     size_t n = (size_t)N;
     size_t b = 0;
-    b += (n * 8 + 256) * (eb ? 4 : 2);   // a, lnl (+ p, lnl_twin)
+    b += (n * 8 + 256) * 4;              // a, p, lnl of the two branches
     b += (n * 8 + 256) * 2;              // items, cval
     b += (size_t)lnl_grid() * sizeof(LsePartial) * 2 + 512;
     b += (size_t)lse_blocks(N) * sizeof(double) * 2 + 256;   // moments_kernel partials
@@ -358,8 +403,8 @@ int launch_finalize(Slot& S, const Scratch& W, int64_t N, int branches, const tr
 int launch_moments(Slot& S, const Scratch& W, int64_t N, int branches, Col lnprior,
                    cudaStream_t s) {
     MomentsArgs M{};
-    M.lnl[0] = W.lnl;
-    M.lnl[1] = W.lnl_twin;
+    M.lnl[0] = W.lnl[0];
+    M.lnl[1] = W.lnl[1];
     M.lnprior = lnprior;
     M.N = N;
     M.branches = branches;
@@ -378,8 +423,8 @@ int launch_moments(Slot& S, const Scratch& W, int64_t N, int branches, Col lnpri
 int launch_posterior(Slot& S, const Scratch& W, int64_t N, int branches, Col lnprior,
                      cudaStream_t s) {
     PosteriorArgs P{};
-    P.lnl[0] = W.lnl;
-    P.lnl[1] = W.lnl_twin;
+    P.lnl[0] = W.lnl[0];
+    P.lnl[1] = W.lnl[1];
     P.lnprior = lnprior;
     P.N = N;
     P.tiles = post_tiles(N);
@@ -411,147 +456,95 @@ size_t lse_out_bytes(const Slot& S, int branches) {
                                                    : branches * sizeof(LsePartial);
 }
 
-void capture_posterior(Slot& S) {
-    S.post_K = g.post_K;
-    S.post_seed = g.post_seed;
-    S.post_stream = g.post_stream;
+// The LnlArgs fields that every launch of the light-curve kernel sets alike: light curve, orbit
+// table, kind and the model columns of `c` (device pointers), with the period column P and the
+// semi-major axis a given apart.  The caller adds its work list and its outputs.
+LnlArgs lnl_args(const Call& c, Col P, Col a) {
+    LnlArgs A{};
+    A.lc = g.lc; A.tab = g.tab; A.eb = c.branches - 1; A.companion_is_host = c.companion_is_host;
+    A.body = to_col(c.body); A.ebfr = to_col(c.ebfr);
+    A.P = P; A.inc = to_col(c.inc); A.a = a; A.rhost = to_col(c.rhost);
+    A.u1 = to_col(c.u1); A.u2 = to_col(c.u2); A.ecc = to_col(c.ecc); A.argp = to_col(c.argp);
+    A.cfr = to_col(c.cfr);
+    A.scalar_rule = c.scalar_loop ? 1 : 0;
+    return A;
 }
 
-// Queue one TP-type evaluation on `s` for slot S: every pointer in `a` and in `r` (lnL_out,
-// mask_out, top_idx, top_lnL) is a device pointer.  Nothing here waits for the GPU; the small
-// result record lands in the slot's pinned buffers and is read by finish_slot.
-int enqueue_tp(Slot& S, const tri_tp_args& a, const tri_result& r, cudaStream_t s) {
-    const int64_t N = a.N;
+// Queue one evaluation on `s` for slot S: every pointer in `c` and in r[0 .. c.branches - 1]
+// (lnL_out, mask_out, top_idx, top_lnL) is a device pointer.  The two branches of an EB-type
+// call, EB (period P) and EBx2P (period 2P), share one geometry launch and one work list.
+// Nothing here waits for the GPU; the small result record lands in the slot's pinned buffers and
+// is read by finish_slot.
+int enqueue(Slot& S, const Call& c, const tri_result* r, cudaStream_t s) {
+    const int64_t N = c.N;
+    const bool eb = c.branches == 2;
     S.scratch.reset();
-    int rc = S.scratch.reserve(scratch_bytes(N, false));
+    int rc = S.scratch.reserve(scratch_bytes(N));
     if (rc) return rc;
     Scratch W;
     W.a = S.scratch.take<double>(N);
-    W.lnl = r.lnL_out ? r.lnL_out : S.scratch.take<double>(N);
+    double* p = S.scratch.take<double>(N);   // EB-type: the period of each draw's branch
+    for (int b = 0; b < c.branches; ++b)
+        W.lnl[b] = r[b].lnL_out ? r[b].lnL_out : S.scratch.take<double>(N);
     W.items = S.scratch.take<int64_t>(N);
     W.cval = S.scratch.take<double>(N);
     W.partials = S.scratch.take<LsePartial>(2 * (size_t)lnl_grid());
     S.launches = 0;
     CU(cudaMemsetAsync(S.d_counters, 0, 8 * sizeof(unsigned long long), s));
     CU(cudaEventRecord(S.ev[0], s));
-    GeomTp G{};
-    G.N = N;
-    G.rp = to_col(a.rp); G.P = to_col(a.P_orb); G.inc = to_col(a.inc); G.ecc = to_col(a.ecc);
-    G.argp = to_col(a.argp); G.mtot = to_col(a.mtot); G.rhost = to_col(a.rhost);
-    G.extra_mask = a.extra_mask;
-    G.a_out = W.a; G.lnl_out = W.lnl; G.mask_out = r.mask_out;
-    G.items = W.items; G.n_items = S.d_counters + 0;
-    int gb = (int)std::min<int64_t>((N + 255) / 256, (int64_t)g.sm_count * 8);
-    geometry_tp_kernel<<<std::max(gb, 1), 256, 0, s>>>(G);
+    int gb = std::max(1, (int)std::min<int64_t>((N + 255) / 256, (int64_t)g.sm_count * 8));
+    if (eb) {
+        GeomEb G{};
+        G.N = N;
+        G.reb = to_col(c.body); G.q = to_col(c.q); G.P = to_col(c.P); G.inc = to_col(c.inc);
+        G.ecc = to_col(c.ecc); G.argp = to_col(c.argp); G.mtot = to_col(c.mtot);
+        G.rhost = to_col(c.rhost);
+        G.extra_mask = c.extra_mask;
+        G.scalar_loop = c.scalar_loop;
+        G.a_out = W.a; G.p_out = p; G.lnl_out = W.lnl[0]; G.lnl_twin_out = W.lnl[1];
+        G.mask_out = r[0].mask_out; G.mask_twin_out = r[1].mask_out;
+        G.items = W.items; G.n_items = S.d_counters + 0;
+        geometry_eb_kernel<<<gb, 256, 0, s>>>(G);
+    } else {
+        GeomTp G{};
+        G.N = N;
+        G.rp = to_col(c.body); G.P = to_col(c.P); G.inc = to_col(c.inc); G.ecc = to_col(c.ecc);
+        G.argp = to_col(c.argp); G.mtot = to_col(c.mtot); G.rhost = to_col(c.rhost);
+        G.extra_mask = c.extra_mask;
+        G.a_out = W.a; G.lnl_out = W.lnl[0]; G.mask_out = r[0].mask_out;
+        G.items = W.items; G.n_items = S.d_counters + 0;
+        geometry_tp_kernel<<<gb, 256, 0, s>>>(G);
+    }
     S.launches += 1;
     CU(cudaGetLastError());
     CU(cudaEventRecord(S.ev[1], s));
 
     // the work-list length stays on the device: no host round trip between the two kernels
-    LnlArgs A{};
-    A.lc = g.lc; A.tab = g.tab; A.eb = 0; A.companion_is_host = a.companion_is_host; A.raw = 0;
-    A.twin_uniform = 0;
-    A.body = to_col(a.rp); A.ebfr = Col{nullptr, 0};
-    A.P = to_col(a.P_orb); A.inc = to_col(a.inc); A.a = Col{W.a, 1}; A.rhost = to_col(a.rhost);
-    A.u1 = to_col(a.u1); A.u2 = to_col(a.u2); A.ecc = to_col(a.ecc); A.argp = to_col(a.argp);
-    A.cfr = to_col(a.cfr);
-    A.items = W.items; A.items_cap = N; A.count = 0; A.count_dev = S.d_counters + 0;
+    LnlArgs A = lnl_args(c, eb ? Col{p, 1} : to_col(c.P), Col{W.a, 1});
+    A.items = W.items; A.items_cap = N; A.count_dev = S.d_counters + 0;
     A.next = S.d_counters + 2;
-    A.out = W.lnl; A.out_twin = nullptr; A.counters = S.d_counters + 4;
-    A.lnprior = to_col(a.lnprior); A.lse_partials = W.partials; A.cval = W.cval;
+    A.out = W.lnl[0]; A.out_twin = W.lnl[1]; A.counters = S.d_counters + 4;
+    A.lnprior = to_col(c.lnprior); A.lse_partials = W.partials; A.cval = W.cval;
     A.hist16 = S.d_hist16;
     rc = launch_lnl(S, A, s);
     if (rc) return rc;
     CU(cudaEventRecord(S.ev[2], s));
-    rc = launch_finalize(S, W, N, 1, &r, s);
+    rc = launch_finalize(S, W, N, c.branches, r, s);
     if (rc) return rc;
-    S.moments = g.moments;
     if (S.moments) {
-        rc = launch_moments(S, W, N, 1, to_col(a.lnprior), s);
+        rc = launch_moments(S, W, N, c.branches, to_col(c.lnprior), s);
         if (rc) return rc;
     }
-    capture_posterior(S);
     if (S.post_K > 0) {
-        rc = launch_posterior(S, W, N, 1, to_col(a.lnprior), s);
+        rc = launch_posterior(S, W, N, c.branches, to_col(c.lnprior), s);
         if (rc) return rc;
     }
-    CU(cudaMemcpyAsync(S.h_topk, S.d_topk, sizeof(TopkState), cudaMemcpyDeviceToHost, s));
-    S.lnl[0] = W.lnl; S.lnl[1] = nullptr;
-    CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, lse_out_bytes(S, 1), cudaMemcpyDeviceToHost,
-                       s));
-    CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
+    CU(cudaMemcpyAsync(S.h_topk, S.d_topk, c.branches * sizeof(TopkState),
                        cudaMemcpyDeviceToHost, s));
-    return TRI_OK;
-}
-
-// EB-type: the EB (period P) and EBx2P (period 2P) branches share one geometry launch and one
-// work list; r[0] / r[1] hold the device-side output pointers of the two branches.
-int enqueue_eb(Slot& S, const tri_eb_args& a, const tri_result r[2], cudaStream_t s) {
-    const int64_t N = a.N;
-    S.scratch.reset();
-    int rc = S.scratch.reserve(scratch_bytes(N, true));
-    if (rc) return rc;
-    Scratch W;
-    W.a = S.scratch.take<double>(N);
-    W.p = S.scratch.take<double>(N);
-    W.lnl = r[0].lnL_out ? r[0].lnL_out : S.scratch.take<double>(N);
-    W.lnl_twin = r[1].lnL_out ? r[1].lnL_out : S.scratch.take<double>(N);
-    W.items = S.scratch.take<int64_t>(N);
-    W.cval = S.scratch.take<double>(N);
-    W.partials = S.scratch.take<LsePartial>(2 * (size_t)lnl_grid());
-    S.launches = 0;
-    CU(cudaMemsetAsync(S.d_counters, 0, 8 * sizeof(unsigned long long), s));
-    CU(cudaEventRecord(S.ev[0], s));
-    GeomEb G{};
-    G.N = N;
-    G.reb = to_col(a.reb); G.q = to_col(a.q); G.P = to_col(a.P_orb); G.inc = to_col(a.inc);
-    G.ecc = to_col(a.ecc); G.argp = to_col(a.argp); G.mtot = to_col(a.mtot);
-    G.rhost = to_col(a.rhost);
-    G.extra_mask = a.extra_mask;
-    G.scalar_loop = a.scalar_loop;
-    G.a_out = W.a; G.p_out = W.p; G.lnl_out = W.lnl; G.lnl_twin_out = W.lnl_twin;
-    G.mask_out = r[0].mask_out; G.mask_twin_out = r[1].mask_out;
-    G.items = W.items; G.n_items = S.d_counters + 0;
-    int gb = (int)std::min<int64_t>((N + 255) / 256, (int64_t)g.sm_count * 8);
-    geometry_eb_kernel<<<std::max(gb, 1), 256, 0, s>>>(G);
-    S.launches += 1;
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(S.ev[1], s));
-
-    LnlArgs A{};
-    A.lc = g.lc; A.tab = g.tab; A.eb = 1; A.companion_is_host = a.companion_is_host; A.raw = 0;
-    A.twin_uniform = 0;
-    A.body = to_col(a.reb); A.ebfr = to_col(a.ebfr);
-    A.P = Col{W.p, 1}; A.inc = to_col(a.inc); A.a = Col{W.a, 1}; A.rhost = to_col(a.rhost);
-    A.u1 = to_col(a.u1); A.u2 = to_col(a.u2); A.ecc = to_col(a.ecc); A.argp = to_col(a.argp);
-    A.cfr = to_col(a.cfr);
-    A.items = W.items; A.items_cap = N; A.count = 0; A.count_dev = S.d_counters + 0;
-    A.next = S.d_counters + 2;
-    A.out = W.lnl; A.out_twin = W.lnl_twin; A.counters = S.d_counters + 4;
-    A.scalar_rule = a.scalar_loop ? 1 : 0;
-    A.lnprior = to_col(a.lnprior); A.lse_partials = W.partials; A.cval = W.cval;
-    A.hist16 = S.d_hist16;
-    rc = launch_lnl(S, A, s);
-    if (rc) return rc;
-    CU(cudaEventRecord(S.ev[2], s));
-    rc = launch_finalize(S, W, N, 2, r, s);
-    if (rc) return rc;
-    S.moments = g.moments;
-    if (S.moments) {
-        rc = launch_moments(S, W, N, 2, to_col(a.lnprior), s);
-        if (rc) return rc;
-    }
-    capture_posterior(S);
-    if (S.post_K > 0) {
-        rc = launch_posterior(S, W, N, 2, to_col(a.lnprior), s);
-        if (rc) return rc;
-    }
-    CU(cudaMemcpyAsync(S.h_topk, S.d_topk, 2 * sizeof(TopkState), cudaMemcpyDeviceToHost, s));
-    S.lnl[0] = W.lnl; S.lnl[1] = W.lnl_twin;
+    S.lnl[0] = W.lnl[0]; S.lnl[1] = W.lnl[1];
     CU(cudaEventRecord(S.ev[3], s));
-    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, lse_out_bytes(S, 2), cudaMemcpyDeviceToHost,
-                       s));
+    CU(cudaMemcpyAsync(S.h_lse_out, S.d_lse_out, lse_out_bytes(S, c.branches),
+                       cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(S.h_counters, S.d_counters, 8 * sizeof(unsigned long long),
                        cudaMemcpyDeviceToHost, s));
     return TRI_OK;
@@ -658,39 +651,39 @@ int no_slot() {
     return fail(TRI_ESTATE, "TRI_MAX_INFLIGHT evaluations are already in flight: tri_wait one");
 }
 
-int check_cols(int64_t N, std::initializer_list<const tri_col*> req) {
-    if (N < 0) return fail(TRI_EINVAL, "N must be >= 0");
-    for (const tri_col* c : req) {
-        if (c->ptr == nullptr) return fail(TRI_EINVAL, "a required column is NULL");
-        if (c->stride != 0 && c->stride != 1)
+// The checks of every submission (before anything is queued), then a free slot that holds the
+// call's switches: tri_set_moments and tri_set_posterior as they are now.
+int open_slot(const Call* c, const tri_result* want, const int64_t* ticket, Slot** out) {
+    int rc = need_ready(true);
+    if (rc) return rc;
+    if (!c || !want || !ticket) return fail(TRI_EINVAL, "NULL argument");
+    if (c->N < 0) return fail(TRI_EINVAL, "N must be >= 0");
+    for (const CallCol& k : kCallCols) {
+        const tri_col& x = c->*k.col;
+        if (x.ptr == nullptr) {
+            if (k.need && c->branches >= k.need)
+                return fail(TRI_EINVAL, "a required column is NULL");
+        } else if (x.stride != 0 && x.stride != 1) {
             return fail(TRI_EINVAL, "column stride must be 0 or 1");
+        }
     }
+    Slot* S = free_slot();
+    if (!S) return no_slot();
+    CU(cudaSetDevice(g.device));
+    S->moments = g.moments;
+    S->post_K = g.post_K;
+    S->post_seed = g.post_seed;
+    S->post_stream = g.post_stream;
+    *out = S;
     return TRI_OK;
 }
 
-int check_tp(const tri_tp_args* a, const void* out) {
-    if (!a || !out) return fail(TRI_EINVAL, "NULL argument");
-    return check_cols(a->N, {&a->rp, &a->P_orb, &a->inc, &a->ecc, &a->argp, &a->mtot, &a->rhost,
-                             &a->u1, &a->u2, &a->cfr});
-}
-
-int check_eb(const tri_eb_args* a, const void* out) {
-    if (!a || !out) return fail(TRI_EINVAL, "NULL argument");
-    return check_cols(a->N, {&a->reb, &a->ebfr, &a->q, &a->P_orb, &a->inc, &a->ecc, &a->argp,
-                             &a->mtot, &a->rhost, &a->u1, &a->u2, &a->cfr});
-}
-
 // mark the slot in flight and hand out its ticket
-void commit(Slot& S, int branches, int64_t N, bool host, const tri_result* want,
-            int64_t* ticket) {
-    if (N == 0) {   // (no kernels: enqueue_* did not run)
-        S.moments = g.moments;
-        capture_posterior(S);
-    }
-    S.branches = branches;
-    S.N = N;
+void commit(Slot& S, const Call& c, bool host, const tri_result* want, int64_t* ticket) {
+    S.branches = c.branches;
+    S.N = c.N;
     S.host = host;
-    for (int b = 0; b < branches; ++b) S.want[b] = want[b];
+    for (int b = 0; b < c.branches; ++b) S.want[b] = want[b];
     S.ticket = g.next_ticket++;
     *ticket = S.ticket;
 }
@@ -1081,46 +1074,32 @@ int tri_set_lightcurve_cadence(const double* time, const double* flux, const dou
 }
 
 // ---- submit / wait --------------------------------------------------------------------------
-int tri_submit_tp_dev(const tri_tp_args* a, const tri_result* want, void* stream,
-                      int64_t* ticket) {
-    int rc = need_ready(true);
+// Device-pointer submission: the kernels go on the caller's stream.
+static int submit_dev(const Call* c, const tri_result* want, void* stream, int64_t* ticket) {
+    Slot* S = nullptr;
+    int rc = open_slot(c, want, ticket, &S);
     if (rc) return rc;
-    if (!ticket) return fail(TRI_EINVAL, "NULL argument");
-    rc = check_tp(a, want);
-    if (rc) return rc;
-    Slot* S = free_slot();
-    if (!S) return no_slot();
-    CU(cudaSetDevice(g.device));
     cudaStream_t s = (cudaStream_t)stream;   // NULL is the CUDA default stream, as everywhere
-    if (a->N > 0) {
-        rc = grow_slots(*S, scratch_bytes(a->N, true), 0, 0);
-        if (!rc) rc = enqueue_tp(*S, *a, *want, s);
+    if (c->N > 0) {
+        rc = grow_slots(*S, scratch_bytes(c->N), 0, 0);
+        if (!rc) rc = enqueue(*S, *c, want, s);
         if (rc) { cudaStreamSynchronize(s); return abandon(*S, rc); }
     }
     CU(cudaEventRecord(S->done, s));
-    commit(*S, 1, a->N, false, want, ticket);
+    commit(*S, *c, false, want, ticket);
     return TRI_OK;
+}
+
+int tri_submit_tp_dev(const tri_tp_args* a, const tri_result* want, void* stream,
+                      int64_t* ticket) {
+    Call c;
+    return submit_dev(as_call(a, c), want, stream, ticket);
 }
 
 int tri_submit_eb_dev(const tri_eb_args* a, const tri_result want[2], void* stream,
                       int64_t* ticket) {
-    int rc = need_ready(true);
-    if (rc) return rc;
-    if (!ticket) return fail(TRI_EINVAL, "NULL argument");
-    rc = check_eb(a, want);
-    if (rc) return rc;
-    Slot* S = free_slot();
-    if (!S) return no_slot();
-    CU(cudaSetDevice(g.device));
-    cudaStream_t s = (cudaStream_t)stream;   // NULL is the CUDA default stream, as everywhere
-    if (a->N > 0) {
-        rc = grow_slots(*S, scratch_bytes(a->N, true), 0, 0);
-        if (!rc) rc = enqueue_eb(*S, *a, want, s);
-        if (rc) { cudaStreamSynchronize(s); return abandon(*S, rc); }
-    }
-    CU(cudaEventRecord(S->done, s));
-    commit(*S, 2, a->N, false, want, ticket);
-    return TRI_OK;
+    Call c;
+    return submit_dev(as_call(a, c), want, stream, ticket);
 }
 
 // device-side landing buffers of one branch's outputs, and the copies back to the caller's
@@ -1168,131 +1147,74 @@ static int reserve_top(Slot& S, int64_t cap) {
     return TRI_OK;
 }
 
-static int submit_tp_body(Slot* S, const tri_tp_args* a, const tri_result* want,
-                          int64_t* ticket) {
+// Host-buffer submission into slot S: the columns go to the slot's staging arena on the copy
+// stream, the kernels follow on the compute stream.
+static int submit_host_body(Slot& S, const Call& h, const tri_result* want, int64_t* ticket) {
     int rc;
-    const int64_t N = a->N;
+    const int64_t N = h.N;
     if (N > 0) {
         cudaStream_t cs = g.copy_stream;
+        int64_t top_cap = 0;
+        for (int b = 0; b < h.branches; ++b) top_cap = std::max(top_cap, want[b].top_cap);
         // pageable caller columns go through the pinned arena (sized for the EB-type column
         // set too: a slot serves both kinds in turn)
-        rc = grow_slots(*S, scratch_bytes(N, true),
-                        (size_t)N * 8 * 16 + (size_t)N * 3 + 8192
-                            + (size_t)std::max<int64_t>(want->top_cap, 0) * 32,
-                        is_pinned(a->inc.ptr)
+        rc = grow_slots(S, scratch_bytes(N),
+                        (size_t)N * 8 * 16 + (size_t)N * 3 + 8192 + (size_t)top_cap * 32,
+                        is_pinned(h.inc.ptr)
                             ? 0 : std::min(kPinnedLimit, (size_t)N * 8 * 14 + (size_t)N + 8192));
         if (rc) return rc;
-        S->staging.reset();
-        S->pinned.reset();
-        tri_tp_args d = *a;
-        Col c;
-#define STAGE(field)                                   \
-    rc = stage(*S, a->field, N, c, cs);                \
-    if (rc) return rc;                                 \
-    d.field = tri_col{c.p, c.stride};
-        STAGE(rp) STAGE(P_orb) STAGE(inc) STAGE(ecc) STAGE(argp) STAGE(mtot) STAGE(rhost)
-        STAGE(u1) STAGE(u2) STAGE(cfr) STAGE(lnprior)
-        if (a->extra_mask) {
-            uint8_t* m = S->staging.take<uint8_t>(N);
-            CU(cudaMemcpyAsync(m, via_pinned(*S, a->extra_mask, (size_t)N), (size_t)N,
+        S.staging.reset();
+        S.pinned.reset();
+        Call d = h;
+        rc = stage_call(S, d, cs);
+        if (rc) return rc;
+        if (h.extra_mask) {
+            uint8_t* m = S.staging.take<uint8_t>(N);
+            CU(cudaMemcpyAsync(m, via_pinned(S, h.extra_mask, (size_t)N), (size_t)N,
                                cudaMemcpyHostToDevice, cs));
             d.extra_mask = m;
         }
-        rc = reserve_top(*S, want->top_cap);
-        if (rc) return rc;
-        tri_result r;
-        stage_outputs(*S, N, *want, r);
-        if (r.top_cap > 0) {
-            CU(cudaMemsetAsync(r.top_idx, 0, (size_t)r.top_cap * 8, cs));
-            CU(cudaMemsetAsync(r.top_lnL, 0, (size_t)r.top_cap * 8, cs));
-        }
-        // the kernels start when the columns have landed; the next call's copies overlap them
-        CU(cudaEventRecord(S->copied, cs));
-        CU(cudaStreamWaitEvent(g.stream, S->copied, 0));
-        rc = enqueue_tp(*S, d, r, g.stream);
-        if (rc) return rc;
-        rc = queue_outputs(*S, 0, *want, r, g.stream);
-        if (rc) return rc;
-    }
-    CU(cudaEventRecord(S->done, g.stream));
-    commit(*S, 1, N, true, want, ticket);
-    return TRI_OK;
-}
-
-int tri_submit_tp(const tri_tp_args* a, const tri_result* want, int64_t* ticket) {
-    int rc = need_ready(true);
-    if (rc) return rc;
-    if (!ticket) return fail(TRI_EINVAL, "NULL argument");
-    rc = check_tp(a, want);
-    if (rc) return rc;
-    Slot* S = free_slot();
-    if (!S) return no_slot();
-    CU(cudaSetDevice(g.device));
-    rc = submit_tp_body(S, a, want, ticket);
-    return rc ? abandon(*S, rc) : TRI_OK;
-}
-
-static int submit_eb_body(Slot* S, const tri_eb_args* a, const tri_result want[2],
-                          int64_t* ticket) {
-    int rc;
-    const int64_t N = a->N;
-    if (N > 0) {
-        cudaStream_t cs = g.copy_stream;
-        rc = grow_slots(*S, scratch_bytes(N, true),
-                        (size_t)N * 8 * 16 + (size_t)N * 3 + 8192
-                            + (size_t)std::max<int64_t>(want[0].top_cap, 0) * 16
-                            + (size_t)std::max<int64_t>(want[1].top_cap, 0) * 16,
-                        is_pinned(a->inc.ptr)
-                            ? 0 : std::min(kPinnedLimit, (size_t)N * 8 * 14 + (size_t)N + 8192));
-        if (rc) return rc;
-        S->staging.reset();
-        S->pinned.reset();
-        tri_eb_args d = *a;
-        Col c;
-        STAGE(reb) STAGE(ebfr) STAGE(q) STAGE(P_orb) STAGE(inc) STAGE(ecc) STAGE(argp)
-        STAGE(mtot) STAGE(rhost) STAGE(u1) STAGE(u2) STAGE(cfr) STAGE(lnprior)
-#undef STAGE
-        if (a->extra_mask) {
-            uint8_t* m = S->staging.take<uint8_t>(N);
-            CU(cudaMemcpyAsync(m, via_pinned(*S, a->extra_mask, (size_t)N), (size_t)N,
-                               cudaMemcpyHostToDevice, cs));
-            d.extra_mask = m;
-        }
-        rc = reserve_top(*S, std::max(want[0].top_cap, want[1].top_cap));
+        rc = reserve_top(S, top_cap);
         if (rc) return rc;
         tri_result r[2];
-        for (int b = 0; b < 2; ++b) {
-            stage_outputs(*S, N, want[b], r[b]);
+        for (int b = 0; b < h.branches; ++b) {
+            stage_outputs(S, N, want[b], r[b]);
             if (r[b].top_cap > 0) {
                 CU(cudaMemsetAsync(r[b].top_idx, 0, (size_t)r[b].top_cap * 8, cs));
                 CU(cudaMemsetAsync(r[b].top_lnL, 0, (size_t)r[b].top_cap * 8, cs));
             }
         }
-        CU(cudaEventRecord(S->copied, cs));
-        CU(cudaStreamWaitEvent(g.stream, S->copied, 0));
-        rc = enqueue_eb(*S, d, r, g.stream);
+        // the kernels start when the columns have landed; the next call's copies overlap them
+        CU(cudaEventRecord(S.copied, cs));
+        CU(cudaStreamWaitEvent(g.stream, S.copied, 0));
+        rc = enqueue(S, d, r, g.stream);
         if (rc) return rc;
-        for (int b = 0; b < 2; ++b) {
-            rc = queue_outputs(*S, b, want[b], r[b], g.stream);
+        for (int b = 0; b < h.branches; ++b) {
+            rc = queue_outputs(S, b, want[b], r[b], g.stream);
             if (rc) return rc;
         }
     }
-    CU(cudaEventRecord(S->done, g.stream));
-    commit(*S, 2, N, true, want, ticket);
+    CU(cudaEventRecord(S.done, g.stream));
+    commit(S, h, true, want, ticket);
     return TRI_OK;
 }
 
-int tri_submit_eb(const tri_eb_args* a, const tri_result want[2], int64_t* ticket) {
-    int rc = need_ready(true);
+static int submit_host(const Call* h, const tri_result* want, int64_t* ticket) {
+    Slot* S = nullptr;
+    int rc = open_slot(h, want, ticket, &S);
     if (rc) return rc;
-    if (!ticket) return fail(TRI_EINVAL, "NULL argument");
-    rc = check_eb(a, want);
-    if (rc) return rc;
-    Slot* S = free_slot();
-    if (!S) return no_slot();
-    CU(cudaSetDevice(g.device));
-    rc = submit_eb_body(S, a, want, ticket);
+    rc = submit_host_body(*S, *h, want, ticket);
     return rc ? abandon(*S, rc) : TRI_OK;
+}
+
+int tri_submit_tp(const tri_tp_args* a, const tri_result* want, int64_t* ticket) {
+    Call c;
+    return submit_host(as_call(a, c), want, ticket);
+}
+
+int tri_submit_eb(const tri_eb_args* a, const tri_result want[2], int64_t* ticket) {
+    Call c;
+    return submit_host(as_call(a, c), want, ticket);
 }
 
 int tri_wait(int64_t ticket, tri_result* out) {
@@ -1377,28 +1299,24 @@ static int lnl_seam(int eb, int64_t n, const double* body, const double* ebfr, c
     S.staging.reset();
     rc = S.staging.reserve((size_t)n * 8 * 14 + 8192 + (model_out ? (size_t)n * npts * 8 : 0));
     if (rc) return rc;
-    LnlArgs A{};
-    A.lc = g.lc; A.tab = g.tab; A.eb = eb; A.companion_is_host = is_host; A.raw = 1;
+    // (no mass, q or prior: the caller gives the semi-major axis, and there is no evidence)
+    Call c{eb ? 2 : 1, n, {body, 1}, {ebfr, 1}, {}, {P, 1}, {inc, 1}, {ecc, 1}, {argp, 1}, {},
+           {R_s, 1}, {u1, 1}, {u2, 1}, {cfr, 1}, {}, nullptr, is_host, scalar_rule};
+    tri_col d_a{a, 1};
+    rc = stage_call(S, c, s);
+    if (!rc) rc = stage(S, d_a, n, s);
+    if (rc) return rc;
+    LnlArgs A = lnl_args(c, to_col(c.P), to_col(d_a));
+    A.raw = 1;
     A.twin_uniform = twin ? 1 : 0;
-    Col c;
-#define UP(dst, src)                                           \
-    rc = stage(S, tri_col{src, 1}, n, c, s);                   \
-    if (rc) return rc;                                         \
-    A.dst = c;
-    UP(body, body)
-    if (eb) { UP(ebfr, ebfr) }
-    UP(P, P) UP(inc, inc) UP(a, a) UP(rhost, R_s) UP(u1, u1) UP(u2, u2) UP(ecc, ecc)
-    UP(argp, argp) UP(cfr, cfr)
-#undef UP
     double* d_out = S.staging.take<double>(n);
     double* d_model = model_out ? S.staging.take<double>((size_t)n * npts) : nullptr;
     double* d_sec = secdepth_out ? S.staging.take<double>(n) : nullptr;
     S.launches = 0;
     CU(cudaMemsetAsync(S.d_counters, 0, 8 * sizeof(unsigned long long), s));
-    A.items = nullptr; A.count = n; A.count_dev = nullptr; A.next = S.d_counters + 2;
-    A.out = d_out; A.out_twin = nullptr; A.counters = S.d_counters + 4;
+    A.count = n; A.next = S.d_counters + 2;
+    A.out = d_out; A.counters = S.d_counters + 4;
     A.model_out = d_model; A.secdepth_out = d_sec; A.perm = g.d_perm;
-    A.scalar_rule = scalar_rule;
     CU(cudaEventRecord(S.ev[0], s));
     CU(cudaEventRecord(S.ev[1], s));
     rc = launch_lnl(S, A, s);

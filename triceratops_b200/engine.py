@@ -63,6 +63,11 @@ def cadence_columns(exptime, nsamples, npts):
     return np.ascontiguousarray(e), np.ascontiguousarray(n)
 
 
+def _columns(args_type, values):
+    """The columns of tri_tp_args / tri_eb_args (their tri_col fields), picked from `values`."""
+    return {name: values[name] for name, t in args_type._fields_ if t is tri_col}
+
+
 class BranchResult:
     """One scenario branch: lnZ pieces + optional per-draw arrays."""
     __slots__ = ("lnZ", "m", "s", "n_finite", "n_posinf", "n_pass", "n_stamps", "n_interior",
@@ -196,7 +201,6 @@ class Engine:
         self.device = int(device)
         _cabi.check(self.lib.tri_init(self.device))
         self._lc_key = None
-        self._keep = []
         self._inflight = []      # Pendings not waited for yet, oldest first
         self._side_streams = None
         self._side_turn = 0
@@ -263,8 +267,10 @@ class Engine:
         self._lc_key = key
 
     # ------------------------------------------------------------------ helpers
-    def _col(self, x, N):
-        """numpy array of N values (stride 1) or scalar (stride 0) -> tri_col (keeps a ref)."""
+    @staticmethod
+    def _col(x, N, keep):
+        """numpy array of N values (stride 1) or scalar (stride 0) -> tri_col (`keep` holds a
+        reference)."""
         if x is None:
             return tri_col(None, 0)
         a = np.asarray(x, dtype=np.float64)
@@ -276,10 +282,11 @@ class Engine:
             if a.shape != (N,):
                 raise ValueError("column has shape %s, expected (%d,)" % (a.shape, N))
             stride = 1
-        self._keep.append(a)
+        keep.append(a)
         return tri_col(a.ctypes.data, stride)
 
-    def _mask(self, m, N):
+    @staticmethod
+    def _mask(m, N, keep):
         if m is None:
             return None
         a = np.asarray(m)
@@ -289,7 +296,7 @@ class Engine:
             a = np.ascontiguousarray(a.astype(np.uint8))
         if a.shape != (N,):
             raise ValueError("extra_mask has shape %s, expected (%d,)" % (a.shape, N))
-        self._keep.append(a)
+        keep.append(a)
         return a.ctypes.data
 
     def _result(self, N, want_lnL, want_mask, n_best=0):
@@ -313,13 +320,16 @@ class Engine:
         return out
 
     # ------------------------------------------------------------------ L2 seam
+    # per argument layout: branch count, host-buffer and device-pointer entry points
+    _KINDS = {tri_tp_args: (1, "tri_submit_tp", "tri_submit_tp_dev"),
+              tri_eb_args: (2, "tri_submit_eb", "tri_submit_eb_dev")}
+
     def eval_tp(self, *args, **kw):
         return self.submit_tp(*args, **kw).result()
 
     def eval_eb(self, *args, **kw):
         return self.submit_eb(*args, **kw).result()
 
-    @_locked
     def submit_tp(self, N, rp, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr, lnprior=None,
                   extra_mask=None, companion_is_host=False, want_lnL=True, want_mask=False,
                   n_best=0, lightcurve=None, post_stream=0):
@@ -328,70 +338,66 @@ class Engine:
         `lightcurve` = (time, flux, sigma, exptime, nsamples) makes that the current light
         curve in the same critical section (callers in several threads).  `post_stream`: the
         stream of the posterior samples' U (set_posterior)."""
-        N = int(N)
-        if lightcurve is not None:
-            self.set_lightcurve(*lightcurve)
-        self._make_room()
-        self._keep = []
-        a = tri_tp_args()
-        a.N = N
-        for name, val in (("rp", rp), ("P_orb", P_orb), ("inc", inc), ("ecc", ecc),
-                          ("argp", argp), ("mtot", mtot), ("rhost", rhost), ("u1", u1),
-                          ("u2", u2), ("cfr", cfr), ("lnprior", lnprior)):
-            setattr(a, name, self._col(val, N))
-        a.extra_mask = self._mask(extra_mask, N)
-        a.companion_is_host = int(bool(companion_is_host))
-        r, lnL, mask, top = self._result(N, want_lnL, want_mask, n_best)
-        rr = (tri_result * 1)(r)
-        ticket = ctypes.c_int64()
-        self._arm_posterior(post_stream)
-        _cabi.check(self.lib.tri_submit_tp(ctypes.byref(a), rr, ctypes.byref(ticket)))
-        keep, self._keep = self._keep + [a, lnL, mask, top], []
+        return self._submit_host(tri_tp_args, N, _columns(tri_tp_args, locals()), extra_mask,
+                                 companion_is_host, want_lnL, want_mask, n_best, lightcurve,
+                                 post_stream=post_stream)
 
-        def build(rr):
-            return [BranchResult(rr[0], N, lnL, mask.astype(bool) if mask is not None else None,
-                                 top, 0)]
-        p = Pending(self, ticket.value, rr, 1, keep, build, n_best)
-        self._inflight.append(p)
-        return p
-
-    @_locked
     def submit_eb(self, N, reb, ebfr, q, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr,
                   lnprior=None, extra_mask=None, companion_is_host=False, want_lnL=True,
                   want_mask=False, n_best=0, lightcurve=None, scalar_loop=False, post_stream=0):
         """EB-type counterpart of submit_tp.  scalar_loop=True evaluates with the semantics of
         the reference's parallel=False loops (see tri_eb_args.scalar_loop)."""
+        return self._submit_host(tri_eb_args, N, _columns(tri_eb_args, locals()), extra_mask,
+                                 companion_is_host, want_lnL, want_mask, n_best, lightcurve,
+                                 scalar_loop, post_stream)
+
+    @_locked
+    def _submit_host(self, args_type, N, cols, extra_mask, companion_is_host, want_lnL,
+                     want_mask, n_best, lightcurve, scalar_loop=False, post_stream=0):
         N = int(N)
+        keep = []
+        a = self._args(args_type, N, cols, lambda x: self._col(x, N, keep),
+                       self._mask(extra_mask, N, keep), companion_is_host, scalar_loop)
+        nb, fn, _ = self._KINDS[args_type]
+        rr = (tri_result * nb)()
+        outs = []
+        for b in range(nb):
+            rr[b], lnL, mask, top = self._result(N, want_lnL, want_mask, n_best)
+            outs.append((lnL, mask, top))
+        keep.append(outs)
+
+        def build(rr):
+            return [BranchResult(rr[b], N, lnL, mask.astype(bool) if mask is not None else None,
+                                 top, b)
+                    for b, (lnL, mask, top) in enumerate(outs)]
+        return self._submit(getattr(self.lib, fn), a, rr, None, keep, build, n_best, lightcurve,
+                            post_stream)
+
+    @staticmethod
+    def _args(args_type, N, cols, col, extra_mask, companion_is_host, scalar_loop):
+        """tri_tp_args / tri_eb_args of a submission; `col(value)` makes each tri_col."""
+        a = args_type()
+        a.N = N
+        for name, val in cols.items():
+            setattr(a, name, col(val))
+        a.extra_mask = extra_mask
+        a.companion_is_host = int(bool(companion_is_host))
+        if args_type is tri_eb_args:
+            a.scalar_loop = int(bool(scalar_loop))
+        return a
+
+    def _submit(self, fn, a, rr, stream, keep, build, n_best, lightcurve, post_stream):
+        """The steps every submission shares (lock held): make `lightcurve` current, wait for
+        room in the library, hand over the posterior stream, call tri_submit_* (`fn`; `stream`
+        None for the host-buffer calls) and register the Pending, which keeps `keep` alive."""
         if lightcurve is not None:
             self.set_lightcurve(*lightcurve)
         self._make_room()
-        self._keep = []
-        a = tri_eb_args()
-        a.N = N
-        for name, val in (("reb", reb), ("ebfr", ebfr), ("q", q), ("P_orb", P_orb), ("inc", inc),
-                          ("ecc", ecc), ("argp", argp), ("mtot", mtot), ("rhost", rhost),
-                          ("u1", u1), ("u2", u2), ("cfr", cfr), ("lnprior", lnprior)):
-            setattr(a, name, self._col(val, N))
-        a.extra_mask = self._mask(extra_mask, N)
-        a.companion_is_host = int(bool(companion_is_host))
-        a.scalar_loop = int(bool(scalar_loop))
-        rr = (tri_result * 2)()
-        outs = []
-        for b in range(2):
-            r, lnL, mask, top = self._result(N, want_lnL, want_mask, n_best)
-            rr[b] = r
-            outs.append((lnL, mask, top))
         ticket = ctypes.c_int64()
         self._arm_posterior(post_stream)
-        _cabi.check(self.lib.tri_submit_eb(ctypes.byref(a), rr, ctypes.byref(ticket)))
-        keep, self._keep = self._keep + [a, outs], []
-
-        def build(rr):
-            return [BranchResult(rr[b], N, outs[b][0],
-                                 outs[b][1].astype(bool) if outs[b][1] is not None else None,
-                                 outs[b][2], b)
-                    for b in range(2)]
-        p = Pending(self, ticket.value, rr, 2, keep, build, n_best)
+        extra = () if stream is None else (ctypes.c_void_p(stream),)
+        _cabi.check(fn(ctypes.byref(a), rr, *extra, ctypes.byref(ticket)))
+        p = Pending(self, ticket.value, rr, len(rr), keep + [a], build, n_best)
         self._inflight.append(p)
         return p
 
@@ -440,26 +446,19 @@ class Engine:
         return idx[order], val[order]
 
     @_locked
-    def _submit_tensors(self, kind, N, cols, extra_mask, companion_is_host, n_best,
+    def _submit_tensors(self, args_type, N, cols, extra_mask, companion_is_host, n_best,
                         lightcurve=None, scalar_loop=False, post_stream=0):
         import torch
         N = int(N)
-        if lightcurve is not None:
-            self.set_lightcurve(*lightcurve)
-        self._make_room()
         keep = []
-        a = tri_tp_args() if kind == "tp" else tri_eb_args()
-        a.N = N
-        for name, val in cols.items():
-            setattr(a, name, self._tensor_col(val, N, keep))
+        mask = None
         if extra_mask is not None:
             m = extra_mask.to(torch.uint8).contiguous()
             keep.append(m)
-            a.extra_mask = m.data_ptr()
-        a.companion_is_host = int(bool(companion_is_host))
-        if kind == "eb":
-            a.scalar_loop = int(bool(scalar_loop))
-        nb = 1 if kind == "tp" else 2
+            mask = m.data_ptr()
+        a = self._args(args_type, N, cols, lambda x: self._tensor_col(x, N, keep), mask,
+                       companion_is_host, scalar_loop)
+        nb, _, fn = self._KINDS[args_type]
         rr = (tri_result * nb)()
         tops = []
         for b in range(nb):
@@ -475,31 +474,24 @@ class Engine:
         side = self._side_streams[self._side_turn]
         self._side_turn ^= 1
         side.wait_stream(cur)
-        stream = side.cuda_stream
-        fn = self.lib.tri_submit_tp_dev if kind == "tp" else self.lib.tri_submit_eb_dev
-        ticket = ctypes.c_int64()
-        self._arm_posterior(post_stream)
-        _cabi.check(fn(ctypes.byref(a), rr, ctypes.c_void_p(stream), ctypes.byref(ticket)))
-        keep.append(a)
 
         def build(rr):
             return [BranchResult(rr[b], N, None, None, self._sorted_top(rr[b], *tops[b]), b)
                     for b in range(nb)]
-        p = Pending(self, ticket.value, rr, nb, keep, build, 0)
-        self._inflight.append(p)
-        return p
+        return self._submit(getattr(self.lib, fn), a, rr, side.cuda_stream, keep, build, 0,
+                            lightcurve, post_stream)
 
     def submit_tp_tensors(self, N, cols, extra_mask=None, companion_is_host=False, n_best=100,
                           lightcurve=None, post_stream=0):
         """tri_submit_tp_dev on torch CUDA tensors (columns: rp, P_orb, inc, ecc, argp, mtot,
         rhost, u1, u2, cfr, lnprior; tensors of N values or scalars), queued on torch's current
         stream behind the kernels that produce them.  Returns a Pending."""
-        return self._submit_tensors("tp", N, cols, extra_mask, companion_is_host, n_best,
+        return self._submit_tensors(tri_tp_args, N, cols, extra_mask, companion_is_host, n_best,
                                     lightcurve, post_stream=post_stream)
 
     def submit_eb_tensors(self, N, cols, extra_mask=None, companion_is_host=False, n_best=100,
                           lightcurve=None, scalar_loop=False, post_stream=0):
-        return self._submit_tensors("eb", N, cols, extra_mask, companion_is_host, n_best,
+        return self._submit_tensors(tri_eb_args, N, cols, extra_mask, companion_is_host, n_best,
                                     lightcurve, scalar_loop, post_stream)
 
     def eval_tp_tensors(self, *args, **kw):
