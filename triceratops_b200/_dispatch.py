@@ -4,9 +4,11 @@ ranks (one process per GPU), the single small collective that merges the per-ran
 (reference marginal_likelihoods.py:152-154).
 
 Sharding follows SURVEY.md section 8e: rank r evaluates the contiguous slice
-[r*N/G, (r+1)*N/G) of every scenario's draws and contributes one 207-double record per scenario
-branch -- (m, s, counts) + its 100 best (lnL, global index) candidates; no per-draw data is
-exchanged.
+[r*N/G, (r+1)*N/G) of every scenario's draws and contributes one record per scenario branch
+(pack_slice): the evidence header, its 100 best (lnL, global index) candidates -- with their
+rows where only this rank holds them (device sampler) -- and with posterior samples their
+indices (and rows); no per-draw data is exchanged.  merge_slices merges the records of the
+ranks, and likewise those of the rounds of fpp_err_target refinement (triceratops._merge_round).
 
   * a single lnZ_* call under a process group: every rank makes the same host draws (same
     seed) and the records are merged with one all-gather per call;
@@ -187,21 +189,23 @@ def _post_kw(eng, post):
 
 
 class Branch:
-    """Globally combined result of one scenario branch: lnZ, its (m, s, s2, n_finite, n_posinf)
-    record (s2 None without moments), the best draws' indices and finite lnL values; with
-    posterior samples, their global draw indices (ascending) and total weight relative to
-    exp(m), else None."""
-    __slots__ = ("lnZ", "idx", "n_pass", "n_evaluated", "lnL_local", "lo", "hi", "N", "m", "s",
-                 "s2", "n_finite", "n_posinf", "vals", "post_idx", "post_total")
+    """One scenario branch merged over its slices of draws (merge_slices): lnZ over all N draws;
+    record = (m, s, s2, n_finite, n_posinf) (s2 None without moments); the finite best-draw
+    candidates, best first: global draw indices `idx`, lnL `vals` and, where their rows travelled
+    with them, `rows` [k, R]; with posterior samples, their global draw indices `post_idx`
+    (ascending), rows `post_rows` and total weight `post_total` relative to exp(record[0]), else
+    None."""
+    __slots__ = ("lnZ", "N", "record", "n_pass", "n_evaluated", "idx", "vals", "rows",
+                 "post_idx", "post_rows", "post_total")
 
 
 def _local_best(res, eng, single_rank):
     """(indices, lnL values, number of draws with finite lnL) of this rank's best draws.
 
-    The CUDA engine selects them on the device (no per-draw read-back).  With fewer than N_BEST
-    finite draws the reference pads its table with zero-weight draws in the order numpy's
-    argsort happens to give the -inf entries; a single rank reproduces that by fetching the
-    array, ranks of a sharded run pad nothing."""
+    The CUDA engine selects them on the device (no per-draw read-back), best first, ties in
+    index order.  With fewer than N_BEST finite draws the reference pads its table with
+    zero-weight draws in the order numpy's argsort happens to give the -inf entries; a single
+    rank reproduces that by fetching the array (single_rank=True)."""
     top_idx = getattr(res, "top_idx", None)
     if top_idx is not None:
         if single_rank and res.n_evaluated < N_BEST and res.N > 0:
@@ -214,9 +218,6 @@ def _local_best(res, eng, single_rank):
         return np.zeros(0, dtype=np.int64), np.zeros(0), 0
     idx = best_indices(res.lnL)
     return idx, res.lnL[idx], int(np.isfinite(res.lnL).sum())
-
-
-H = 7   # header of a branch record: m, s, n_finite, n_posinf, n_pass, n_evaluated, s2
 
 
 def _allgather(mat, d):
@@ -241,105 +242,119 @@ def gather_records(records, N_total):
                                     N_total) for j in range(len(records))]
 
 
-def record_row(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals, post=None):
-    """The 207-double record of a branch over one slice of draws (a rank's, or a round's of
-    refinement): header, then its best finite (lnL, global index) candidates; s2 None -> NaN.
-    With posterior samples, post = (K, T, global indices) appends [T, K indices] (NaN where
-    the posterior is empty)."""
-    rec = np.full(H + 2 * N_BEST + (0 if post is None else 1 + post[0]), np.nan)
-    if post is not None:
-        rec[H + 2 * N_BEST] = post[1]
-        rec[H + 2 * N_BEST + 1:H + 2 * N_BEST + 1 + len(post[2])] = post[2]
-    rec[0:H] = (m, s, n_finite, n_posinf, n_pass, n_eval, np.nan if s2 is None else s2)
-    idx, vals = np.asarray(idx), np.asarray(vals)
+# ---- the record of a branch over one slice of draws, and the merge of slices -------------------
+H = 7   # header: m, s, n_finite, n_posinf, n_pass, n_evaluated, s2
+
+
+def pack_slice(m, s, n_finite, n_posinf, n_pass, n_eval, s2, idx, vals, rows=None, post=None):
+    """A branch over one slice of draws (a rank's, or a round's of refinement) as one float64
+    row: the header (s2 None -> NaN); the N_BEST finite candidates' lnL values, then their
+    GLOBAL draw indices (NaN past them); with `rows` ([candidates, R]) their N_BEST x R rows;
+    with posterior samples, post = (K, T, global indices[, rows]) appends T, K indices and K x R
+    rows (NaN where the posterior is empty).  R = 0 where the rows can be looked up by index
+    after the merge (host sampler); R = len(RESULT_KEYS) where they live only where they were
+    drawn (device sampler) or in an earlier round (refinement)."""
+    R = 0 if rows is None else np.shape(rows)[1]
+    P = H + N_BEST * (2 + R)
+    K = 0 if post is None else post[0]
+    rec = np.full(P + (0 if post is None else 1 + K * (1 + R)), np.nan)
+    rec[:H] = (m, s, n_finite, n_posinf, n_pass, n_eval, np.nan if s2 is None else s2)
+    vals = np.asarray(vals)
     fin = np.isfinite(vals)
-    idx, vals = idx[fin], vals[fin]
-    k = idx.size
-    rec[H:H + k] = vals
-    rec[H + N_BEST:H + N_BEST + k] = idx.astype(np.float64)
+    k = int(fin.sum())
+    rec[H:H + k] = vals[fin]
+    rec[H + N_BEST:H + N_BEST + k] = np.asarray(idx)[fin]
+    if R:
+        rec[H + 2 * N_BEST:H + 2 * N_BEST + k * R] = np.asarray(rows)[fin].ravel()
+    if post is not None:
+        n = len(post[2])
+        rec[P] = post[1]
+        rec[P + 1:P + 1 + n] = post[2]
+        if R:
+            rec[P + 1 + K:P + 1 + K + n * R] = np.asarray(post[3]).ravel()
     return rec
 
 
-def _local_record(res, lo, eng, post=None):
-    """This rank's record of one branch (zero-weight padding is not exchanged)."""
-    local_best, local_vals, n_eval = _local_best(res, eng, False)
-    return record_row(res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval,
-                      getattr(res, "s2", None), np.asarray(local_best) + lo, local_vals,
-                      _local_post(res, lo, post))
-
-
-def _local_post(res, lo, post):
-    """(K, T, global indices) of a local result's posterior samples, None when off."""
-    idx = getattr(res, "post_idx", None)
-    if idx is None or post is None:
-        return None
-    return post[0], res.post_total, np.asarray(idx, dtype=np.int64) + lo
-
-
-def merge_record_posteriors(allrec, post, branch):
-    """(global indices, total weight relative to the merged maximum) of the posterior tails of
-    [slices, ...] records (record_row), merged in slice order; (None, None) without them."""
-    P = H + 2 * N_BEST
-    if post is None or allrec.shape[1] <= P:
-        return None, None
-    parts = []
-    for r in allrec:
-        t = r[P + 1:P + 1 + post[0]]
-        parts.append((r[0], r[P], t[~np.isnan(t)].astype(np.int64)))
-    idx, _, W = _numerics.merge_posteriors(parts, post[0], post[1], post[2], branch)
-    return idx, W
-
-
-def _merge_records(allrec, lo, hi, N, lnL_local=None, post=None, branch=0):
-    """[slices, 207] -> Branch: lnZ from the (m, s) records, best draws from the candidates,
-    posterior samples (post = (K, seed, stream) of the call) from the records' tails.  The
-    slices are ranks, or rounds of refinement (calc_probs)."""
+def merge_slices(allrec, N, R=0, lnZ=None, post=None, branch=0):
+    """Branch of [slices, width] records (pack_slice, slices in draw order) over N draws in all.
+    lnZ and the record merge with combine_lse / combine_moments; one slice keeps the engine's
+    numbers: `lnZ` and its header as they are.  The candidates are the finite ones ordered by
+    (lnL descending, global index ascending), cut to N_BEST, with their rows where R > 0.  With
+    post = (K, seed, stream) of the call and the records' tails, the posterior samples merge with
+    merge_posteriors, each taking its row along.  No padding: the callers fill their tables."""
     br = Branch()
-    br.lo, br.hi, br.lnL_local, br.N = lo, hi, lnL_local, N
-    br.post_idx, br.post_total = merge_record_posteriors(allrec, post, branch)
-    parts = [(r[0], r[1], int(r[2]), int(r[3])) for r in allrec]
-    br.lnZ = _engine_mod.combine_lse(parts, N)
-    br.n_pass = int(sum(r[4] for r in allrec))
-    br.n_evaluated = int(sum(r[5] for r in allrec))
-    br.m, br.s, s2, br.n_finite, br.n_posinf = _engine_mod.combine_moments(
-        [(r[0], r[1], r[6], r[2], r[3]) for r in allrec])
-    br.s2 = None if np.isnan(allrec[:, 6]).any() else s2
+    hd = allrec[:, :H].tolist()
+    br.N, br.n_pass, br.n_evaluated = N, int(sum(r[4] for r in hd)), int(sum(r[5] for r in hd))
+    if len(hd) == 1:
+        br.lnZ = lnZ
+        m, s, n_fin, n_pinf, _, _, s2 = hd[0]
+    else:
+        br.lnZ = _engine_mod.combine_lse([(r[0], r[1], int(r[2]), int(r[3])) for r in hd], N)
+        m, s, s2, n_fin, n_pinf = _engine_mod.combine_moments(
+            [(r[0], r[1], r[6], r[2], r[3]) for r in hd])
+    br.record = (m, s, None if any(np.isnan(r[6]) for r in hd) else s2, int(n_fin), int(n_pinf))
+    P = H + N_BEST * (2 + R)
     vals = allrec[:, H:H + N_BEST].ravel()
     gidx = allrec[:, H + N_BEST:H + 2 * N_BEST].ravel()
     ok = ~np.isnan(gidx)
     vals, gidx = vals[ok], gidx[ok].astype(np.int64)
-    order = np.lexsort((gidx, -vals))
-    idx = gidx[order][:N_BEST]
-    br.vals = vals[order][:N_BEST]
-    want = min(N_BEST, N)
-    if idx.size < want:
-        # fewer finite draws than table rows: the reference fills the table with zero-weight
-        # draws in whatever order its argsort leaves them; here every rank appends the lowest
-        # draw indices not yet listed, so that all ranks build the same table
-        taken = set(idx.tolist())
-        extra = [i for i in range(min(N, want + idx.size)) if i not in taken][:want - idx.size]
-        idx = np.concatenate([idx, np.asarray(extra, dtype=np.int64)])
-    br.idx = idx
+    order = np.lexsort((gidx, -vals))[:N_BEST]
+    br.vals, br.idx, br.rows = vals[order], gidx[order], None
+    if R:
+        br.rows = allrec[:, H + 2 * N_BEST:P].reshape(-1, R)[ok][order]
+    br.post_idx = br.post_rows = br.post_total = None
+    if post is not None and allrec.shape[1] > P:
+        K = post[0]
+        parts, rows = [], []
+        for r in allrec:
+            t = r[P + 1:P + 1 + K]
+            n = int((~np.isnan(t)).sum())
+            parts.append((r[0], r[P], t[:n].astype(np.int64)))
+            rows.append(r[P + 1 + K:P + 1 + K + n * R].reshape(n, R))
+        br.post_idx, _, br.post_total = _numerics.merge_posteriors(parts, K, *post[1:], branch)
+        if R:   # (the slices' samples are disjoint and ascending)
+            pos = np.searchsorted(np.concatenate([p[2] for p in parts]), br.post_idx)
+            br.post_rows = np.concatenate(rows)[pos]
     return br
 
 
-def _gather_branch(res, lo, hi, N, eng=None, post=None, branch=0):
-    """Merge per-rank results of one branch right away (a single lnZ_* call)."""
+def gather_slices(rec, group=None, key=None):
+    """[ranks, width] records of one branch: this rank's alone without a process group, the
+    rows of `key` after the CallGroup's exchange, else those of an all-gather of its own."""
     d = _dist()
     if d is None:
-        br = Branch()
-        br.lo, br.hi, br.lnL_local, br.N = lo, hi, res.lnL, N
-        br.idx, vals, br.n_evaluated = _local_best(res, eng, True)
-        br.vals = np.asarray(vals)[np.isfinite(vals)]
-        br.lnZ, br.n_pass = res.lnZ, res.n_pass
-        br.m, br.s, br.n_finite, br.n_posinf = res.m, res.s, res.n_finite, res.n_posinf
-        br.s2 = getattr(res, "s2", None)
-        lp = _local_post(res, lo, post)
-        br.post_idx, br.post_total = (None, None) if lp is None else (lp[2], lp[1])
+        return rec[None, :]
+    if group is not None:
+        return group.rows(key)
+    return _allgather(rec[None, :], d)[:, 0, :]
+
+
+def _host_record(res, lo, eng, post):
+    """This rank's record of one branch of the host sampler (R = 0: _result looks the rows up by
+    index); post = (K, seed, stream) of the call or None."""
+    idx, vals, n_eval = _local_best(res, eng, False)
+    tail = None
+    if post is not None and getattr(res, "post_idx", None) is not None:
+        tail = (post[0], res.post_total, np.asarray(res.post_idx, dtype=np.int64) + lo)
+    return pack_slice(res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval,
+                      getattr(res, "s2", None), np.asarray(idx) + lo, vals, post=tail)
+
+
+def _host_branch(allrec, res, N, eng, post, branch):
+    """Merged Branch of the host sampler with idx holding the table's min(N_BEST, N) draws.  The
+    rows past the finite candidates carry zero weight: on one rank they come in the order of
+    the reference's argsort over the whole lnL array; across ranks every rank appends the lowest
+    draw indices not yet listed, so that all ranks build the same table."""
+    br = merge_slices(allrec, N, lnZ=res.lnZ, post=post, branch=branch)
+    if len(allrec) == 1:
+        br.idx = _local_best(res, eng, True)[0]
         return br
-    rec = _local_record(res, lo, eng, post)
-    return _merge_records(_allgather(rec[None, :], d)[:, 0, :], lo, hi, N, res.lnL, post,
-                          branch)
+    idx, want = br.idx, min(N_BEST, N)
+    if idx.size < want:
+        taken = set(idx.tolist())
+        extra = [i for i in range(min(N, want + idx.size)) if i not in taken][:want - idx.size]
+        br.idx = np.concatenate([idx, np.asarray(extra, dtype=np.int64)])
+    return br
 
 
 # ---- one exchange per calc_probs ----------------------------------------------------------------
@@ -418,7 +433,7 @@ class CallGroup:
     def scatter_submit(self, eng, kind, N, cols, extra_mask, is_host, scalar_loop=False,
                        post=None):
         """Rank 0: announce one engine call, scatter its per-draw columns, evaluate the own
-        slice.  Returns (pending, lo, hi, seq)."""
+        slice.  Returns (pending, lo, seq)."""
         import torch
         lc = current_lightcurve()
         arrays = [k for k, v in cols.items()
@@ -461,7 +476,7 @@ class CallGroup:
             self.d.scatter(mine, scatter_list=list(dev.unbind(0)), src=0)
             self.scatters += 1
             pending = self._evaluate(eng, hdr, mine, lc)
-        return pending, bounds[0], bounds[1], seq
+        return pending, bounds[0], seq
 
     def finish_root(self, error=False):
         """Rank 0, after its last engine call: release the followers."""
@@ -490,7 +505,7 @@ class CallGroup:
             res = pending.result()
             lo = hdr["bounds"][self.rank]
             for b, r in enumerate(res if isinstance(res, tuple) else (res,)):
-                self.add(_local_record(r, lo, eng, hdr["post"]), ("s", hdr["seq"], b))
+                self.add(_host_record(r, lo, eng, hdr["post"]), ("s", hdr["seq"], b))
         self.exchange()
         return self._bcast()
 
@@ -563,15 +578,16 @@ def _submit(eng, name, *args, post=None, **kw):
 
 class PendingBranches:
     """A scenario evaluation in flight on this rank.  `prepare()` waits for the local result and
-    (inside a CallGroup) registers this rank's records; `finish()` returns the globally merged
-    Branch (TP-type) or the (EB, EBx2P) pair -- right away with its own collective for a single
-    lnZ_* call, after the group's one exchange inside calc_probs.  Both are idempotent."""
+    packs this rank's records (inside a CallGroup, registered for its exchange); `finish()`
+    returns the globally merged Branch (TP-type) or the (EB, EBx2P) pair -- right away with its
+    own collective for a single lnZ_* call, after the group's one exchange inside calc_probs.
+    Both are idempotent."""
 
-    def __init__(self, pending, lo, hi, N, eng, seq=None, post=None):
-        self._pending, self._lo, self._hi, self._N, self._eng = pending, lo, hi, N, eng
+    def __init__(self, pending, lo, N, eng, seq=None, post=None):
+        self._pending, self._lo, self._N, self._eng = pending, lo, N, eng
         self._post = post
         self._seq, self._group = seq, _group
-        self._res = self._keys = self._out = None
+        self._res = self._out = None
         self._lock = threading.Lock()
 
     def prepare(self):
@@ -581,25 +597,20 @@ class PendingBranches:
                 self._res = res if isinstance(res, tuple) else (res,)
                 self._tuple = isinstance(res, tuple)
                 self._pending = None
+                self._recs = [_host_record(r, self._lo, self._eng, self._post)
+                              for r in self._res]
                 g = self._group
-                if g is not None:
-                    self._keys = [g.add(_local_record(r, self._lo, self._eng, self._post),
-                                        None if self._seq is None else ("s", self._seq, b))
-                                  for b, r in enumerate(self._res)]
+                self._keys = [None if g is None else
+                              g.add(rec, None if self._seq is None else ("s", self._seq, b))
+                              for b, rec in enumerate(self._recs)]
 
     def finish(self):
         self.prepare()
         with self._lock:
             if self._out is None:
-                g = self._group
-                if g is None:
-                    out = [_gather_branch(r, self._lo, self._hi, self._N, self._eng,
-                                          self._post, b)
-                           for b, r in enumerate(self._res)]
-                else:
-                    out = [_merge_records(g.rows(k), self._lo, self._hi, self._N, r.lnL,
-                                          self._post, b)
-                           for b, (k, r) in enumerate(zip(self._keys, self._res))]
+                out = [_host_branch(gather_slices(rec, self._group, key), r, self._N, self._eng,
+                                    self._post, b)
+                       for b, (rec, key, r) in enumerate(zip(self._recs, self._keys, self._res))]
                 self._out = tuple(out) if self._tuple else out[0]
         return self._out
 
@@ -610,9 +621,9 @@ def _submit_sharded(kind, N, cols, extra_mask, companion_is_host, scalar_loop=Fa
     post = _next_post()
     if g is not None and g.scatter:
         # calc_probs under a process group, numpy draws: this is rank 0 (the others follow)
-        pending, lo, hi, seq = g.scatter_submit(eng, kind, N, cols, extra_mask,
-                                                companion_is_host, scalar_loop, post)
-        return PendingBranches(pending, lo, hi, N, eng, seq, post)
+        pending, lo, seq = g.scatter_submit(eng, kind, N, cols, extra_mask, companion_is_host,
+                                            scalar_loop, post)
+        return PendingBranches(pending, lo, N, eng, seq, post)
     lo, hi = shard_bounds(N)
     sl = {k: _slice(v, lo, hi) for k, v in cols.items()}
     lnprior = sl.pop("lnprior")
@@ -621,7 +632,7 @@ def _submit_sharded(kind, N, cols, extra_mask, companion_is_host, scalar_loop=Fa
                 extra_mask=_mask_slice(extra_mask, lo, hi),
                 companion_is_host=companion_is_host, want_lnL=False, n_best=N_BEST, post=post,
                 **kw)
-    return PendingBranches(p, lo, hi, N, eng, post=post)
+    return PendingBranches(p, lo, N, eng, post=post)
 
 
 def submit_tp(N, rp, P_orb, inc, ecc, argp, mtot, rhost, u1, u2, cfr, lnprior=None,
@@ -763,118 +774,3 @@ def gil_switch_interval():
         return max(1e-5, float(os.environ.get("TRI_B200_SWITCH_INTERVAL", "0.0002")))
     except ValueError:
         return 0.0002
-
-
-# ---- device-sampler mode: every rank owns its own draws --------------------------------------
-class LocalBranch:
-    """This rank's share of a branch: evidence record and its best LOCAL draws."""
-    __slots__ = ("res", "idx", "vals", "N")
-
-
-def gather_local(res, N, eng=None):
-    lb = LocalBranch()
-    lb.res, lb.N = res, N
-    idx, vals, _ = _local_best(res, eng, False)
-    fin = np.isfinite(vals)
-    lb.idx, lb.vals = np.asarray(idx)[fin], np.asarray(vals)[fin]
-    return lb
-
-
-class TableExchange:
-    """Per-rank evidence record + best-draw ROWS of one branch (device-sampler mode: the draws
-    themselves live on the rank that made them), merged across ranks by `result()` -- with the
-    CallGroup's one exchange inside calc_probs, with its own all-gather otherwise."""
-
-    def __init__(self, lb, table, keys, post=None):
-        """post: ((K, seed, stream) of the call, branch, this rank's posterior table -- the
-        keys and `draw`, global draw indices) or None without posterior samples."""
-        self.lb, self.keys = lb, keys
-        self.post = post
-        res = lb.res
-        self.n_eval = int(res.n_evaluated) if res.n_evaluated is not None else int(len(lb.idx))
-        self.rows = np.stack([np.asarray(table[k], dtype=np.float64) for k in keys], axis=1) \
-            if len(lb.idx) else np.zeros((0, len(keys)))
-        self.group, self.key = _group if _dist() is not None else None, None
-        self.s2 = getattr(res, "s2", None)
-        if _dist() is not None:
-            W = H + N_BEST * (1 + len(keys))
-            if post is not None:   # tail: T, K draw indices, K rows (NaN where empty)
-                W += 1 + post[0][0] * (1 + len(keys))
-            rec = np.full(W, np.nan)
-            if post is not None:
-                P, pt = H + N_BEST * (1 + len(keys)), post[2]
-                n = len(pt["draw"])
-                rec[P] = res.post_total
-                rec[P + 1:P + 1 + n] = pt["draw"]
-                rec[P + 1 + post[0][0]:P + 1 + post[0][0] + n * len(keys)] = np.stack(
-                    [np.asarray(pt[k], dtype=np.float64) for k in keys], axis=1).ravel()
-            rec[0:H] = (res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, self.n_eval,
-                        np.nan if self.s2 is None else self.s2)
-            k = len(lb.vals)
-            rec[H:H + k] = lb.vals
-            rec[H + N_BEST:H + N_BEST + k * len(keys)] = self.rows.ravel()
-            self.rec = rec
-            if self.group is not None:
-                self.key = self.group.add(rec)
-
-    def result(self):
-        """(lnZ, n_pass, n_evaluated, merged table padded to N_BEST rows).  Also sets
-        `record` = (m, s, s2, n_finite, n_posinf) of the whole branch (s2 None without
-        moments) and, on one rank, `top` = (lnL, draw index) of the table's finite rows."""
-        lb, keys, res = self.lb, self.keys, self.lb.res
-        vals, rows, n_eval = lb.vals, self.rows, self.n_eval
-        d = _dist()
-        self.top = None
-        self.posterior = self.post_total = None
-        if d is None and self.post is not None:
-            self.posterior, self.post_total = self.post[2], res.post_total
-        if d is None:
-            lnZ, n_pass = res.lnZ, int(res.n_pass)
-            self.record = (res.m, res.s, self.s2, res.n_finite, res.n_posinf)
-            order = np.argsort(-vals, kind="stable")[:N_BEST]
-            self.top = (vals[order], np.asarray(lb.idx)[order])
-        else:
-            allrec = (self.group.rows(self.key) if self.group is not None
-                      else _allgather(self.rec[None, :], d)[:, 0, :])
-            lnZ = _engine_mod.combine_lse([(r[0], r[1], int(r[2]), int(r[3])) for r in allrec],
-                                          lb.N)
-            n_pass = int(sum(r[4] for r in allrec))
-            n_eval = int(sum(r[5] for r in allrec))
-            m, s, s2, n_fin, n_pinf = _engine_mod.combine_moments(
-                [(r[0], r[1], r[6], r[2], r[3]) for r in allrec])
-            self.record = (m, s, None if np.isnan(allrec[:, 6]).any() else s2, n_fin, n_pinf)
-            if self.post is not None:
-                self._merge_posterior(allrec)
-            vs, rs = [], []
-            for r in allrec:
-                v = r[H:H + N_BEST]
-                ok = ~np.isnan(v)
-                vs.append(v[ok])
-                rs.append(r[H + N_BEST:H + N_BEST + int(ok.sum()) * len(keys)]
-                          .reshape(-1, len(keys)))
-            vals, rows = np.concatenate(vs), np.concatenate(rs)
-        order = np.argsort(-vals, kind="stable")[:N_BEST]
-        rows = rows[order]
-        if len(rows) < N_BEST:
-            # zero-weight padding rows so that the table always has N_BEST entries
-            pad = rows[-1:] if len(rows) else np.zeros((1, len(keys)))
-            rows = np.concatenate([rows, np.repeat(pad, N_BEST - len(rows), axis=0)])
-        return lnZ, n_pass, n_eval, {k: rows[:, i].copy() for i, k in enumerate(keys)}
-
-    def _merge_posterior(self, allrec):
-        """Posterior table of the whole branch from the ranks' record tails (rank order)."""
-        (K, seed, stream), branch, nk = self.post[0], self.post[1], len(self.keys)
-        P = H + N_BEST * (1 + nk)
-        parts, draws, rows = [], [], []
-        for r in allrec:
-            dr = r[P + 1:P + 1 + K]
-            n = int((~np.isnan(dr)).sum())
-            parts.append((r[0], r[P], dr[:n].astype(np.int64)))
-            draws.append(dr[:n].astype(np.int64))
-            rows.append(r[P + 1 + K:P + 1 + K + n * nk].reshape(n, nk))
-        idx, _, W = _numerics.merge_posteriors(parts, K, seed, stream, branch)
-        draws, rows = np.concatenate(draws), np.concatenate(rows)
-        pos = np.searchsorted(draws, idx)      # (slices are disjoint and ascending)
-        self.posterior = {k: rows[pos, i] for i, k in enumerate(self.keys)}
-        self.posterior["draw"] = idx
-        self.post_total = W

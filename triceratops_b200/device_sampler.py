@@ -24,6 +24,7 @@ agrees on one seed first (rank 0's entropy).
 """
 import contextlib
 import ctypes
+import functools
 import math
 import os
 
@@ -333,40 +334,49 @@ def _take_rows(columns, idx, dev):
     return out
 
 
-def _table(lb, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, rps=None,
-           masses=None, radii=None, fluxratios=None, post=None, branch=0, coords=None):
-    """This rank's half of a result dictionary: the rows of its best local draws (and of its
-    posterior samples, post = (K, seed, stream) of the call), registered for the merge across
-    ranks (_finished)."""
+def _table(res, eng, N, dev, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr,
+           rps=None, masses=None, radii=None, fluxratios=None, post=None, branch=0, coords=None):
+    """This rank's record of one branch: its best local draws with their rows, and with
+    posterior samples (post = (K, seed, stream) of the call) those with theirs, registered for
+    the merge across ranks; returns the merge as a function (_finished)."""
     cols = dict(M_s=M_host, R_s=R_host, u1=u1, u2=u2, P=P, mtot=mtot, inc=incs, ecc=eccs,
                 argp=argps, R_p=rps, M_EB=masses, R_EB=radii, fluxratio_EB=fluxratios,
                 fluxratio_comp=cfr if torch.is_tensor(cfr) else None)
-    idx = torch.as_tensor(np.asarray(lb.idx, dtype=np.int64), device=dev)
-    got = _take_rows(cols, idx, dev)
-    ptab = pcoords = None
-    if post is not None and lb.res.post_idx is not None:
-        pidx = np.asarray(lb.res.post_idx, dtype=np.int64)
+
+    def rows(idx):
+        tab = ml.result_table(len(idx), twin, **_take_rows(cols, idx, dev))
+        return np.stack([tab[k] for k in ml.RESULT_KEYS], axis=1)
+    lo = _dispatch.shard_bounds(N)[0]
+    idx, vals, n_eval = _dispatch._local_best(res, eng, False)
+    fin = np.isfinite(vals)
+    idx, vals = np.asarray(idx, dtype=np.int64)[fin], np.asarray(vals)[fin]
+    tail = pcoords = None
+    if post is not None and res.post_idx is not None:
+        pidx = np.asarray(res.post_idx, dtype=np.int64)
         tidx = torch.as_tensor(pidx, device=dev)
-        ptab = ml.result_table(len(pidx), twin, **_take_rows(cols, tidx, dev))
-        ptab["draw"] = pidx + _dispatch.shard_bounds(lb.N)[0]
+        tail = (post[0], res.post_total, pidx + lo, rows(tidx))
         if coords is not None and _dispatch._dist() is None:
             # gathered on the device by posterior index, one copy (as _take_rows)
             pcoords = coords[:, tidx].T.contiguous().cpu().numpy() if len(pidx) else \
                 np.zeros((0, _cabi.TRI_PROP_SLOTS))
-    ex = _dispatch.TableExchange(lb, ml.result_table(len(lb.idx), twin, **got), ml.RESULT_KEYS,
-                                 None if ptab is None else (post, branch, ptab))
-    ex.post_coords = pcoords
-    return ex
+    rec = _dispatch.pack_slice(res.m, res.s, res.n_finite, res.n_posinf, res.n_pass, n_eval,
+                               getattr(res, "s2", None), idx + lo, vals,
+                               rows(torch.as_tensor(idx, device=dev)), tail)
+    group = _dispatch._group if _dispatch._dist() is not None else None
+    key = None if group is None else group.add(rec)
+    return functools.partial(_finished, rec, group, key, res.lnZ, N, post, branch, pcoords)
 
 
-def _finished(exchange):
-    lnZ, n_pass, n_eval, merged = exchange.result()
-    merged['lnZ'] = lnZ
-    out = ml.ScenarioResult(merged)
-    out.n_pass, out.n_evaluated = n_pass, n_eval
-    out.set_moments(exchange.lb.N, exchange.record, exchange.top)
-    out.posterior, out.post_total = exchange.posterior, exchange.post_total
-    out.post_coords = exchange.post_coords
+def _finished(rec, group, key, lnZ, N, post, branch, pcoords):
+    br = _dispatch.merge_slices(_dispatch.gather_slices(rec, group, key), N,
+                                len(ml.RESULT_KEYS), lnZ, post, branch)
+    rows = br.rows
+    if len(rows) < N_SAMPLES:
+        # zero-weight padding: the last row repeated, so that the table always has N_SAMPLES rows
+        pad = rows[-1:] if len(rows) else np.zeros((1, rows.shape[1]))
+        rows = np.concatenate([rows, np.repeat(pad, N_SAMPLES - len(rows), axis=0)])
+    out = ml.branch_result(br, {k: rows[:, i].copy() for i, k in enumerate(ml.RESULT_KEYS)})
+    out.post_coords = pcoords
     return out
 
 
@@ -388,14 +398,13 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
 
         def prepare():
             if not state:
-                lb = _dispatch.gather_local(p.result(), N, eng)
-                state.append(_table(lb, dev, False, M_host, R_host, u1, u2, P, c["mtot"],
-                                    c["inc"], c["ecc"], c["argp"], cfr, rps=c["body"],
-                                    post=post, coords=c["_coords"]))
+                state.append(_table(p.result(), eng, N, dev, False, M_host, R_host, u1, u2, P,
+                                    c["mtot"], c["inc"], c["ecc"], c["argp"], cfr,
+                                    rps=c["body"], post=post, coords=c["_coords"]))
 
         def table():
             prepare()
-            return _finished(state[0])
+            return state[0]()
         return _dispatch.deliver(table, prepare)
     kw = {"scalar_loop": True} if scalar_loop else {}
     p = _dispatch._submit(eng, "eb_tensors", n,
@@ -409,14 +418,13 @@ def _run(sampled, N, M_s, R_s, u12, is_host, scalar_loop=False):
     def prepare():   # both branches at the first request, in a fixed order
         if not state:
             r0, r1 = p.result()
-            state.append(_table(_dispatch.gather_local(r0, N, eng), dev, False, *args, **tkw))
-            state.append(_table(_dispatch.gather_local(r1, N, eng), dev, True, *args, **tkw,
-                                branch=1))
+            state.append(_table(r0, eng, N, dev, False, *args, **tkw))
+            state.append(_table(r1, eng, N, dev, True, *args, **tkw, branch=1))
 
     def table(b):
         prepare()
         if not done:   # (collectives inside when no CallGroup is open: fixed order)
-            done[0], done[1] = _finished(state[0]), _finished(state[1])
+            done[0], done[1] = state[0](), state[1]()
         return done[b]
     return (_dispatch.deliver(lambda: table(0), prepare),
             _dispatch.deliver(lambda: table(1), prepare))

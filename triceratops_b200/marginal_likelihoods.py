@@ -332,28 +332,33 @@ class ScenarioResult(dict):
                                                  record[4])
 
 
-def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, **body):
-    """ScenarioResult of one branch: rows br.idx of the scenario's columns; `body` holds the
-    per-draw columns of the transiting body (R_p, or M_EB, R_EB and fluxratio_EB)."""
-    idx = br.idx
-    rows = {k: v[idx] for k, v in body.items()}
-    out = ScenarioResult(result_table(
-        N_SAMPLES, twin, _take(M_host, idx), _take(R_host, idx), _take(u1, idx), _take(u2, idx),
-        _take(P, idx), _take(mtot, idx), incs[idx], eccs[idx], argps[idx],
-        fluxratio_comp=_take(cfr, idx) if np.ndim(cfr) else None, **rows), lnZ=br.lnZ)
+def branch_result(br, table, posterior=None):
+    """ScenarioResult of a merged branch (_dispatch.Branch) with the best-draw table `table` and,
+    with posterior samples, their rows `posterior` (dicts of RESULT_KEYS columns; by default the
+    rows that travelled with the samples, br.post_rows)."""
+    out = ScenarioResult(table, lnZ=br.lnZ)
     out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
-    out.set_moments(br.N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
-                    (br.vals, np.asarray(idx)[:len(br.vals)]))
+    out.set_moments(br.N, br.record, (br.vals, np.asarray(br.idx)[:len(br.vals)]))
     if br.post_idx is not None:
-        p = np.asarray(br.post_idx, dtype=np.int64)
-        rows = {k: v[p] for k, v in body.items()}
-        out.posterior = result_table(
-            len(p), twin, _take(M_host, p), _take(R_host, p), _take(u1, p), _take(u2, p),
-            _take(P, p), _take(mtot, p), incs[p], eccs[p], argps[p],
-            fluxratio_comp=_take(cfr, p) if np.ndim(cfr) else None, **rows)
-        out.posterior["draw"] = p
+        if posterior is None:
+            posterior = {k: br.post_rows[:, i] for i, k in enumerate(RESULT_KEYS)}
+        out.posterior = dict(posterior, draw=br.post_idx)
         out.post_total = br.post_total
     return out
+
+
+def _result(br, twin, M_host, R_host, u1, u2, P, mtot, incs, eccs, argps, cfr, **body):
+    """ScenarioResult of one branch: rows br.idx (and br.post_idx) of the scenario's columns;
+    `body` holds the per-draw columns of the transiting body (R_p, or M_EB, R_EB and
+    fluxratio_EB)."""
+    def table(idx, n_zeros):
+        return result_table(
+            n_zeros, twin, _take(M_host, idx), _take(R_host, idx), _take(u1, idx),
+            _take(u2, idx), _take(P, idx), _take(mtot, idx), incs[idx], eccs[idx], argps[idx],
+            fluxratio_comp=_take(cfr, idx) if np.ndim(cfr) else None,
+            **{k: v[idx] for k, v in body.items()})
+    p = br.post_idx
+    return branch_result(br, table(br.idx, N_SAMPLES), None if p is None else table(p, len(p)))
 
 
 def _run_tp(N, M_host, R_host, u1, u2, P, mtot, rps, incs, eccs, argps, cfr, lnprior,

@@ -23,10 +23,9 @@ from pandas import DataFrame, concat
 from scipy.special import ndtr
 
 from . import _bufpool, _dispatch
-from ._numerics import (_normalize_probabilities, mc_error, merge_posteriors,
-                        probability_errors)
+from ._numerics import _normalize_probabilities, mc_error, probability_errors
 from .funcs import renorm_flux
-from .marginal_likelihoods import (RESULT_KEYS, ScenarioResult, lnZ_BEB, lnZ_BTP, lnZ_DEB,
+from .marginal_likelihoods import (RESULT_KEYS, branch_result, lnZ_BEB, lnZ_BTP, lnZ_DEB,
                                    lnZ_DTP, lnZ_PEB, lnZ_PTP, lnZ_SEB, lnZ_STP, lnZ_TEB, lnZ_TTP)
 
 _STAR_COLUMNS = ("ID", "Tmag", "Jmag", "Hmag", "Kmag", "ra", "dec", "mass", "rad", "Teff", "plx",
@@ -273,12 +272,7 @@ class target:
         group = _dispatch.open_group(scatter=host_sampler)
 
         def fill(rows, parts):
-            for j, res in zip(rows, parts):
-                res = _dispatch.resolve(res)
-                for k in RESULT_KEYS:
-                    best[k][j] = res[k][0]
-                lnZ[j] = res["lnZ"]
-                row_results[j] = res
+            _store(rows, [_dispatch.resolve(res) for res in parts], lnZ, best, row_results)
 
         def settle(keep):
             while len(waiting) > keep:
@@ -553,11 +547,7 @@ def _adapt(calls, row_results, lnZ, best, N, N_pilot, seed, post):
         with post() if final else _pilot(seed):
             parts = _round(calls, props, N if final else N_pilot, stage)
     for (rows, _), pt in zip(calls, parts):
-        for j, res in zip(rows, pt):
-            for k in RESULT_KEYS:
-                best[k][j] = res[k][0]
-            lnZ[j] = res["lnZ"]
-            row_results[j] = res
+        _store(rows, pt, lnZ, best, row_results)
 
 
 def _in_stream(make, stream, n):
@@ -595,40 +585,41 @@ def _row_errors(calls, lnZ):
 
 def _merge_round(old, new, offset, post=None):
     """One branch's result over the draws of `old` followed by `new` (drawn after them: its
-    indices start at `offset`), merged like the records of two ranks (_dispatch._merge_records):
-    lnZ over all draws, the best-draw table the top 100 of both, each row from the round that
-    drew it."""
-    N = old.N + new.N
-    allrec = np.stack([
-        _dispatch.record_row(r.record[0], r.record[1], r.record[3], r.record[4], r.n_pass,
-                             r.n_evaluated, r.record[2], np.asarray(r.top[1]) + off, r.top[0])
-        for r, off in ((old, 0), (new, offset))])
-    br = _dispatch._merge_records(allrec, 0, N, N)
-    where = {}
-    for src, off in ((new, offset), (old, 0)):
-        for pos, i in enumerate(np.asarray(src.top[1])[:len(src.top[0])]):
-            where.setdefault(int(i) + off, (src, pos))
-    k = len(br.vals)
-    picks = [where[int(i)] for i in br.idx[:k]]
+    indices start at `offset`), merged as two slices of draws (_dispatch.merge_slices): lnZ over
+    all draws, the best-draw table the top 100 of both, each row from the round that drew it,
+    and with post = (K, seed, stream of the new round, branch) the posterior samples of both."""
+    tails = post is not None and old.posterior is not None and new.posterior is not None
+
+    def pack(r, off):
+        k = len(r.top[0])
+        tail = None
+        if tails:
+            t = r.posterior
+            tail = (post[0], r.post_total, np.asarray(t["draw"]) + off,
+                    np.stack([np.asarray(t[key]) for key in RESULT_KEYS], axis=1))
+        return _dispatch.pack_slice(
+            r.record[0], r.record[1], r.record[3], r.record[4], r.n_pass, r.n_evaluated,
+            r.record[2], np.asarray(r.top[1]) + off, r.top[0],
+            np.stack([np.asarray(r[key][:k]) for key in RESULT_KEYS], axis=1), tail)
+    br = _dispatch.merge_slices(np.stack([pack(old, 0), pack(new, offset)]), old.N + new.N,
+                                len(RESULT_KEYS), post=post[:3] if tails else None,
+                                branch=post[3] if tails else 0)
     # rows of zero weight (fewer than 100 finite draws in all): old's padding rows
-    picks += [(old, pos) for pos in range(k, len(old[RESULT_KEYS[0]]))]
-    out = ScenarioResult({key: np.array([src[key][pos] for src, pos in picks])
-                          for key in RESULT_KEYS}, lnZ=br.lnZ)
-    out.n_pass, out.n_evaluated = br.n_pass, br.n_evaluated
-    out.set_moments(N, (br.m, br.s, br.s2, br.n_finite, br.n_posinf),
-                    (br.vals, br.idx[:k]))
-    if post is not None and old.posterior is not None and new.posterior is not None:
-        # post = (K, seed, stream of the new round, branch): merged like two slices of draws
-        tabs = (old.posterior, {**new.posterior, "draw": new.posterior["draw"] + offset})
-        idx, _, W = merge_posteriors(
-            [(r.record[0], r.post_total, t["draw"]) for r, t in zip((old, new), tabs)], *post)
-        draws = np.concatenate([t["draw"] for t in tabs])
-        pos = np.searchsorted(draws, idx)
-        out.posterior = {key: np.concatenate([np.asarray(t[key]) for t in tabs])[pos]
-                         for key in tabs[0] if key != "draw"}
-        out.posterior["draw"] = idx
-        out.post_total = W
-    return out
+    n = len(old[RESULT_KEYS[0]])
+    pad = np.stack([np.asarray(old[key][len(br.vals):n]) for key in RESULT_KEYS], axis=1)
+    rows = np.concatenate([br.rows, pad])
+    return branch_result(br, {key: rows[:, i] for i, key in enumerate(RESULT_KEYS)})
+
+
+def _store(rows, parts, lnZ, best, row_results=None):
+    """Write the results of one scenario call into its table rows: lnZ, the best draw's columns
+    and (row_results given) the results themselves."""
+    for j, res in zip(rows, parts):
+        lnZ[j] = res["lnZ"]
+        for k in RESULT_KEYS:
+            best[k][j] = res[k][0]
+        if row_results is not None:
+            row_results[j] = res
 
 
 def _refine(calls, row_results, lnZ, best, target, N_max, post=None):
@@ -660,9 +651,6 @@ def _refine(calls, row_results, lnZ, best, target, N_max, post=None):
                                      None if post is None else (*post, stream, b))
                         for b, (old, new) in enumerate(zip(c["cur"], parts))]
             c["N"] += n_new
-            for j, res in zip(c["rows"], c["cur"]):
-                lnZ[j] = res["lnZ"]
-                for k in RESULT_KEYS:
-                    best[k][j] = res[k][0]
+            _store(c["rows"], c["cur"], lnZ, best)
         err, contrib = _row_errors(state, lnZ)
     return err
